@@ -3,6 +3,9 @@
 
     python bench.py --gpus N --steps K --warmup W            our arm (one rank per GPU under torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...   the reference's CPU decoder on the host cores
+    python bench.py ... --dump-outputs DIR                    also writes the per-frame results of the last timed step (the
+                                                              inputs are a function of the arguments: two builds compare
+                                                              output for output)
 
 Headline (BASELINE config 2).  A *step* draws 4 NEW graph realisations (one per eps of the 0.46..0.49 sweep) on the device
 -- scldpc_graph_generate + scldpc_graph_build_tables run INSIDE the timed region -- and decodes --frames-per-graph
@@ -106,16 +109,17 @@ def _ref_worker(args):
 
 
 def _port_worker(args):
-    """Fallback when oracle/_ref is absent: the oracle port (same algorithm, table-driven reverse-edge lookup)."""
+    """Fallback when oracle/_ref is absent: the oracle port (same algorithm, table-driven reverse-edge lookup), timed like
+    _ref_worker, expurgation scan skipped too."""
     seed, eps, cap = args
     import oracle
     oracle.srandom(seed)
     g, _ = oracle.generate_code(L, M, M * DV // DC, DV, DC)
     ch = oracle.channel_doped(g.n, eps, M)
     t0 = time.perf_counter()
-    a = oracle.decode_bp(g, ch, CAP_LO, 1, max_rows=1)
+    a = oracle.decode_bp(g, ch, CAP_LO, 1, max_rows=1, exp_positions=0)
     t1 = time.perf_counter()
-    b = oracle.decode_bp(g, ch, CAP_LO + cap, 1, max_rows=1)
+    b = oracle.decode_bp(g, ch, CAP_LO + cap, 1, max_rows=1, exp_positions=0)
     t2 = time.perf_counter()
     return b["iters"] - a["iters"], (t2 - t1) - (t1 - t0)
 
@@ -664,6 +668,8 @@ def run_ours(args):
     iters_launched = [0]                                       # iterations launched by this rank in the timed region
     graph_events = []
     lock = threading.Lock()
+    last_timed = args.warmup + args.steps - 1
+    last_res = []                                              # per-frame results of the last timed step (--dump-outputs)
 
     def step(s, acc=True, t=0):
         fbt = fbs[t]
@@ -679,6 +685,8 @@ def run_ours(args):
             fbt.generate_erasures(eps, seed=args.seed + 1, first_graph_id=gid)
             res, erased, rows, launched = eng.decode_bp_full(fbt, eng.UNLIMITED, True, collect=False)
             it, resid = res[0, :, :lanes].to(torch.int64), res[1, :, :lanes].to(torch.int64)
+        if s == last_timed:
+            last_res.append(res[:5])                           # a fresh tensor per call: nothing overwrites it later
         if acc:
             with lock:
                 graph_events.append((g0, g1))
@@ -945,9 +953,30 @@ def run_ours(args):
             "cpu_baseline": cpu_baseline, "workloads": workloads,
         }
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_res[0])
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_NAMES = ("iters", "residual", "blocks_err", "erasures_exp", "blocks_err_exp")
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir: str, res) -> None:
+    """Per-frame results of one step (int32 [5][graphs][frames], DUMP_NAMES) -> out_dir/<name>.npy, float64 [graphs][frames].
+    Above DUMP_LIMIT bytes in all, every array keeps the same seeded sample of frame ids, listed in frame_ids.npy."""
+    import numpy as np
+    r = res.cpu().numpy().astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    k = DUMP_LIMIT // (8 * (r.shape[0] * r.shape[1] + 1))
+    if r.shape[2] > k:
+        ids = np.sort(np.random.default_rng(0).choice(r.shape[2], k, replace=False))
+        r = r[:, :, ids]
+        np.save(os.path.join(out_dir, "frame_ids.npy"), ids.astype(np.float64))
+    for name, a in zip(DUMP_NAMES, r):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def main():
@@ -970,7 +999,13 @@ def main():
     ap.add_argument("--frames-per-graph", type=int, default=FRAMES_PER_STREAM)
     ap.add_argument("--pipeline", type=int, default=2, help="stream mode: batches in flight (host threads x CUDA streams); 1 = one batch after the other")
     ap.add_argument("--harvest-every", type=int, default=0, help="stream mode: iterations between harvests (0: adaptive)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the per-frame results of the last timed step as DIR/<name>.npy "
+                                                          "(float64 [graphs][frames]; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     N_WORDS = args.n_words
     if args.impl == "reference":
         return run_reference(args)

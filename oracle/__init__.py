@@ -102,16 +102,19 @@ def is_position_doped_streaming(pos: int, doped) -> bool:
 
 
 def decode_bp(g: Graph, chan: np.ndarray, max_it: int, is_term: int = 1, max_rows: int | None = None,
-              want_msgs: bool = False) -> dict:
-    """``orc_decode_bp`` (reference ``decodeBP``)."""
+              want_msgs: bool = False, exp_positions: int | None = None) -> dict:
+    """``orc_decode_bp`` (reference ``decodeBP``).  ``exp_positions`` is the ``L`` argument, which a terminated decode
+    uses only as the range of its post-decoding expurgation scan; 0 skips that scan, as ``ref_driver``'s does."""
     chan = np.ascontiguousarray(chan, np.int32)
+    Larg = g.L if exp_positions is None else exp_positions
+    assert is_term or Larg == g.L
     erased = np.zeros(g.n, np.uint8)
     max_rows = max(1, max_it) if max_rows is None else max_rows
     rows = np.zeros((max_rows, 3), np.int32)
     it, nb, ne, nbe = (ctypes.c_int(0) for _ in range(4))
     lji = np.zeros((g.n, g.dv), np.int32) if want_msgs else None
     lij = np.zeros((g.n, g.dv), np.int32) if want_msgs else None
-    res = lib().orc_decode_bp(g.n, g.nk, g.L, g.vns_pos, g.cns_pos, g.dv, g.dc, _ptr(g.vn_cn), _ptr(g.cn_deg),
+    res = lib().orc_decode_bp(g.n, g.nk, Larg, g.vns_pos, g.cns_pos, g.dv, g.dc, _ptr(g.vn_cn), _ptr(g.cn_deg),
                               _ptr(g.cn_vn), _ptr(g.cn_ei), _ptr(g.vn_slot), _ptr(chan), max_it, is_term,
                               _ptr(erased), ctypes.byref(it), ctypes.byref(nb), ctypes.byref(ne), ctypes.byref(nbe),
                               _ptr(rows), max_rows, _ptr(lji), _ptr(lij))
