@@ -47,6 +47,7 @@ def lib():
         _lib.orc_decode_bp_sw.restype = ctypes.c_int
         _lib.orc_build_cn.restype = ctypes.c_int
         _lib.orc_peel_trajectory.restype = ctypes.c_int
+        _lib.orc_peel_trajectory_fast.restype = ctypes.c_int
         _lib.orc_is_position_doped_streaming.restype = ctypes.c_int
     return _lib
 
@@ -180,6 +181,20 @@ def peel_trajectory(vn_cn: np.ndarray, erased: np.ndarray, total_size: int, n_cn
     r1 = np.zeros(num_steps + 1, np.int64)
     rec = lib().orc_peel_trajectory(vn_cn.shape[0], vn_cn.shape[1], total_size, n_cn_all, _ptr(vn_cn), _ptr(erased),
                                     num_steps, _ptr(picks), _ptr(r1))
+    return r1, int(rec)
+
+
+def peel_trajectory_fast(vn_cn: np.ndarray, erased: np.ndarray, total_size: int, n_cn_all: int, num_steps: int,
+                         picks: np.ndarray):
+    """``orc_peel_trajectory_fast``: what ``peel_trajectory`` returns, in O(log #CN) per step (a Fenwick tree over the
+    degree-one CNs) instead of a scan -- full-length trajectories at M >= 10^4."""
+    vn_cn = np.ascontiguousarray(vn_cn, np.int32)
+    erased = np.ascontiguousarray(erased, np.uint8)
+    picks = np.ascontiguousarray(picks, np.uint32)
+    assert picks.size >= num_steps
+    r1 = np.zeros(num_steps + 1, np.int64)
+    rec = lib().orc_peel_trajectory_fast(vn_cn.shape[0], vn_cn.shape[1], total_size, n_cn_all, _ptr(vn_cn), _ptr(erased),
+                                         num_steps, _ptr(picks), _ptr(r1))
     return r1, int(rec)
 
 

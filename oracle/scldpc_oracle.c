@@ -376,6 +376,63 @@ int orc_peel_trajectory(int n_vn, int l, int total_size, int n_cn_all, const int
     return recovered;
 }
 
+/* orc_peel_trajectory with the same inputs and outputs, O(log total_size) per step instead of O(total_size): the
+ * degree-one indicator of the CNs [0, total_size) is kept in a Fenwick tree (1-based, fw[i] = number of degree-one CNs
+ * in (i - lowbit(i), i]), and "the k-th degree-one CN in ascending order" is the usual top-down descent over it.
+ * Written from the PD.py semantics above, not from the kernel's bitmap hierarchy, so that it stays an independent check;
+ * tests/test_peel_oracle_cpu.py holds it to orc_peel_trajectory. */
+static void fw_add(int *fw, int n, int t, int d)
+{
+    for (int i = t + 1; i <= n; i += i & -i) fw[i] += d;
+}
+
+static int fw_select(const int *fw, int n, int64_t k)   /* 0-based index of the (k+1)-th set position */
+{
+    int pos = 0, top = 1;
+    while (top * 2 <= n) top *= 2;
+    for (int b = top; b; b >>= 1)
+        if (pos + b <= n && fw[pos + b] <= k) { pos += b; k -= fw[pos]; }
+    return pos;
+}
+
+int orc_peel_trajectory_fast(int n_vn, int l, int total_size, int n_cn_all, const int *vn_cn, const unsigned char *erased,
+                             int num_steps, const uint32_t *picks, int64_t *r1)
+{
+    int *r = (int *)calloc((size_t)n_cn_all, sizeof(int));
+    uint32_t *xr = (uint32_t *)calloc((size_t)n_cn_all, sizeof(uint32_t));
+    int *fw = (int *)calloc((size_t)total_size + 1, sizeof(int));
+    for (int v = 0; v < n_vn; v++)
+        if (erased[v])
+            for (int i = 0; i < l; i++) { int c = vn_cn[(size_t)v * l + i]; r[c]++; xr[c] ^= (uint32_t)v; }
+    int64_t cnt1 = 0;
+    for (int t = 0; t < total_size; t++)                         /* linear-time build: push each node into its parent */
+        if (r[t] == 1) { fw[t + 1] += 1; cnt1++; }
+    for (int i = 1; i <= total_size; i++) {
+        int p = i + (i & -i);
+        if (p <= total_size) fw[p] += fw[i];
+    }
+    r1[0] = cnt1;
+    int recovered = 0;
+    for (int step = 0; step < num_steps; step++) {
+        if (cnt1 == 0) { r1[step + 1] = r1[step]; continue; }
+        int m = fw_select(fw, total_size, (int64_t)(picks[step] % (uint64_t)cnt1));
+        int v = (int)xr[m];
+        recovered++;
+        for (int i = 0; i < l; i++) {
+            int c = vn_cn[(size_t)v * l + i];
+            xr[c] ^= (uint32_t)v;
+            r[c]--;
+            if (c < total_size) {
+                if (r[c] == 1) { fw_add(fw, total_size, c, 1); cnt1++; }
+                else if (r[c] == 0) { fw_add(fw, total_size, c, -1); cnt1--; }
+            }
+        }
+        r1[step + 1] = cnt1;
+    }
+    free(r); free(xr); free(fw);
+    return recovered;
+}
+
 /* Peeling to the fixed point = residual of unlimited flooding BP (simulate_sc_ldpc's sic_round scan,
  * PD.py:270-320,:656-657, reaches the same maximal stopping set; SURVEY.md section 3.5).  Slots are scanned from
  * scan_lo = ignored_head_schedule*cns_per_pos up to cn_hi = total_size (PD.py:656); a cascade
