@@ -1,6 +1,7 @@
 """Drop-ins for the three reference executables (``simulators_sc_ldpc/bp_decoding/CMakeLists.txt:8-10``):
 
     bp_lim_iter INDEX W NUM_DOPED MAX_IT [DOPED...]            full BP, iteration-limited      (BP_FULL.c main_terminated :2057)
+                [--caps T1,T2,...]                              ... and at several caps from one decode (one file per cap)
     sw_lim_iter INDEX W NUM_DOPED MAX_IT INIT_IT [DOPED...]    sliding window (square window)  (BP_SW.c :2072)
     bp_traj     INDEX W NUM_DOPED MAX_IT IS_TERM [DOPED...]    full BP trajectories            (BP_TRAJ.c :2068)
 
@@ -56,6 +57,38 @@ def new_counters():
     return dict(users_err=0, frame_err=0, block_err=0, users_err_exp=0, frame_err_exp=0, block_err_exp=0, frame_errP1=0)
 
 
+def parse_caps(max_it: int, caps_arg: str) -> list[int]:
+    """``bp_lim_iter --caps``: MAX_IT together with the listed caps, each through max(1, .) like MAX_IT itself, sorted and
+    deduplicated."""
+    vals = [max_it] + [int(x) for x in caps_arg.split(",") if x.strip()]
+    return sorted({max(1, v) for v in vals})
+
+
+def replay_caps(records, max_frames: int, min_frame_err: int, state=None):
+    """Per-cap ``plr_computation`` / ``willIstop`` over one round of frames of a shared checkpointed stream.
+
+    ``records``: int array [N][K][4], per frame in global frame order and per cap (ascending) the residual, blocks_err,
+    erasures_exp and blocks_err_exp.  Every cap accounts frames in order until its own ``frame_err >= min_frame_err``
+    or ``max_frames``, exactly as a separate run at that cap would over the same frames.  ``state``: the result of the
+    previous round of the same point (None for the first); returns the updated list of K dicts with ``counters``,
+    ``frames`` and ``stopped``."""
+    rec = np.asarray(records)
+    K = rec.shape[1]
+    if state is None:
+        state = [dict(counters=new_counters(), frames=0, stopped=False) for _ in range(K)]
+    for k in range(K):
+        s = state[k]
+        c = s["counters"]
+        for i in range(rec.shape[0]):
+            if s["frames"] >= max_frames or s["stopped"]:
+                break
+            account(c, rec[i, k, 0], rec[i, k, 1], rec[i, k, 2], rec[i, k, 3])
+            s["frames"] += 1
+            if c["frame_err"] >= min_frame_err:
+                s["stopped"] = True
+    return state
+
+
 def trajectory_text(rows: np.ndarray, iters: int) -> str:
     """decodeBP's per-frame text (BP_TRAJ.c:988,1051,1145): ``iter\\tdeg1\\tdVNs\\tfirst_pos`` lines + a blank line."""
     out = []
@@ -95,6 +128,16 @@ def _parser(prog):
     ap.add_argument("--graphs-per-batch", type=int, default=16)
     ap.add_argument("--stream", choices=["auto", "on", "off"], default="auto",
                     help="bp_lim_iter: decode each graph's frames as a stream with lane recycling (auto: from 1024 frames per graph)")
+    if prog == "bp_lim_iter":
+        ap.add_argument("--caps", default=None, metavar="T1,T2,...",
+                        help="error rates at several iteration limits from one decode: the caps are MAX_IT and these values (each "
+                             "max(1, .)), and every cap gets the file, name and rows a run with that MAX_IT writes, with its own "
+                             "early stop and counters.  Always on the stream path (--stream off is an error).  The frames are "
+                             "decoded once up to the largest cap.  A frame in error at a cap is in error at every smaller cap, so "
+                             "the largest cap stops last and the points advance as in a separate run at the largest cap: its file "
+                             "is byte-identical to that run's; every cap's first point is, and so is every point when no cap "
+                             "stops early.  For later points a smaller cap's rows come from the frames the shared run drew, "
+                             "which differ from the ones a separate run at that cap would draw")
     if prog == "bp_traj":
         ap.add_argument("--moments-file", default=None,
                         help="also accumulate the per-iteration moments of the rows on the device (engine.MOMENT_NAMES) and pickle "
@@ -137,6 +180,16 @@ def run(prog: str, argv=None) -> int:
     moments_all = {}
     sw = prog == "sw_lim_iter"
     use_stream = prog == "bp_lim_iter" and (a.stream == "on" or (a.stream == "auto" and fpg >= 1024))
+    caps = None
+    if getattr(a, "caps", None) is not None:
+        if a.stream == "off":
+            raise SystemExit(f"{prog}: --caps decodes on the stream path; it cannot be combined with --stream off")
+        caps = parse_caps(a.max_it, a.caps)
+        if len(caps) > engine._lib.MAX_CAPS:
+            raise SystemExit(f"{prog}: at most {engine._lib.MAX_CAPS} caps")
+        use_stream = True
+        # a run with MAX_IT = T writes "%dit" with T as given; the cap MAX_IT itself keeps that name
+        cap_names = {c: name.replace("_%dit_" % a.max_it, "_%dit_" % (a.max_it if c == max_it else c)) for c in caps}
     for sim in range(a.points):
         eps = a.eps_ini - sim * a.eps_delta                            # inizio_sim, BP_FULL.c:300
         c = new_counters()
@@ -153,6 +206,7 @@ def run(prog: str, argv=None) -> int:
         # per-frame results are all-gathered and every rank replays plr_computation / willIstop over them in frame order,
         # so the files are the same for any number of GPUs.
         rnd = 0
+        cap_state = None
         while f < a.max_frames and not stop:
             gid = graph_id + (rnd * world + rank) * G
             rnd += 1
@@ -162,6 +216,17 @@ def run(prog: str, argv=None) -> int:
                 lanes = min(fpg, 1024)
                 fb = engine.FrameBatch(ens, G, lanes, engine.words_for(lanes))
                 fb.generate_graphs(seed, first_graph_id=gid)
+                if caps is not None:
+                    # one record of 1 + 4K integers per frame: iterations under the largest cap, then the statistics per cap
+                    r = engine.decode_bp_stream(fb, fpg, eps, seed + 1, first_graph_id=gid, is_term=True, doping_points=doped, caps=caps)
+                    K = len(caps)
+                    st = np.stack([r.residual, r.blocks_err, r.erasures_exp, r.blocks_err_exp], axis=-1)      # [K][G][B][4]
+                    rec = np.concatenate([r.iters.reshape(-1, 1), st.transpose(1, 2, 0, 3).reshape(-1, 4 * K)], axis=1).astype(np.int64)
+                    rec = D.allgather_rows(rec).reshape(-1, 1 + 4 * K)
+                    cap_state = replay_caps(rec[:, 1:].reshape(-1, K, 4), a.max_frames, a.min_frame_err, cap_state)
+                    f, stop = cap_state[-1]["frames"], cap_state[-1]["stopped"]        # the largest cap stops last
+                    c = cap_state[-1]["counters"]
+                    continue
                 r = engine.decode_bp_stream(fb, fpg, eps, seed + 1, first_graph_id=gid, is_term=True, doping_points=doped, max_it=max_it)
                 rec = np.stack([r.residual, r.blocks_err, r.erasures_exp, r.blocks_err_exp, np.zeros_like(r.residual), r.iters],
                                axis=-1).astype(np.int64)
@@ -220,6 +285,13 @@ def run(prog: str, argv=None) -> int:
         if rank == 0:
             print("%s: eps=%f frames=%d frames_per_graph=%d graphs=%d frame_err=%d (the reference draws one graph per frame)"
                   % (prog, eps, f, fpg, n_graphs_point, c["frame_err"]), file=sys.stderr)
+        if rank == 0 and caps is not None:
+            for cap, s in zip(caps, cap_state):
+                with open(os.path.join(a.outdir, cap_names[cap]), "w" if sim == 0 else "a") as out:
+                    if sim == 0:
+                        out.write(HEADER)
+                    out.write(result_row(eps, ens.n, a.L, s["frames"], s["counters"]))
+            continue
         # BP_TRAJ.c's main_terminated only writes the trajectories file (its risultati call is commented out, :2176)
         if rank == 0 and prog != "bp_traj":
             with open(os.path.join(a.outdir, name), "w" if sim == 0 else "a") as out:

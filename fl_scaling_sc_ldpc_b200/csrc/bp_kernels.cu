@@ -341,8 +341,10 @@ __global__ void __launch_bounds__(256) bp_pos_count_kernel(BpParams p)
     __syncthreads();
     const u128 *x = p.x + ((size_t)g * p.n + (size_t)pos * p.vns_pos) * ch;
     const int items = p.vns_pos * ch;
-    // a thread keeps its chunk (blockDim and the stride are multiples of ch); chunks without a selected lane are skipped
-    const u128 mask = p.lane_mask ? reinterpret_cast<const u128 *>(p.lane_mask)[g * ch + (threadIdx.x & (ch - 1))] : ones128();
+    // a thread keeps its chunk (blockDim and the stride are multiples of ch); chunks without a selected lane are skipped.
+    // Streams with checkpoints also count the frames paused at a checkpoint.
+    u128 mask = p.lane_mask ? reinterpret_cast<const u128 *>(p.lane_mask)[g * ch + (threadIdx.x & (ch - 1))] : ones128();
+    if (p.pause_mask) mask |= reinterpret_cast<const u128 *>(p.pause_mask)[g * ch + (threadIdx.x & (ch - 1))];
     if (nz(mask))
         for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < items; idx += gridDim.x * blockDim.x) {
             const u128 xv = x[idx] & mask;

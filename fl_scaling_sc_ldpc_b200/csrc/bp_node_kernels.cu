@@ -60,9 +60,13 @@ namespace scldpc {
 // The sweep is bound by L2 latency and instruction issue, not by HBM (DESIGN.md section 4).
 // CAPPED (streams with an iteration cap): a frame that hit the cap is not at a fixed point, so its bits must not be cleared
 // while it waits for the harvest -- the resolutions are masked with the frames still iterating.
-template <int DV, int DC, bool CAPPED>
+// CKPT (streams with checkpoints, CAPPED as well): a frame that reaches its next checkpoint caps[lane_ck] without stopping
+// in that iteration pauses -- it leaves active for pause_mask, not done_mask -- and the harvest records its statistics and
+// puts it back into active.  A paused lane is masked like a capped one, and its lane_iter does not advance.
+template <int DV, int DC, bool CAPPED, bool CKPT = false>
 __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
 {
+    static_assert(CAPPED || !CKPT, "a paused frame must not be cleared");
     static_assert(DC <= 16, "neighbour index is encoded in four bit planes");
     pdl_wait_then_release();
     const int g = graph_of(p, blockIdx.y);
@@ -192,8 +196,12 @@ __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
     __threadfence();
     // ---- end of the iteration for graph g ----
     __shared__ u64 s_act[SCLDPC_MAX_WORDS], s_cap[SCLDPC_MAX_WORDS];
+    __shared__ u64 s_ck[CKPT ? SCLDPC_MAX_WORDS : 1];
     const int W = p.W;
-    for (int w = threadIdx.x; w < W; w += blockDim.x) { s_act[w] = p.active[g * W + w]; s_cap[w] = 0; }
+    for (int w = threadIdx.x; w < W; w += blockDim.x) {
+        s_act[w] = p.active[g * W + w]; s_cap[w] = 0;
+        if (CKPT) s_ck[w] = 0;
+    }
     __syncthreads();
     for (int l = threadIdx.x; l < p.lanes; l += blockDim.x) {
         const int w = l >> 6, b = l & 63;
@@ -201,6 +209,10 @@ __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
             const int li = p.lane_iter[g * p.lanes + l] + 1;
             p.lane_iter[g * p.lanes + l] = li;
             if (CAPPED && li >= p.stream_cap) atomicOr(reinterpret_cast<unsigned long long *>(&s_cap[w]), 1ull << b);   // while (iter < MaxNumIt)
+            else if (CKPT) {
+                const int ck = p.lane_ck[g * p.lanes + l];
+                if (ck < p.n_caps - 1 && li >= p.caps[ck]) atomicOr(reinterpret_cast<unsigned long long *>(&s_ck[w]), 1ull << b);
+            }
         }
     }
     __syncthreads();
@@ -210,7 +222,12 @@ __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
         // channel left some VN known (first_new)
         const u64 nw = ld_cg(p.any_new + g * W + w) | ld_cg(p.first_new + g * W + w);
         const u64 stop = a & (~nw | s_cap[w]);                  // NumErasures == NumErasuresPrec (or == 0, one iteration late) || cap
-        p.active[g * W + w] = a & ~stop;
+        if (CKPT) {
+            const u64 pause = s_ck[w] & ~stop;                  // a frame that stops at a checkpoint stops
+            p.active[g * W + w] = a & ~stop & ~pause;
+            if (pause) p.pause_mask[g * W + w] |= pause;
+        } else
+            p.active[g * W + w] = a & ~stop;
         p.done_mask[g * W + w] |= stop;
         p.noprog[g * W + w] |= a & ~nw;
         p.any_new[g * W + w] = 0;
@@ -368,14 +385,15 @@ __global__ void __launch_bounds__(256, 4) ns_arm_kernel(BpParams p)
 // over all chunks -- about 1000 of the 14 500 iterations of the benchmarked eps = 0.49 graph run with a few dozen live frames
 // at the full price.  After a harvest that armed nothing, when the live frames fit into half the chunks in use, they move to
 // the lowest lanes: a frame's whole decoder state is its bit column in the (equal, settled) planes plus lane_frame and
-// lane_iter, so the move is one pass over the plane; gshift[g] then tells ns_iter_kernel to spread its threads over the
-// occupied chunks only.  Frame results are stored under the frame id, so nothing downstream sees the lane change.
+// lane_iter (and lane_ck in a stream with checkpoints, whose paused frames the harvest has just put back into active), so the
+// move is one pass over the plane; gshift[g] then tells ns_iter_kernel to spread its threads over the occupied chunks only.
+// Frame results are stored under the frame id, so nothing downstream sees the lane change.
 __global__ void ns_compact_plan_kernel(BpParams p)
 {
     const int g = graph_of(p, blockIdx.x), W = p.W;
     __shared__ u64 s_act[SCLDPC_MAX_WORDS];
     __shared__ int s_rank[SCLDPC_MAX_WORDS + 1], s_go;
-    __shared__ int s_fr[SCLDPC_MAX_LANES], s_it[SCLDPC_MAX_LANES];
+    __shared__ int s_fr[SCLDPC_MAX_LANES], s_it[SCLDPC_MAX_LANES], s_ck[SCLDPC_MAX_LANES];
     if (threadIdx.x == 0) {
         p.cmp_cnt[g] = 0;
         int go = ld_cg(p.alive + g) != 0 && p.next_frame[g] >= p.frames_per_graph && p.gshift[g] > 0;
@@ -400,12 +418,14 @@ __global__ void ns_compact_plan_kernel(BpParams p)
             p.cmp_src[g * p.lanes + i] = l;
             s_fr[i] = p.lane_frame[g * p.lanes + l];
             s_it[i] = p.lane_iter[g * p.lanes + l];
+            if (p.lane_ck) s_ck[i] = p.lane_ck[g * p.lanes + l];
         }
     }
     __syncthreads();
     for (int l = threadIdx.x; l < p.lanes; l += blockDim.x) {
         p.lane_frame[g * p.lanes + l] = l < A ? s_fr[l] : -1;
         p.lane_iter[g * p.lanes + l] = l < A ? s_it[l] : 0;
+        if (p.lane_ck) p.lane_ck[g * p.lanes + l] = l < A ? s_ck[l] : 0;
     }
     for (int w = threadIdx.x; w < W; w += blockDim.x)
         p.active[g * W + w] = A >= 64 * (w + 1) ? ~0ull : (A <= 64 * w ? 0ull : ((1ull << (A - 64 * w)) - 1ull));
@@ -517,7 +537,8 @@ static void launch_node_iteration(const BpParams &p, bool after_harvest, cudaStr
     g_prof.launches += 1;
     static const bool pdl = getenv("SCLDPC_NO_PDL") == nullptr;
     // the first launch after a harvest follows ordinary kernels: full serialisation there
-    if (p.stream_cap > 0) launch_pdl(ns_iter_kernel<DV, DC, true>, grid, block, st, pdl && !after_harvest && !sample, p);
+    if (p.n_caps > 0) launch_pdl(ns_iter_kernel<DV, DC, true, true>, grid, block, st, pdl && !after_harvest && !sample, p);
+    else if (p.stream_cap > 0) launch_pdl(ns_iter_kernel<DV, DC, true>, grid, block, st, pdl && !after_harvest && !sample, p);
     else launch_pdl(ns_iter_kernel<DV, DC, false>, grid, block, st, pdl && !after_harvest && !sample, p);
     if (sample) {
         cudaEventRecord(ev[1], st);

@@ -490,18 +490,37 @@ __global__ void __launch_bounds__(256, ARM ? 3 : 4) bp_vn_stream_kernel(BpParams
     if (threadIdx.x == 0) p.ticket[g] = 0;
 }
 
-// harvest step 3 (one block per graph): results of the lanes in done_mask, then re-arm them with the next frame ids
+// statistics of frame slot o ([G][B]) into the checkpoint slots [k0, k1) of the [K][G][B] outputs
+__device__ __forceinline__ void store_ck_slots(const BpParams &p, size_t o, int k0, int k1, int residual, int blocks, int e_exp, int b_exp)
+{
+    const size_t GB = (size_t)p.G * p.frames_per_graph;
+    for (int k = k0; k < k1; k++) {
+        p.s_residual[k * GB + o] = residual;
+        p.s_blocks_err[k * GB + o] = blocks;
+        p.s_erasures_exp[k * GB + o] = e_exp;
+        p.s_blocks_err_exp[k * GB + o] = b_exp;
+    }
+}
+
+// harvest step 3 (one block per graph): results of the lanes in done_mask, then re-arm them with the next frame ids.
+// CKPT (node-state streams with checkpoints): a frame paused at checkpoint k = lane_ck gets its statistics recorded into
+// slot k, advances lane_ck and goes back into active -- it is not re-armed, so its next iteration continues from the settled
+// planes with the stall test it had.  A frame that stopped fills every slot from lane_ck on: the caps it has not reached are
+// at least its stop iteration.
+template <bool CKPT>
 __global__ void bp_stream_harvest_kernel(BpParams p, int exp_all)
 {
     const int g = graph_of(p, blockIdx.x), L = p.L, W = p.W, B = p.frames_per_graph;
     if (ld_cg(p.alive + g) == 0) return;
     __shared__ int s_rank[SCLDPC_MAX_WORDS + 1];
     __shared__ u64 s_done[SCLDPC_MAX_WORDS], s_arm[SCLDPC_MAX_WORDS];
+    __shared__ u64 s_pause[CKPT ? SCLDPC_MAX_WORDS : 1];
     __shared__ int s_frames;
     __shared__ unsigned long long s_its;
     // (the word loops of this kernel run one word per thread: as thread-0 loops they were chains of dependent global round trips,
     // two thirds of the kernel's 21 us)
     if (threadIdx.x < W) { s_done[threadIdx.x] = p.done_mask[g * W + threadIdx.x]; s_arm[threadIdx.x] = 0; }
+    if (CKPT && threadIdx.x < W) s_pause[threadIdx.x] = p.pause_mask[g * W + threadIdx.x];
     if (threadIdx.x == 0) { s_frames = 0; s_its = 0; }
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -515,7 +534,8 @@ __global__ void bp_stream_harvest_kernel(BpParams p, int exp_all)
     // frame's counts are zero by construction
     for (int l = threadIdx.x >> 5; l < p.lanes; l += blockDim.x >> 5) {
         const int w = l >> 6, b = l & 63;
-        if (!((s_done[w] >> b) & 1ull) || !((p.fail_mask[g * W + w] >> b) & 1ull)) continue;
+        const u64 counted = CKPT ? (s_done[w] | s_pause[w]) : s_done[w];
+        if (!((counted >> b) & 1ull) || !((p.fail_mask[g * W + w] >> b) & 1ull)) continue;
         const int fr = p.lane_frame[g * p.lanes + l];
         int residual = 0, blocks = 0, e_exp = 0, b_exp = 0, first_q = INT_MAX, first_ex = 0;
         for (int q = threadIdx.x & 31; q < L; q += 32) {
@@ -544,15 +564,26 @@ __global__ void bp_stream_harvest_kernel(BpParams p, int exp_all)
         }
         if ((threadIdx.x & 31) == 0 && fr >= 0 && fr < B) {
             const size_t o = (size_t)g * B + fr;
-            p.s_residual[o] = residual;
-            p.s_blocks_err[o] = blocks;
-            p.s_erasures_exp[o] = e_exp;
-            p.s_blocks_err_exp[o] = b_exp;
+            if (CKPT) {
+                const int k0 = p.lane_ck[g * p.lanes + l];
+                store_ck_slots(p, o, k0, ((s_pause[w] >> b) & 1ull) ? k0 + 1 : p.n_caps, residual, blocks, e_exp, b_exp);
+            } else {
+                p.s_residual[o] = residual;
+                p.s_blocks_err[o] = blocks;
+                p.s_erasures_exp[o] = e_exp;
+                p.s_blocks_err_exp[o] = b_exp;
+            }
         }
     }
     __syncthreads();
     for (int l = threadIdx.x; l < p.lanes; l += blockDim.x) {
         const int w = l >> 6, b = l & 63;
+        if (CKPT && ((s_pause[w] >> b) & 1ull)) {              // paused: snapshot without erasures, next checkpoint, resume
+            const int fr = p.lane_frame[g * p.lanes + l], k = p.lane_ck[g * p.lanes + l];
+            if (fr >= 0 && fr < B && !((p.fail_mask[g * W + w] >> b) & 1ull)) store_ck_slots(p, (size_t)g * B + fr, k, k + 1, 0, 0, 0, 0);
+            p.lane_ck[g * p.lanes + l] = k + 1;
+            continue;
+        }
         if (!((s_done[w] >> b) & 1ull)) continue;
         const int fr = p.lane_frame[g * p.lanes + l];
         if (fr >= 0 && fr < B) {
@@ -564,12 +595,16 @@ __global__ void bp_stream_harvest_kernel(BpParams p, int exp_all)
             atomicAdd(&s_frames, 1);
             atomicAdd(&s_its, (unsigned long long)its);
             if (!((p.fail_mask[g * W + w] >> b) & 1ull)) {
-                p.s_residual[o] = 0;
-                p.s_blocks_err[o] = 0;
-                p.s_erasures_exp[o] = 0;
-                p.s_blocks_err_exp[o] = 0;
+                if (CKPT) store_ck_slots(p, o, p.lane_ck[g * p.lanes + l], p.n_caps, 0, 0, 0, 0);
+                else {
+                    p.s_residual[o] = 0;
+                    p.s_blocks_err[o] = 0;
+                    p.s_erasures_exp[o] = 0;
+                    p.s_blocks_err_exp[o] = 0;
+                }
             }
         }
+        if (CKPT) p.lane_ck[g * p.lanes + l] = 0;
         // freed lanes take the next frame ids in ascending lane order
         const int nf = next0 + s_rank[w] + __popcll(s_done[w] & ((1ull << b) - 1ull));
         if (nf < B) {
@@ -584,7 +619,11 @@ __global__ void bp_stream_harvest_kernel(BpParams p, int exp_all)
     __syncthreads();
     if (threadIdx.x < W) {
         const int w = threadIdx.x;
-        const u64 act = p.active[g * W + w];
+        u64 act = p.active[g * W + w];
+        if (CKPT) {                                             // paused frames are live: they continue with the next iteration
+            act |= s_pause[w];
+            p.pause_mask[g * W + w] = 0;
+        }
         p.done_mask[g * W + w] = 0;
         p.fail_mask[g * W + w] = 0;
         p.arm_mask[g * W + w] = s_arm[w];
@@ -743,7 +782,9 @@ void bp_launch_stream_init(const BpParams &p, int n_lanes_used, cudaStream_t st)
 void bp_launch_stream_harvest(const BpParams &p, int exp_all, cudaStream_t st)
 {
     g_prof.launches += 1;
-    bp_stream_harvest_kernel<<<graphs_in_grid(p), 1024, 0, st>>>(p, exp_all);   // one warp per failed frame: 32 at a time
+    // one warp per failed frame: 32 at a time
+    if (p.n_caps > 0) bp_stream_harvest_kernel<true><<<graphs_in_grid(p), 1024, 0, st>>>(p, exp_all);
+    else bp_stream_harvest_kernel<false><<<graphs_in_grid(p), 1024, 0, st>>>(p, exp_all);
 }
 
 void bp_launch_wave_init(const BpParams &p, cudaStream_t st)

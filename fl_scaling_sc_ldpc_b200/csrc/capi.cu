@@ -173,6 +173,9 @@ static size_t list_stride(size_t max_nodes, size_t ch)
     return s;
 }
 
+// internal: workspace of scldpc_bp_stream_caps (per-lane checkpoint state on top of the node-state stream's)
+#define F_CAPS_WS 0x10000u
+
 static size_t carve(const scldpc_dims_t *d, uint32_t flags, void *ws, BpParams *p)
 {
     const size_t G = d->n_graphs, W = d->n_words, ch = W / 2, lanes = 64 * W;
@@ -233,6 +236,10 @@ static size_t carve(const scldpc_dims_t *d, uint32_t flags, void *ws, BpParams *
             q.gshift = c.take<int>(G);
             q.cmp_cnt = c.take<int>(G);
             q.cmp_src = c.take<int>(G * lanes);
+            if (flags & F_CAPS_WS) {
+                q.lane_ck = c.take<int>(G * lanes);
+                q.pause_mask = c.take<u64>(G * W);
+            }
         }
     }
     q.cn_dis = (flags & SCLDPC_F_STREAM) ? nullptr : c.take<u128>(G * nk * ch);   // sized for the largest possible ignored head
@@ -595,10 +602,17 @@ extern "C" size_t scldpc_bp_stream_workspace_bytes(const scldpc_dims_t *d, uint3
     return carve(d, SCLDPC_F_STREAM | (flags & SCLDPC_F_MESSAGES), nullptr, nullptr);
 }
 
-// Full BP (unlimited iterations) over a stream of cfg->frames_per_graph frames per graph with lane recycling.
-extern "C" int scldpc_bp_stream(const scldpc_dims_t *d, const scldpc_batch_t *b, const scldpc_stream_cfg_t *cfg,
-                                const scldpc_stream_out_t *out, void *workspace_dev, size_t workspace_bytes,
-                                long long *iters_launched_host, void *stream)
+extern "C" size_t scldpc_bp_stream_caps_workspace_bytes(const scldpc_dims_t *d)
+{
+    if (check_dims(d)) return 0;
+    return carve(d, SCLDPC_F_STREAM | F_CAPS_WS, nullptr, nullptr);
+}
+
+// Frame stream of scldpc_bp_stream (n_caps == 0: `out` holds the [G][B] results) or scldpc_bp_stream_caps (n_caps >= 1:
+// `out` holds iters [G][B] and the [K][G][B] statistics; the caps are validated by the caller).
+static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const scldpc_stream_cfg_t *cfg, const int32_t *caps,
+                          int n_caps, const scldpc_stream_out_t *out, void *workspace_dev, size_t workspace_bytes,
+                          long long *iters_launched_host, void *stream)
 {
     int rc = check_dims(d);
     if (rc) return rc;
@@ -613,7 +627,7 @@ extern "C" int scldpc_bp_stream(const scldpc_dims_t *d, const scldpc_batch_t *b,
     // SCLDPC_F_MESSAGES selects the message-passing sweeps (the implementation of record); the default is the node-state
     // formulation of bp_node_kernels.cu, which yields the same erased set at every iteration with ~6x less HBM traffic
     const bool node = !(cfg->flags & SCLDPC_F_MESSAGES);
-    const uint32_t wflags = SCLDPC_F_STREAM | (cfg->flags & SCLDPC_F_MESSAGES);
+    const uint32_t wflags = SCLDPC_F_STREAM | (cfg->flags & SCLDPC_F_MESSAGES) | (n_caps > 0 ? F_CAPS_WS : 0u);
     const size_t need = carve(d, wflags, nullptr, nullptr);
     if (workspace_bytes < need) return fail(SCLDPC_ENOMEM, "workspace too small: %zu < %zu bytes", workspace_bytes, need);
     if ((rc = have_device())) return rc;
@@ -638,6 +652,9 @@ extern "C" int scldpc_bp_stream(const scldpc_dims_t *d, const scldpc_batch_t *b,
     p.max_it = INT_MAX; p.first_iter = 0; p.stall_at_first = 1;
     p.frames_per_graph = cfg->frames_per_graph; p.seed = cfg->seed; p.first_graph = cfg->first_graph_id;
     p.stream_cap = cfg->max_it > 0 ? cfg->max_it : 0;
+    p.n_caps = n_caps;
+    for (int k = 0; k < n_caps; k++) p.caps[k] = caps[k];
+    if (n_caps > 0) p.stream_cap = caps[n_caps - 1] > 0 ? caps[n_caps - 1] : INT_MAX;
     p.s_iters = out->iters_dev; p.s_residual = out->residual_dev; p.s_blocks_err = out->blocks_err_dev;
     p.s_erasures_exp = out->erasures_exp_dev; p.s_blocks_err_exp = out->blocks_err_exp_dev;
     p.vn_reverse = env_int("SCLDPC_VN_REVERSE", 1, 0, 1);
@@ -670,6 +687,10 @@ extern "C" int scldpc_bp_stream(const scldpc_dims_t *d, const scldpc_batch_t *b,
         CU(cudaMemsetAsync(p.nl_ovf, 0, sizeof(int) * (size_t)p.G * 2, st));
         CU(cudaMemsetAsync(p.swept, 0, sizeof(long long) * (size_t)p.G * 2, st));        // instrumented builds only
         CU(cudaMemsetAsync(p.pos_er, 0, sizeof(u64) * (size_t)p.G * d->L * p.W, st));
+        if (n_caps > 0) {
+            CU(cudaMemsetAsync(p.lane_ck, 0, sizeof(int) * (size_t)p.G * p.lanes, st));
+            CU(cudaMemsetAsync(p.pause_mask, 0, sizeof(u64) * (size_t)p.G * p.W, st));
+        }
         bp_launch_node_tables(p, st);
     } else {
         CU(cudaMemsetAsync(p.c2v, 0xFF, sizeof(u128) * (size_t)p.G * p.nk * d->dc * ch, st));
@@ -754,6 +775,35 @@ extern "C" int scldpc_bp_stream(const scldpc_dims_t *d, const scldpc_batch_t *b,
     }
     if (iters_launched_host) *iters_launched_host = it;
     return 0;
+}
+
+// Full BP (unlimited iterations) over a stream of cfg->frames_per_graph frames per graph with lane recycling.
+extern "C" int scldpc_bp_stream(const scldpc_dims_t *d, const scldpc_batch_t *b, const scldpc_stream_cfg_t *cfg,
+                                const scldpc_stream_out_t *out, void *workspace_dev, size_t workspace_bytes,
+                                long long *iters_launched_host, void *stream)
+{
+    return bp_stream_impl(d, b, cfg, nullptr, 0, out, workspace_dev, workspace_bytes, iters_launched_host, stream);
+}
+
+// The same stream with checkpoints at the caps of an ascending list (include/scldpc.h).
+extern "C" int scldpc_bp_stream_caps(const scldpc_dims_t *d, const scldpc_batch_t *b, const scldpc_stream_cfg_t *cfg,
+                                     const int32_t *caps_host, int n_caps, const scldpc_stream_caps_out_t *out,
+                                     void *workspace_dev, size_t workspace_bytes, long long *iters_launched_host, void *stream)
+{
+    if (n_caps < 1 || n_caps > SCLDPC_MAX_CAPS) return fail(SCLDPC_EINVAL, "n_caps must be in [1, %d], got %d", SCLDPC_MAX_CAPS, n_caps);
+    if (!caps_host) return fail(SCLDPC_EINVAL, "caps_host is NULL");
+    for (int k = 0; k < n_caps; k++) {
+        const bool unlimited_last = k == n_caps - 1 && caps_host[k] <= 0;
+        if (!unlimited_last && caps_host[k] < 1) return fail(SCLDPC_EINVAL, "cap %d is %d: caps must be >= 1 (only the last may be <= 0, unlimited)", k, caps_host[k]);
+        if (k > 0 && !unlimited_last && caps_host[k] <= caps_host[k - 1])
+            return fail(SCLDPC_EINVAL, "caps must be strictly ascending: cap %d (%d) <= cap %d (%d)", k, caps_host[k], k - 1, caps_host[k - 1]);
+    }
+    if (!cfg) return fail(SCLDPC_EINVAL, "bad stream configuration");
+    if (cfg->max_it != 0) return fail(SCLDPC_EINVAL, "cfg->max_it must be 0 with caps: the caps replace it");
+    if (cfg->flags & SCLDPC_F_MESSAGES) return fail(SCLDPC_EINVAL, "frame streams with caps need the node-state sweeps (no SCLDPC_F_MESSAGES)");
+    if (!out) return fail(SCLDPC_EINVAL, "output pointer is NULL");
+    const scldpc_stream_out_t o{out->iters_dev, out->residual_dev, out->blocks_err_dev, out->erasures_exp_dev, out->blocks_err_exp_dev};
+    return bp_stream_impl(d, b, cfg, caps_host, n_caps, &o, workspace_dev, workspace_bytes, iters_launched_host, stream);
 }
 
 // first_window / n_windows: the windows [first_window, first_window + n_windows) of the chain (n_windows < 0: to the end).

@@ -4,6 +4,8 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include "scldpc.h"
+
 typedef unsigned long long u64;
 typedef ulonglong2 u128;   // one 16-byte chunk = 128 bit-sliced frames
 
@@ -300,6 +302,12 @@ struct BpParams {
     int stall_at_first;       // 1: the stall test is meaningful at first_iter (the sweep covers all n VNs)
     int row;                  // trajectory row written by this iteration (-1: none)
     long long win_edges;      // edge updates of one iteration of the current sweep ranges
+    // frame streams with checkpoints (scldpc_bp_stream_caps): a frame that reaches caps[k] (k < n_caps-1) pauses until the
+    // harvest, which records its statistics into slot k and lets it continue; stream_cap is the last cap (INT_MAX: unlimited)
+    int n_caps;               // 0: no checkpoints
+    int caps[SCLDPC_MAX_CAPS];
+    int *lane_ck;             // [G][lanes] index of the next checkpoint of the lane's frame
+    u64 *pause_mask;          // [G][W] lanes paused at a checkpoint, waiting for the harvest (left active, not in done_mask)
 };
 
 // graph handled by block coordinate b of a grid that is sized by the list of graphs still decoding

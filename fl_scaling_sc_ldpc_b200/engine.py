@@ -366,12 +366,32 @@ class StreamResult:
     edge_updates: int = 0
 
 
+@dataclass
+class StreamCapsResult:
+    """Per-frame outputs of ``decode_bp_stream(..., caps=...)``: ``iters`` [n_graphs][frames_per_graph] under the largest cap
+    (under cap ``caps[k]`` a frame takes ``min(iters, caps[k])`` iterations), the statistics [K][n_graphs][frames_per_graph],
+    slot k being what ``decode_bp_stream(..., max_it=caps[k])`` returns."""
+    caps: tuple
+    iters: np.ndarray
+    residual: np.ndarray
+    blocks_err: np.ndarray
+    erasures_exp: np.ndarray
+    blocks_err_exp: np.ndarray
+    iters_launched: int = 0
+    edge_updates: int = 0
+
+
 def decode_bp_stream(fb: FrameBatch, frames_per_graph: int, eps, seed: int, first_graph_id: int = 0, is_term: bool = True,
                      doping_points=(), harvest_every: int = 0, exp_all: bool = False, collect: bool = True, max_it: int = 0,
-                     messages: bool | None = None):
+                     messages: bool | None = None, caps=None):
     """Full BP (unlimited, or at most ``max_it`` iterations per frame) over a stream of ``frames_per_graph`` frames per
     graph with lane recycling (``scldpc_bp_stream``).  Frame f of graph g is the channel realisation ``generate_erasures(..., first_frame=...)``
-    puts in lane f - first_frame; the graphs are the ones resident in ``fb`` (``fb.n_frames`` lanes are used)."""
+    puts in lane f - first_frame; the graphs are the ones resident in ``fb`` (``fb.n_frames`` lanes are used).
+
+    ``caps``: strictly ascending iteration caps (at most 16, each >= 1; the last may be <= 0, unlimited) in place of
+    ``max_it``.  One decode up to the largest cap gives the results of every cap (``scldpc_bp_stream_caps``): a
+    ``StreamCapsResult``, or with ``collect=False`` the device tensors (iters [G][B], statistics [4][K][G][B]) and the
+    iterations launched."""
     L = _lib.lib()
     G, B = fb.n_graphs, int(frames_per_graph)
     eps_arr = np.full(G, float(eps)) if np.ndim(eps) == 0 else np.asarray(eps, np.float64)
@@ -386,6 +406,11 @@ def decode_bp_stream(fb: FrameBatch, frames_per_graph: int, eps, seed: int, firs
     a_h, a_sp, a_sc = arr(hard), arr(soft_p), arr(soft_c)
     ptr = lambda a: a.ctypes.data_as(ctypes.c_void_p).value
     flags = (F_TERMINATED if is_term else 0) | (F_EXP_ALL if exp_all else 0) | _sweep_flags("SCLDPC_STREAM_NODE", messages)
+    if caps is not None:
+        # the library validates the list; max_it goes through unchanged so that a combination with caps is rejected there too
+        cfg = _lib.StreamCfg(B, int(harvest_every), flags, len(hard), len(soft_p), ptr(eps_arr), ptr(a_h), ptr(a_sp), ptr(a_sc),
+                             int(seed), int(first_graph_id), int(max_it))
+        return _decode_bp_stream_caps(fb, cfg, caps, collect)
     cfg = _lib.StreamCfg(B, int(harvest_every), flags, len(hard), len(soft_p), ptr(eps_arr), ptr(a_h), ptr(a_sp), ptr(a_sc),
                          int(seed), int(first_graph_id), max(0, int(max_it)))
     res = torch.zeros((5, G, B), dtype=torch.int32, device=fb.device)
@@ -405,6 +430,32 @@ def decode_bp_stream(fb: FrameBatch, frames_per_graph: int, eps, seed: int, firs
     r = res.cpu().numpy()
     return StreamResult(r[0], r[1], r[2], r[3], r[4], iters_launched=launched.value,
                         edge_updates=int(r[0].astype(np.int64).sum()) * 2 * fb.ens.E)
+
+
+def _decode_bp_stream_caps(fb: FrameBatch, cfg, caps, collect: bool):
+    L = _lib.lib()
+    G, B = fb.n_graphs, int(cfg.frames_per_graph)
+    caps_arr = np.ascontiguousarray([int(c) for c in caps], np.int32)
+    K = len(caps_arr)
+    iters = torch.zeros((G, B), dtype=torch.int32, device=fb.device)
+    stats = torch.zeros((4, max(K, 1), G, B), dtype=torch.int32, device=fb.device)
+    out = _lib.StreamCapsOut(iters.data_ptr(), *[stats[i].data_ptr() for i in range(4)])
+    need = L.scldpc_bp_stream_caps_workspace_bytes(ctypes.byref(fb.dims))
+    if need == 0:
+        raise _lib.ScldpcError(L.scldpc_last_error().decode())
+    if fb._ws is None or fb._ws.numel() < need:
+        fb._ws = None
+        fb._ws = torch.empty(need, dtype=torch.uint8, device=fb.device)
+    launched = ctypes.c_longlong(0)
+    _lib.check(L.scldpc_bp_stream_caps(ctypes.byref(fb.dims), ctypes.byref(fb.cbatch), ctypes.byref(cfg),
+                                       caps_arr.ctypes.data_as(ctypes.c_void_p), K, ctypes.byref(out),
+                                       ctypes.c_void_p(fb._ws.data_ptr()), ctypes.c_size_t(fb._ws.numel()), ctypes.byref(launched),
+                                       _stream()))
+    if not collect:
+        return iters, stats, launched.value
+    it, st = iters.cpu().numpy(), stats.cpu().numpy()
+    return StreamCapsResult(tuple(int(c) for c in caps_arr), it, st[0], st[1], st[2], st[3], iters_launched=launched.value,
+                            edge_updates=int(it.astype(np.int64).sum()) * 2 * fb.ens.E)
 
 
 def decode_host(ens: Ensemble, vn_cn: np.ndarray, erased: np.ndarray, W: int = 0, max_it: int = UNLIMITED, init_it: int = 0,

@@ -199,6 +199,25 @@ int scldpc_bp_stream(const scldpc_dims_t *d, const scldpc_batch_t *b, const scld
                      const scldpc_stream_out_t *out, void *workspace_dev, size_t workspace_bytes,
                      long long *iters_launched_host, void *stream);
 
+/* Frame streams with checkpoints: one decode yields the results of every iteration cap of an ascending list.
+ * On the BEC, flooding BP from the channel erasures is monotone and a stall is a fixed point, so the erased set a frame has
+ * under cap T is the erased set of the unlimited decoder after min(T, stop) iterations.  A frame that reaches caps_host[k]
+ * (k < n_caps-1) pauses until the next harvest, which records its statistics into slot k and lets it continue; when it
+ * stops for good, its final statistics fill the slots it has not reached.  Slot k therefore equals a scldpc_bp_stream call
+ * with cfg->max_it = caps_host[k], frame for frame (its iteration counts are min(iters_dev, caps_host[k])).
+ * caps_host: 1 <= n_caps <= SCLDPC_MAX_CAPS strictly ascending values >= 1; only the last may be <= 0 (unlimited).
+ * cfg->max_it must be 0 and SCLDPC_F_MESSAGES is not supported (node-state sweeps only).  The workspace comes from
+ * scldpc_bp_stream_caps_workspace_bytes. */
+#define SCLDPC_MAX_CAPS 16
+typedef struct {
+    int32_t *iters_dev;                 /* [G][B] iterations under the largest cap                               */
+    int32_t *residual_dev, *blocks_err_dev, *erasures_exp_dev, *blocks_err_exp_dev;   /* [K][G][B] each      */
+} scldpc_stream_caps_out_t;
+size_t scldpc_bp_stream_caps_workspace_bytes(const scldpc_dims_t *d);
+int scldpc_bp_stream_caps(const scldpc_dims_t *d, const scldpc_batch_t *b, const scldpc_stream_cfg_t *cfg,
+                          const int32_t *caps_host, int n_caps, const scldpc_stream_caps_out_t *out,
+                          void *workspace_dev, size_t workspace_bytes, long long *iters_launched_host, void *stream);
+
 /* scldpc_bp_stream with HOST buffers: graph tables vn_cn_host [G][n][dv] in, per-frame results int32
  * [G][frames_per_graph] out (any may be NULL); channel realisations are drawn on the device. */
 int scldpc_stream_host(const scldpc_dims_t *d, const int32_t *vn_cn_host, const scldpc_stream_cfg_t *cfg,
