@@ -18,8 +18,6 @@
 // VN is left" per lane (warp shuffles -> shared memory -> one atomicOr per block and word), and the last block of
 // the VN sweep (atomic ticket) retires lanes: NumErasures == 0, NumErasures == NumErasuresPrec (messages are
 // monotone, so equal counts <=> no VN resolved) or the iteration cap (BP_FULL.c:1044-1065).
-#include <cooperative_groups.h>
-
 #include <cstdlib>
 
 #include "common.cuh"
@@ -182,8 +180,8 @@ __global__ void __launch_bounds__(256) bp_cn_sweep_kernel(BpParams p)
 // ------------------------------------------------------------------------------------------------------------
 // variable-node sweep + decision + stop flags
 // ------------------------------------------------------------------------------------------------------------
-// TICKET: the last block to finish (atomic ticket) retires the lanes; otherwise the caller does it after a grid-wide sync
-template <int DV, bool TRAJ, bool FREEZE, bool TICKET>
+// the last block to finish (atomic ticket) retires the lanes
+template <int DV, bool TRAJ, bool FREEZE>
 __device__ __forceinline__ void bp_vn_sweep_body(const BpParams &p, const int g)
 {
     __shared__ int s_cnt[TRAJ ? SCLDPC_MAX_LANES : 1];
@@ -268,14 +266,12 @@ __device__ __forceinline__ void bp_vn_sweep_body(const BpParams &p, const int g)
         for (int i = threadIdx.x; i < p.lanes; i += blockDim.x)
             if (s_cnt[i]) atomicAdd(p.cnt_dvn + ((size_t)g * SCLDPC_CNT_SLOTS + (blockIdx.x % SCLDPC_CNT_SLOTS)) * p.lanes + i, s_cnt[i]);
     __threadfence();
-    if (TICKET) {
-        __syncthreads();
-        if (threadIdx.x == 0) s_last = (atomicAdd(p.ticket + g, 1u) == gridDim.x - 1);
-        __syncthreads();
-        if (s_last) {
-            __threadfence();
-            bp_retire_lanes<TRAJ>(p, g);
-        }
+    __syncthreads();
+    if (threadIdx.x == 0) s_last = (atomicAdd(p.ticket + g, 1u) == gridDim.x - 1);
+    __syncthreads();
+    if (s_last) {
+        __threadfence();
+        bp_retire_lanes<TRAJ>(p, g);
     }
 }
 
@@ -284,35 +280,7 @@ __global__ void __launch_bounds__(256) bp_vn_sweep_kernel(BpParams p)
 {
     const int g = blockIdx.y;
     if (ld_cg(p.alive + g) == 0) return;
-    bp_vn_sweep_body<DV, TRAJ, FREEZE, true>(p, g);
-}
-
-// ------------------------------------------------------------------------------------------------------------
-// persistent window kernel: all iterations of one window in one cooperative launch
-// ------------------------------------------------------------------------------------------------------------
-// A window of a few positions is a few tens of microseconds of work per sweep, so two launches per iteration (plus a
-// host round trip whenever the cap is large) leave the GPU waiting.  This kernel keeps one resident grid for the whole
-// window: CN sweep, grid sync, VN sweep + flag reduction, grid sync, block 0 of each graph retires lanes, grid sync --
-// until every frame of every graph has stopped or the window's cap is reached.  Same device code as the two-launch
-// path (bp_cn_sweep_body / bp_vn_sweep_body with FREEZE), so results are identical.
-template <int DV, int DC>
-__global__ void __launch_bounds__(256) bp_window_persistent_kernel(BpParams p0, int num_it)
-{
-    cooperative_groups::grid_group grid = cooperative_groups::this_grid();
-    const int g = blockIdx.y;
-    BpParams p = p0;
-    for (int it = 0; it < num_it; it++) {
-        if (ld_cg(p.alive_total) == 0) break;                  // uniform: written before the last grid sync
-        p.iter = it;
-        p.first_iter = (it == 0);
-        const bool live = ld_cg(p.alive + g) != 0;
-        if (live && p.c1 > p.c0) bp_cn_sweep_body<DC, false, true>(p, g);
-        grid.sync();
-        if (live) bp_vn_sweep_body<DV, false, true, false>(p, g);
-        grid.sync();
-        if (live && blockIdx.x == 0) bp_retire_lanes<false>(p, g);
-        grid.sync();
-    }
+    bp_vn_sweep_body<DV, TRAJ, FREEZE>(p, g);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -519,36 +487,12 @@ __global__ void bp_lane_final_kernel(BpParams p, BpFinalOut o)
 // ------------------------------------------------------------------------------------------------------------
 // host-side launchers
 // ------------------------------------------------------------------------------------------------------------
-static int g_num_sms = 0;
-static int num_sms()
-{
-    if (!g_num_sms) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev);
-        if (g_num_sms <= 0) g_num_sms = 148;
-    }
-    return g_num_sms;
-}
-
-// grid.x for a grid-stride sweep over `items` threads-worth of work replicated over G graphs:
-// a whole number of waves of the machine (multiples of the SM count), capped by the work available.
-static dim3 sweep_grid(long long items, int G, int block, int blocks_per_sm)
-{
-    long long need = (items + block - 1) / block;
-    long long per_graph = (long long)num_sms() * blocks_per_sm;   // each graph can fill the machine on its own
-    (void)G;
-    long long gx = need < per_graph ? need : per_graph;
-    if (gx < 1) gx = 1;
-    return dim3((unsigned)gx, (unsigned)G, 1);
-}
-
 template <int DV, int DC>
-static void launch_iteration(const BpParams &p, bool traj, bool freeze, cudaStream_t st, int blocks_per_sm)
+static void launch_iteration(const BpParams &p, bool traj, bool freeze, cudaStream_t st)
 {
     const int block = 256;
-    dim3 gc = sweep_grid((long long)(p.c1 - p.c0) << p.chunk_shift, p.G, block, blocks_per_sm);
-    dim3 gv = sweep_grid((long long)(p.v1 - p.v0) << p.chunk_shift, p.G, block, blocks_per_sm);
+    dim3 gc = sweep_grid((long long)(p.c1 - p.c0) << p.chunk_shift, p.G, block, SWEEP_BLOCKS_PER_SM);
+    dim3 gv = sweep_grid((long long)(p.v1 - p.v0) << p.chunk_shift, p.G, block, SWEEP_BLOCKS_PER_SM);
     const bool sample = g_prof.sample_every > 0 && g_prof.n_samples < g_prof.max_samples && (p.iter % g_prof.sample_every) == 0;
     cudaEvent_t *ev = sample ? g_prof.ev + 3 * g_prof.n_samples : nullptr;
     if (sample) cudaEventRecord(ev[0], st);
@@ -580,53 +524,9 @@ static void launch_finalize(const BpParams &p, const BpFinalOut &o, cudaStream_t
     bp_lane_final_kernel<<<dim3((p.lanes + 127) / 128, p.G), 128, 0, st>>>(p, o);
 }
 
-// dispatch on the compile-time degrees
-#define SCLDPC_DISPATCH(dv, dc, CALL)                                  \
-    do {                                                               \
-        if ((dv) == 4 && (dc) == 8) { CALL(4, 8); }                    \
-        else if ((dv) == 3 && (dc) == 6) { CALL(3, 6); }               \
-        else if ((dv) == 5 && (dc) == 10) { CALL(5, 10); }             \
-        else if ((dv) == 3 && (dc) == 9) { CALL(3, 9); }               \
-        else if ((dv) == 4 && (dc) == 12) { CALL(4, 12); }             \
-        else return -1;                                                \
-    } while (0)
-
-template <int DV, int DC>
-static int launch_window_persistent(const BpParams &p, int num_it, cudaStream_t st)
+int bp_launch_iteration(int dv, int dc, const BpParams &p, bool traj, bool freeze, cudaStream_t st)
 {
-    static int resident = 0;
-    if (!resident) {
-        int occ = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, bp_window_persistent_kernel<DV, DC>, 256, 0) != cudaSuccess || occ < 1) return -2;
-        resident = occ * num_sms();
-    }
-    if (p.G > resident) return -2;
-    const long long items = (long long)((p.v1 - p.v0) > (p.c1 - p.c0) ? (p.v1 - p.v0) : (p.c1 - p.c0)) << p.chunk_shift;
-    long long gx = resident / p.G, need = (items + 255) / 256;
-    if (gx > need) gx = need;
-    if (gx < 1) gx = 1;
-    BpParams q = p;
-    void *args[2] = {&q, &num_it};
-    g_prof.launches += 1;
-    if (cudaLaunchCooperativeKernel((void *)bp_window_persistent_kernel<DV, DC>, dim3((unsigned)gx, (unsigned)p.G), dim3(256), args, 0, st) != cudaSuccess) {
-        cudaGetLastError();
-        return -2;
-    }
-    return 0;
-}
-
-// all iterations of one window (at most num_it) in one cooperative launch; -2: not available, use the two-launch path
-int bp_launch_window_persistent(int dv, int dc, const BpParams &p, int num_it, cudaStream_t st)
-{
-#define CALL_WP(A, B) return launch_window_persistent<A, B>(p, num_it, st)
-    SCLDPC_DISPATCH(dv, dc, CALL_WP);
-#undef CALL_WP
-    return 0;
-}
-
-int bp_launch_iteration(int dv, int dc, const BpParams &p, bool traj, bool freeze, cudaStream_t st, int blocks_per_sm)
-{
-#define CALL_IT(A, B) launch_iteration<A, B>(p, traj, freeze, st, blocks_per_sm)
+#define CALL_IT(A, B) launch_iteration<A, B>(p, traj, freeze, st)
     SCLDPC_DISPATCH(dv, dc, CALL_IT);
 #undef CALL_IT
     return 0;

@@ -30,8 +30,6 @@
 // derived statistic stay bit-identical; the ride-along iteration costs about 1/350 of the work.
 //
 // Useful work is still accounted as the reference's: 2E edge updates per frame-iteration.
-#include <cstdlib>
-
 #include "common.cuh"
 
 // NS_VARIANT: timing experiments only (tools/build_variants.sh); bits: 1 = ld.cg gathers instead of ld.nc.L1::no_allocate
@@ -501,16 +499,6 @@ __global__ void ns_cn_row_kernel(BpParams p)
 // ------------------------------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------------------------------
-template <typename K>
-static int resident_blocks_ns(K kernel, int block)
-{
-    int occ = 0, dev = 0, sms = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, block, 0) != cudaSuccess || occ < 1) occ = 2;
-    return occ * (sms > 0 ? sms : 148);
-}
-
 // every graph gets enough blocks to fill the machine on its own (blocks of finished graphs return at once); the same
 // geometry for every launch of a stream call, because a warp replays the region it wrote itself
 template <int DV, int DC>
@@ -519,7 +507,7 @@ static dim3 node_grid(const BpParams &p)
     const int block = 32 * NS_WARPS;
     static int res = 0;
     if (!res) {
-        res = resident_blocks_ns(ns_iter_kernel<DV, DC, false>, block);
+        res = resident_blocks(ns_iter_kernel<DV, DC, false>, block);
         if (res > NS_MAX_BLOCKS) res = NS_MAX_BLOCKS;
     }
     long long need = (((long long)p.cn_pos_lim * p.cns_pos << p.chunk_shift) + block - 1) / block;
@@ -535,11 +523,11 @@ static void launch_node_iteration(const BpParams &p, bool after_harvest, cudaStr
     cudaEvent_t *ev = sample ? g_prof.ev + 3 * g_prof.n_samples : nullptr;
     if (sample) cudaEventRecord(ev[0], st);
     g_prof.launches += 1;
-    static const bool pdl = getenv("SCLDPC_NO_PDL") == nullptr;
     // the first launch after a harvest follows ordinary kernels: full serialisation there
-    if (p.n_caps > 0) launch_pdl(ns_iter_kernel<DV, DC, true, true>, grid, block, st, pdl && !after_harvest && !sample, p);
-    else if (p.stream_cap > 0) launch_pdl(ns_iter_kernel<DV, DC, true>, grid, block, st, pdl && !after_harvest && !sample, p);
-    else launch_pdl(ns_iter_kernel<DV, DC, false>, grid, block, st, pdl && !after_harvest && !sample, p);
+    const bool pdl = !after_harvest && !sample;
+    if (p.n_caps > 0) launch_pdl(ns_iter_kernel<DV, DC, true, true>, grid, block, st, pdl, p);
+    else if (p.stream_cap > 0) launch_pdl(ns_iter_kernel<DV, DC, true>, grid, block, st, pdl, p);
+    else launch_pdl(ns_iter_kernel<DV, DC, false>, grid, block, st, pdl, p);
     if (sample) {
         cudaEventRecord(ev[1], st);
         cudaEventRecord(ev[2], st);                             // one kernel per iteration: the second interval is empty
@@ -550,36 +538,29 @@ static void launch_node_iteration(const BpParams &p, bool after_harvest, cudaStr
 // one iteration of every graph's frame stream; after_harvest: the launch follows the harvest kernels
 int bp_launch_node_iteration(int dv, int dc, const BpParams &p, bool after_harvest, cudaStream_t st)
 {
-    if (dv == 4 && dc == 8) launch_node_iteration<4, 8>(p, after_harvest, st);
-    else if (dv == 3 && dc == 6) launch_node_iteration<3, 6>(p, after_harvest, st);
-    else if (dv == 5 && dc == 10) launch_node_iteration<5, 10>(p, after_harvest, st);
-    else if (dv == 3 && dc == 9) launch_node_iteration<3, 9>(p, after_harvest, st);
-    else if (dv == 4 && dc == 12) launch_node_iteration<4, 12>(p, after_harvest, st);
-    else return -1;
+#define CALL_NI(A, B) launch_node_iteration<A, B>(p, after_harvest, st)
+    SCLDPC_DISPATCH(dv, dc, CALL_NI);
+#undef CALL_NI
     return 0;
 }
 
-static dim3 node_grid_any(int dv, int dc, const BpParams &p)
-{
-    if (dv == 4 && dc == 8) return node_grid<4, 8>(p);
-    if (dv == 3 && dc == 6) return node_grid<3, 6>(p);
-    if (dv == 5 && dc == 10) return node_grid<5, 10>(p);
-    if (dv == 3 && dc == 9) return node_grid<3, 9>(p);
-    return node_grid<4, 12>(p);
-}
-
 // p.iter = the iteration that runs next; both planes equal and all lists empty afterwards
-void bp_launch_node_settle(int dv, int dc, const BpParams &p, cudaStream_t st)
+int bp_launch_node_settle(int dv, int dc, const BpParams &p, cudaStream_t st)
 {
+    dim3 grid;
+#define CALL_NG(A, B) grid = node_grid<A, B>(p)
+    SCLDPC_DISPATCH(dv, dc, CALL_NG);
+#undef CALL_NG
     g_prof.launches += 2;
-    ns_settle_kernel<<<node_grid_any(dv, dc, p), 32 * NS_WARPS, 0, st>>>(p);
+    ns_settle_kernel<<<grid, 32 * NS_WARPS, 0, st>>>(p);
     ns_settle_done_kernel<<<graphs_in_grid(p), 256, 0, st>>>(p);
+    return 0;
 }
 
 void bp_launch_node_arm(const BpParams &p, cudaStream_t st)
 {
     static int res = 0;
-    if (!res) res = resident_blocks_ns(ns_arm_kernel, 256);
+    if (!res) res = resident_blocks(ns_arm_kernel, 256);
     long long need = ((long long)p.n + ARM_ROWS - 1) / ARM_ROWS;
     long long gx = need < res ? need : res;
     g_prof.launches += 1;

@@ -354,9 +354,9 @@ __global__ void __launch_bounds__(256, TRAJ ? 3 : 4) bp_vn_wave_kernel(BpParams 
 template <int DV, bool ARM>
 __global__ void __launch_bounds__(256, ARM ? 3 : 4) bp_vn_stream_kernel(BpParams p)
 {
-    // The CN sweep walks graphs and positions upwards; this sweep walks them downwards (vn_reverse), so each sweep starts on
-    // the rows the other one touched last -- its first gathers (and the x / y rows) are L2 hits instead of HBM reads.
-    const int g = graph_of(p, p.vn_reverse ? gridDim.y - 1 - blockIdx.y : blockIdx.y);
+    // The CN sweep walks graphs and positions upwards; this sweep walks them downwards, so each sweep starts on the rows
+    // the other one touched last -- its first gathers (and the x / y rows) are L2 hits instead of HBM reads.
+    const int g = graph_of(p, gridDim.y - 1 - blockIdx.y);
     if (ld_cg(p.alive + g) == 0) return;
     __shared__ u64 s_new[SCLDPC_MAX_WORDS], s_er[SCLDPC_MAX_WORDS];
     __shared__ int s_last;
@@ -382,7 +382,8 @@ __global__ void __launch_bounds__(256, ARM ? 3 : 4) bp_vn_stream_kernel(BpParams
         const bool work = lane_work && idx < items;
         u128 changed = zero128(), xn = zero128(), yn = zero128(), xo = zero128(), yo = zero128();
         u128 out[DV];
-        const int v = p.vn_reverse ? p.n - 1 - (idx >> p.chunk_shift) : (idx >> p.chunk_shift);
+        // unsigned: the row offsets widen to 64 bits for free (a sign-extended copy of an int row spills at DV = 5, ARM)
+        const unsigned v = p.n - 1 - (idx >> p.chunk_shift);
         if (work) {
             int s[DV];
             load_row<DV>(vn_slot + (size_t)v * DV, s);
@@ -639,14 +640,10 @@ __global__ void bp_stream_harvest_kernel(BpParams p, int exp_all)
         const int nn = next0 + s_rank[W];
         p.next_frame[g] = nn < B ? nn : B;
         if (!any) { p.alive[g] = 0; atomicSub(p.alive_total, 1); }
-        // hint for the host's harvest period: mean iterations per harvested frame of the slowest graph still decoding
+        // hint for the host's harvest period: mean iterations per harvested frame of the fastest graph still decoding
         p.h_cum[2 * g] += s_frames;
         p.h_cum[2 * g + 1] += (long long)s_its;
-        if (any && p.h_cum[2 * g] > 0) {
-            const int mean_it = (int)(p.h_cum[2 * g + 1] / p.h_cum[2 * g]);
-            atomicMax(p.alive_total + 1 + p.harvest_parity, mean_it);      // slowest graph still decoding
-            atomicMin(p.alive_total + 4 + p.harvest_parity, mean_it);      // fastest graph still decoding
-        }
+        if (any && p.h_cum[2 * g] > 0) atomicMin(p.alive_total + 1 + p.harvest_parity, (int)(p.h_cum[2 * g + 1] / p.h_cum[2 * g]));
     }
 }
 
@@ -671,18 +668,8 @@ __global__ void bp_stream_init_kernel(BpParams p, int n_lanes_used)
 // ------------------------------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------------------------------
-template <typename K>
-static int resident_blocks(K kernel, int block)
-{
-    int occ = 0, dev = 0, sms = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, block, 0) != cudaSuccess || occ < 1) occ = 2;
-    return occ * (sms > 0 ? sms : 148);
-}
-
 template <int DV, int DC>
-static void launch_wave_iteration(const BpParams &p, bool traj, cudaStream_t st, int waves)
+static void launch_wave_iteration(const BpParams &p, bool traj, cudaStream_t st)
 {
     const int block = 256;
     static int res_cn[2] = {0, 0}, res_vn[2] = {0, 0};
@@ -692,12 +679,11 @@ static void launch_wave_iteration(const BpParams &p, bool traj, cudaStream_t st,
         res_vn[0] = resident_blocks(bp_vn_wave_kernel<DV, false>, block);
         res_vn[1] = resident_blocks(bp_vn_wave_kernel<DV, true>, block);
     }
-    // every graph gets enough blocks to fill the machine on its own (`waves` x the resident block count): blocks
+    // every graph gets enough blocks to fill the machine on its own (one wave: the resident block count): blocks
     // of finished graphs return at once, so the graphs still decoding always have the whole GPU
     auto grid = [&](int resident, long long items_per_graph) {
         long long need = (items_per_graph + block - 1) / block;
-        long long per_graph = (long long)resident * waves;
-        long long gx = need < per_graph ? need : per_graph;
+        long long gx = need < resident ? need : resident;
         return dim3((unsigned)(gx < 1 ? 1 : gx), (unsigned)p.G, 1);
     };
     dim3 gc = grid(res_cn[traj], (long long)p.cn_pos_lim * p.cns_pos << p.chunk_shift);
@@ -718,14 +704,11 @@ static void launch_wave_iteration(const BpParams &p, bool traj, cudaStream_t st,
     }
 }
 
-int bp_launch_wave_iteration(int dv, int dc, const BpParams &p, bool traj, cudaStream_t st, int waves)
+int bp_launch_wave_iteration(int dv, int dc, const BpParams &p, bool traj, cudaStream_t st)
 {
-    if (dv == 4 && dc == 8) launch_wave_iteration<4, 8>(p, traj, st, waves);
-    else if (dv == 3 && dc == 6) launch_wave_iteration<3, 6>(p, traj, st, waves);
-    else if (dv == 5 && dc == 10) launch_wave_iteration<5, 10>(p, traj, st, waves);
-    else if (dv == 3 && dc == 9) launch_wave_iteration<3, 9>(p, traj, st, waves);
-    else if (dv == 4 && dc == 12) launch_wave_iteration<4, 12>(p, traj, st, waves);
-    else return -1;
+#define CALL_WV(A, B) launch_wave_iteration<A, B>(p, traj, st)
+    SCLDPC_DISPATCH(dv, dc, CALL_WV);
+#undef CALL_WV
     return 0;
 }
 
@@ -764,12 +747,9 @@ static void launch_stream_iteration(const BpParams &p, bool arm, cudaStream_t st
 // arm: lanes re-armed by the preceding harvest take their new frames in this iteration's VN sweep
 int bp_launch_stream_iteration(int dv, int dc, const BpParams &p, bool arm, cudaStream_t st)
 {
-    if (dv == 4 && dc == 8) launch_stream_iteration<4, 8>(p, arm, st);
-    else if (dv == 3 && dc == 6) launch_stream_iteration<3, 6>(p, arm, st);
-    else if (dv == 5 && dc == 10) launch_stream_iteration<5, 10>(p, arm, st);
-    else if (dv == 3 && dc == 9) launch_stream_iteration<3, 9>(p, arm, st);
-    else if (dv == 4 && dc == 12) launch_stream_iteration<4, 12>(p, arm, st);
-    else return -1;
+#define CALL_ST(A, B) launch_stream_iteration<A, B>(p, arm, st)
+    SCLDPC_DISPATCH(dv, dc, CALL_ST);
+#undef CALL_ST
     return 0;
 }
 

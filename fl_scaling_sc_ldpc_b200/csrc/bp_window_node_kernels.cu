@@ -19,8 +19,6 @@
 // last one is detected one iteration late as "nothing resolved" and taken off again by the end-of-window kernel, which
 // is the only pass over the VN window (once per window instead of once per iteration).  Frames that stopped keep their
 // bits (FREEZE): resolutions are masked with the frames still iterating.
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace scldpc {
@@ -541,11 +539,7 @@ static dim3 window_grid(const BpParams &p)
     const int block = 32 * NS_WARPS;
     static int res = 0;
     if (!res) {
-        int occ = 0, dev = 0, sms = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, bpw_iter_kernel<DV, DC, false, false>, block, 0) != cudaSuccess || occ < 1) occ = 2;
-        res = occ * (sms > 0 ? sms : 148);
+        res = resident_blocks(bpw_iter_kernel<DV, DC, false, false>, block);
         if (res > NS_MAX_BLOCKS) res = NS_MAX_BLOCKS;
     }
     // the same geometry for every launch of a window (a warp replays the region it wrote itself): a function of the ranges only
@@ -557,41 +551,18 @@ static dim3 window_grid(const BpParams &p)
     return dim3((unsigned)(gx < 1 ? 1 : gx), (unsigned)p.G, 1);
 }
 
-#define SCLDPC_DISPATCH_W(dv, dc, CALL)                                \
-    do {                                                               \
-        if ((dv) == 4 && (dc) == 8) { CALL(4, 8); }                    \
-        else if ((dv) == 3 && (dc) == 6) { CALL(3, 6); }               \
-        else if ((dv) == 5 && (dc) == 10) { CALL(5, 10); }             \
-        else if ((dv) == 3 && (dc) == 9) { CALL(3, 9); }               \
-        else if ((dv) == 4 && (dc) == 12) { CALL(4, 12); }             \
-        else return -1;                                                \
-    } while (0)
-
-static dim3 sweep_grid(long long items, int G, int block, int blocks_per_sm)
-{
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    long long need = (items + block - 1) / block;
-    long long per_graph = (long long)sms * blocks_per_sm;          // each graph can fill the machine on its own
-    long long gx = need < per_graph ? need : per_graph;
-    if (gx < 1) gx = 1;
-    return dim3((unsigned)gx, (unsigned)G, 1);
-}
-
 template <int DV, int DC>
-static void launch_window_copy_iteration(const BpParams &p, cudaStream_t st, int blocks_per_sm)
+static void launch_window_copy_iteration(const BpParams &p, cudaStream_t st)
 {
     const int block = 256;
-    dim3 gc = sweep_grid((long long)(p.c1 - p.c0) << p.chunk_shift, p.G, block, blocks_per_sm);
-    dim3 gv = sweep_grid((((long long)(p.v1 - p.v0) << p.chunk_shift) + 3) / 4, p.G, block, blocks_per_sm);   // four rows per thread and trip
+    dim3 gc = sweep_grid((long long)(p.c1 - p.c0) << p.chunk_shift, p.G, block, SWEEP_BLOCKS_PER_SM);
+    dim3 gv = sweep_grid((((long long)(p.v1 - p.v0) << p.chunk_shift) + 3) / 4, p.G, block, SWEEP_BLOCKS_PER_SM);   // four rows per thread and trip
     const bool sample = g_prof.sample_every > 0 && g_prof.n_samples < g_prof.max_samples && (p.iter % g_prof.sample_every) == 0;
     cudaEvent_t *ev = sample ? g_prof.ev + 3 * g_prof.n_samples : nullptr;
     if (sample) cudaEventRecord(ev[0], st);
     g_prof.launches += (p.c1 > p.c0) ? 2 : 1;
     // programmatic dependent launches inside a window / a call; its first kernel follows ordinary ones
-    static const bool pdl_on = getenv("SCLDPC_NO_PDL") == nullptr;
-    const bool pdl = pdl_on && !sample;
+    const bool pdl = !sample;
     if (p.c1 > p.c0) {
         if (p.cn_dis_lim > 0) launch_pdl(bpw_cn_copy_kernel<DV, DC, true>, gc, dim3(block), st, pdl && !p.first_iter, p);
         else launch_pdl(bpw_cn_copy_kernel<DV, DC, false>, gc, dim3(block), st, pdl && !p.first_iter, p);
@@ -612,9 +583,8 @@ static void launch_window_node_iteration(const BpParams &p, cudaStream_t st)
     cudaEvent_t *ev = sample ? g_prof.ev + 3 * g_prof.n_samples : nullptr;
     if (sample) cudaEventRecord(ev[0], st);
     g_prof.launches += 1;
-    static const bool pdl_on = getenv("SCLDPC_NO_PDL") == nullptr;
     // programmatic dependent launches inside a window; its first kernel follows ordinary ones
-    const bool pdl = pdl_on && !sample && !p.first_iter;
+    const bool pdl = !sample && !p.first_iter;
     if (p.traj_node) launch_pdl(bpw_iter_kernel<DV, DC, false, true>, grid, block, st, pdl, p);
     else if (p.cn_dis_lim > 0) launch_pdl(bpw_iter_kernel<DV, DC, true, false>, grid, block, st, pdl, p);
     else launch_pdl(bpw_iter_kernel<DV, DC, false, false>, grid, block, st, pdl, p);
@@ -625,16 +595,16 @@ static void launch_window_node_iteration(const BpParams &p, cudaStream_t st)
     }
 }
 
-int bp_launch_window_node_iteration(int dv, int dc, const BpParams &p, cudaStream_t st, int blocks_per_sm)
+int bp_launch_window_node_iteration(int dv, int dc, const BpParams &p, cudaStream_t st)
 {
     if (!p.win_lists) {
-#define CALL_WC(A, B) launch_window_copy_iteration<A, B>(p, st, blocks_per_sm)
-        SCLDPC_DISPATCH_W(dv, dc, CALL_WC);
+#define CALL_WC(A, B) launch_window_copy_iteration<A, B>(p, st)
+        SCLDPC_DISPATCH(dv, dc, CALL_WC);
 #undef CALL_WC
         return 0;
     }
 #define CALL_WI(A, B) launch_window_node_iteration<A, B>(p, st)
-    SCLDPC_DISPATCH_W(dv, dc, CALL_WI);
+    SCLDPC_DISPATCH(dv, dc, CALL_WI);
 #undef CALL_WI
     return 0;
 }
@@ -645,7 +615,7 @@ int bp_launch_window_node_end(int dv, int dc, const BpParams &p, cudaStream_t st
     if (!p.win_lists) return 0;                                  // the copy variant leaves nothing pending
     dim3 grid;
 #define CALL_WG(A, B) grid = window_grid<A, B>(p)
-    SCLDPC_DISPATCH_W(dv, dc, CALL_WG);
+    SCLDPC_DISPATCH(dv, dc, CALL_WG);
 #undef CALL_WG
     g_prof.launches += 1;
     bpw_window_end_kernel<<<grid, 32 * NS_WARPS, 0, st>>>(p);
@@ -661,12 +631,9 @@ void bp_launch_window_node_traj_init(const BpParams &p, cudaStream_t st)
 // resume: the caller supplied both planes (scldpc_bp_window_range), only the list bookkeeping is reset
 void bp_launch_window_node_init(const BpParams &p, cudaStream_t st, bool resume)
 {
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     g_prof.launches += resume ? 1 : 2;
     bpw_node_reset_kernel<<<p.G, 256, 0, st>>>(p, resume ? 0 : 1);
-    if (!resume) bpw_node_init_kernel<<<sms * 8, 256, 0, st>>>(p);
+    if (!resume) bpw_node_init_kernel<<<num_sms() * 8, 256, 0, st>>>(p);
 }
 
 }  // namespace scldpc

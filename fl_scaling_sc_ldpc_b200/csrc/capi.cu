@@ -13,22 +13,21 @@
 #include "scldpc.h"
 
 namespace scldpc {
-int bp_launch_iteration(int dv, int dc, const BpParams &p, bool traj, bool freeze, cudaStream_t st, int blocks_per_sm);
+int bp_launch_iteration(int dv, int dc, const BpParams &p, bool traj, bool freeze, cudaStream_t st);
 int bp_launch_finalize(int dv, int dc, const BpParams &p, const BpFinalOut &o, cudaStream_t st);
 void bp_launch_init(const BpParams &p, int dv, int dc, int trajectory, int n_frames, cudaStream_t st);
 void bp_launch_window_begin(const BpParams &p, int n_frames, cudaStream_t st);
 void bp_launch_init_ctrl_only(const BpParams &p, int n_frames, cudaStream_t st);
-int bp_launch_window_persistent(int dv, int dc, const BpParams &p, int num_it, cudaStream_t st);
-int bp_launch_wave_iteration(int dv, int dc, const BpParams &p, bool traj, cudaStream_t st, int waves);
+int bp_launch_wave_iteration(int dv, int dc, const BpParams &p, bool traj, cudaStream_t st);
 void bp_launch_wave_init(const BpParams &p, cudaStream_t st);
 int bp_launch_stream_iteration(int dv, int dc, const BpParams &p, bool arm, cudaStream_t st);
 int bp_launch_node_iteration(int dv, int dc, const BpParams &p, bool after_harvest, cudaStream_t st);
-void bp_launch_node_settle(int dv, int dc, const BpParams &p, cudaStream_t st);
+int bp_launch_node_settle(int dv, int dc, const BpParams &p, cudaStream_t st);
 void bp_launch_node_arm(const BpParams &p, cudaStream_t st);
 void bp_launch_node_compact(const BpParams &p, cudaStream_t st);
 void bp_launch_node_alive_list(const BpParams &p, int parity, cudaStream_t st);
 void bp_launch_node_tables(const BpParams &p, cudaStream_t st);
-int bp_launch_window_node_iteration(int dv, int dc, const BpParams &p, cudaStream_t st, int blocks_per_sm);
+int bp_launch_window_node_iteration(int dv, int dc, const BpParams &p, cudaStream_t st);
 void bp_launch_window_node_init(const BpParams &p, cudaStream_t st, bool resume);
 int bp_launch_window_node_end(int dv, int dc, const BpParams &p, cudaStream_t st);
 void bp_launch_window_node_traj_init(const BpParams &p, cudaStream_t st);
@@ -103,8 +102,9 @@ static int check_dims(const scldpc_dims_t *d)
 
 static bool degrees_supported(int dv, int dc)
 {
-    return (dv == 4 && dc == 8) || (dv == 3 && dc == 6) || (dv == 5 && dc == 10) || (dv == 3 && dc == 9) ||
-           (dv == 4 && dc == 12);
+#define PAIR_(A, B, _) || (dv == A && dc == B)
+    return false SCLDPC_DEGREES(PAIR_, _);
+#undef PAIR_
 }
 
 static int have_device()
@@ -151,7 +151,13 @@ struct Carve {
     }
 };
 
-static int env_int(const char *name, int dflt, int lo, int hi);
+// test hook: an integer from the environment, clamped to [lo, hi]
+static int env_int(const char *name, int dflt, int lo, int hi)
+{
+    const char *s = getenv(name);
+    int v = s ? atoi(s) : dflt;
+    return v < lo ? lo : (v > hi ? hi : v);
+}
 
 // regions of the per-warp resolution lists: one per warp of the largest sweep grid (items = nodes x chunks, 256 per block)
 static size_t list_regions(size_t max_nodes, size_t ch)
@@ -311,18 +317,6 @@ static int host_flag(int **out)
     return 0;
 }
 
-static int blocks_per_sm_env()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char *s = getenv("SCLDPC_BLOCKS_PER_SM");
-        v = s ? atoi(s) : 8;
-        if (v < 1) v = 1;
-        if (v > 32) v = 32;
-    }
-    return v;
-}
-
 // ---- graph / channel ------------------------------------------------------------------------------------------
 extern "C" int scldpc_graph_build_tables(const scldpc_dims_t *d, const scldpc_batch_t *b, int32_t *scratch_dev, void *stream)
 {
@@ -480,14 +474,9 @@ extern "C" int scldpc_channel_pack_host(const scldpc_dims_t *d, const uint8_t *e
 }
 
 // ---- decoders -------------------------------------------------------------------------------------------------
-static int env_int(const char *name, int dflt, int lo, int hi)
-{
-    const char *s = getenv(name);
-    int v = s ? atoi(s) : dflt;
-    return v < lo ? lo : (v > hi ? hi : v);
-}
+#define POLL_EVERY 8   // iterations enqueued between two polls of the device's counter of graphs still decoding
 
-// Runs up to `cap` flooding iterations, in chunks.  The device keeps the number of graphs that still have an active
+// Runs up to `cap` flooding iterations, in chunks of POLL_EVERY.  The device keeps the number of graphs that still have an active
 // frame; after each chunk that counter is copied to pinned host memory and the NEXT chunk is enqueued before the
 // host waits for the copy, so the GPU never idles on the host.  Sweeps of a finished graph return at once, so the
 // overshoot (at most two chunks) costs launch latency only.
@@ -501,20 +490,17 @@ static int run_iterations(BpParams *p, int dv, int dc, int cap, bool traj, bool 
         CU(cudaEventCreateWithFlags(&ev[0], cudaEventDisableTiming));
         CU(cudaEventCreateWithFlags(&ev[1], cudaEventDisableTiming));
     }
-    const int bps = blocks_per_sm_env();
-    const int waves = env_int("SCLDPC_WAVES", 1, 1, 16);
-    const int chunk = env_int("SCLDPC_CHUNK", 8, 1, 64);
     int it = 0, nchunk = 0;
     bool pending[2] = {false, false};
     while (it < cap) {
-        const int todo = (cap - it) < chunk ? (cap - it) : chunk;
+        const int todo = (cap - it) < POLL_EVERY ? (cap - it) : POLL_EVERY;
         for (int q = 0; q < todo; q++, it++) {
             p->iter = it;
             p->max_it = cap;
             p->first_iter = (it == 0);
             p->row = traj ? it : -1;
-            if (window_node ? bp_launch_window_node_iteration(dv, dc, *p, st, bps)
-                            : (wave ? bp_launch_wave_iteration(dv, dc, *p, traj, st, waves) : bp_launch_iteration(dv, dc, *p, traj, freeze, st, bps)))
+            if (window_node ? bp_launch_window_node_iteration(dv, dc, *p, st)
+                            : (wave ? bp_launch_wave_iteration(dv, dc, *p, traj, st) : bp_launch_iteration(dv, dc, *p, traj, freeze, st)))
                 return fail(SCLDPC_EINVAL, "unsupported degrees");
         }
         CU_LAUNCHES();
@@ -657,7 +643,6 @@ static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const
     if (n_caps > 0) p.stream_cap = caps[n_caps - 1] > 0 ? caps[n_caps - 1] : INT_MAX;
     p.s_iters = out->iters_dev; p.s_residual = out->residual_dev; p.s_blocks_err = out->blocks_err_dev;
     p.s_erasures_exp = out->erasures_exp_dev; p.s_blocks_err_exp = out->blocks_err_exp_dev;
-    p.vn_reverse = env_int("SCLDPC_VN_REVERSE", 1, 0, 1);
     p.lane_mask = p.fail_mask;                   // frames that stopped without erasures have all-zero counts already
     p.lazy_success = node ? 1 : 0;
     // per-graph channel thresholds and the doping profile
@@ -715,18 +700,14 @@ static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const
     }
     // Harvest period: a harvest costs about as much as two to three iterations (count / pair kernels, channel draws of the
     // re-armed lanes) and a finished frame idles H/2 iterations on average, so the best period is about sqrt(6 x iterations
-    // per frame); measured flat between 3.5 and 10 at M = 10000.  harvest_every <= 0: adapt it to the frames harvested so far (the slowest graph still decoding); > 0: fixed.
+    // per frame); measured flat between 3.5 and 10 at M = 10000.  harvest_every <= 0: adapt it to the frames harvested so far; > 0: fixed.
     const bool adaptive = cfg->harvest_every <= 0;
-    // The period follows the FASTEST graph still decoding (SCLDPC_HARVEST_POLICY=1: the slowest, as in round 1): a harvest
-    // costs every live graph the same, an idle lane costs a fast graph a larger share of its frame.  Measured flat
-    // (profiles/r02h_harvest_period_ab.txt: 5.62 .. 5.82e13 edge-updates/s for constants 25 .. 60 and both policies).
-    const int hc10 = env_int("SCLDPC_HARVEST_C10", 60, 1, 1000);
-    const int h_policy_max = env_int("SCLDPC_HARVEST_POLICY", 0, 0, 1);
-    const bool compact = env_int("SCLDPC_COMPACT", 1, 0, 1) != 0;
-    const bool glists = env_int("SCLDPC_ALIVE_GRIDS", 1, 0, 1) != 0;   // grids sized by the graphs still decoding (A/B switch)   // lane compaction in the tail of a stream (A/B switch)
+    // The period follows the FASTEST graph still decoding: a harvest costs every live graph the same, an idle lane costs a
+    // fast graph a larger share of its frame.  Measured flat (profiles/r02h_harvest_period_ab.txt: 5.62 .. 5.82e13
+    // edge-updates/s for constants 25 .. 60, following the fastest or the slowest graph).
+    constexpr int HARVEST_C10 = 60;                // H = sqrt(HARVEST_C10 / 10 x mean iterations per frame), clamped to [8, 64]
     int H = adaptive ? 16 : cfg->harvest_every;
-    CU(cudaMemsetAsync(p.alive_total + 1, 0, 2 * sizeof(int), st));
-    CU(cudaMemsetAsync(p.alive_total + 4, 0x7f, 2 * sizeof(int), st));
+    CU(cudaMemsetAsync(p.alive_total + 1, 0x7f, 2 * sizeof(int), st));
     CU(cudaMemsetAsync(p.h_cum, 0, sizeof(long long) * 2 * (size_t)p.G, st));
     long long it = 0;
     int nchunk = 0;
@@ -740,16 +721,15 @@ static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const
         const int slot = nchunk & 1;
         p.harvest_parity = slot;
         p.iter = (int)(it & 0x3fffffff);         // the iteration that runs next (its parity names the planes)
-        if (adaptive) {
-            CU(cudaMemsetAsync(p.alive_total + 1 + slot, 0, sizeof(int), st));
-            CU(cudaMemsetAsync(p.alive_total + 4 + slot, 0x7f, sizeof(int), st));
-        }
+        if (adaptive) CU(cudaMemsetAsync(p.alive_total + 1 + slot, 0x7f, sizeof(int), st));
         if (node) bp_launch_node_settle(d->dv, d->dc, p, st);
         bp_launch_count_pairs(d->dv, d->dc, p, st);
         bp_launch_stream_harvest(p, (cfg->flags & SCLDPC_F_EXP_ALL) ? 1 : 0, st);
-        if (node) bp_launch_node_arm(p, st);
-        if (node && compact) bp_launch_node_compact(p, st);
-        if (glists) bp_launch_node_alive_list(p, slot, st);
+        if (node) {
+            bp_launch_node_arm(p, st);
+            bp_launch_node_compact(p, st);
+        }
+        bp_launch_node_alive_list(p, slot, st);
         CU_LAUNCHES();
         CU(cudaMemcpyAsync(hf + 8 * slot, p.alive_total, 8 * sizeof(int), cudaMemcpyDeviceToHost, st));
         CU(cudaEventRecord(ev[slot], st));
@@ -760,15 +740,13 @@ static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const
             CU(cudaEventSynchronize(ev[prev]));
             pending[prev] = false;
             if (hf[8 * prev] == 0) break;
-            if (glists) {                                        // grids of the next chunk: the graphs that were alive at that harvest
-                p.glist = p.glist2 + (size_t)prev * p.G;
-                p.n_glist = hf[8 * prev + 6 + prev];
-                if (p.n_glist < 1 || p.n_glist > p.G) { p.glist = nullptr; p.n_glist = 0; }
-            }
-            int mean_it = hf[8 * prev + 1 + prev];
-            if (!h_policy_max && hf[8 * prev + 4 + prev] != 0x7f7f7f7f) mean_it = hf[8 * prev + 4 + prev];
-            if (adaptive && mean_it > 0) {
-                H = (int)(sqrt(0.1 * hc10 * mean_it) + 0.5);
+            // grids of the next chunk: the graphs that were alive at that harvest
+            p.glist = p.glist2 + (size_t)prev * p.G;
+            p.n_glist = hf[8 * prev + 6 + prev];
+            if (p.n_glist < 1 || p.n_glist > p.G) { p.glist = nullptr; p.n_glist = 0; }
+            const int mean_it = hf[8 * prev + 1 + prev];   // 0x7f7f7f7f: no graph still decoding has harvested a frame yet
+            if (adaptive && mean_it != 0x7f7f7f7f && mean_it > 0) {
+                H = (int)(sqrt(0.1 * HARVEST_C10 * mean_it) + 0.5);
                 H = H < 8 ? 8 : (H > 64 ? 64 : H);
             }
         }
@@ -859,7 +837,7 @@ static int bp_window_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, int W
         p.xb = pending_dev ? reinterpret_cast<u128 *>(pending_dev) : p.y;   // the wave-tracking plane is free in window mode
         // resolution lists pay when few rows change per iteration, i.e. when the window is long against the wave (about 10
         // positions); short windows copy the VN window instead (bp_window_node_kernels.cu)
-        p.win_lists = env_int("SCLDPC_WINDOW_LISTS", (long long)(W + ms) * 2 >= L ? 1 : 0, 0, 1);
+        p.win_lists = (long long)(W + ms) * 2 >= L ? 1 : 0;
         bp_launch_init_ctrl_only(p, d->n_frames, st);
         bp_launch_window_node_init(p, st, resume != 0);
     } else {
@@ -868,10 +846,6 @@ static int bp_window_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, int W
     }
     CU(cudaGetLastError());
     const int win_end = (n_windows < 0 || first_window + (long long)n_windows > nwin) ? nwin : first_window + n_windows;
-    // Opt-in (SCLDPC_PERSISTENT=1): measured on B200 the cooperative kernel is 15-25 % SLOWER than two launches per
-    // iteration (W=3: 81 vs 70 ms, W=10: 275 vs 215 ms for 4 graphs x 1024 frames, L=100, M=10000) -- three grid-wide
-    // syncs per iteration and 2 instead of 3-4 resident blocks per SM cost more than the launches they replace.
-    bool persistent = !node && env_int("SCLDPC_PERSISTENT", 0, 0, 1) != 0;
     for (int posW = first_window; posW < win_end && d->n_frames > 0; posW++) {
         long long c0 = (long long)posW * cp, c1 = c0 + (long long)W * cp;
         if (c1 > cn_clip) c1 = cn_clip;
@@ -891,15 +865,7 @@ static int bp_window_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, int W
         p.win_edges = ce + (v1 - v0) * d->dv;
         bp_launch_window_begin(p, d->n_frames, st);
         const int NumIt = (square && posW == 0) ? cap0 : cap;      // BP_SW.c:699-702
-        // one cooperative launch per window (grid-wide syncs between the sweeps); two launches per iteration otherwise
-        p.max_it = NumIt;
-        p.row = -1;
-        int prc = persistent ? bp_launch_window_persistent(d->dv, d->dc, p, NumIt, st) : -2;
-        if (prc == -1) return fail(SCLDPC_EINVAL, "unsupported degrees");
-        if (prc == -2) {
-            persistent = false;
-            if ((rc = run_iterations(&p, d->dv, d->dc, NumIt, false, true, false, st, nullptr, node))) return rc;
-        }
+        if ((rc = run_iterations(&p, d->dv, d->dc, NumIt, false, true, false, st, nullptr, node))) return rc;
         if (node && bp_launch_window_node_end(d->dv, d->dc, p, st)) return fail(SCLDPC_EINVAL, "unsupported degrees");
     }
     BpFinalOut fo{out->residual_dev, out->blocks_err_dev, out->erasures_exp_dev, out->blocks_err_exp_dev, out->erasures_p1_dev,

@@ -226,8 +226,8 @@ struct BpParams {
     u64 *pos_er;              // [G][L][W] lanes with an erased VN in position p (trajectory mode)
     unsigned *ticket;         // [G]
     int *alive;               // [G] any active lane
-    int *alive_total;         // [8] graphs with an active lane; [1], [2]: largest, [4], [5]: smallest mean iterations per harvested frame
-                              //   among the graphs still decoding (by harvest parity)
+    int *alive_total;         // [8] graphs with an active lane; [1], [2]: smallest mean iterations per harvested frame among the
+                              //   graphs still decoding (by harvest parity); [6], [7]: length of glist2 (by harvest parity)
     long long *h_cum;         // [G][2] frame streams: frames harvested so far and the iterations they took
     int harvest_parity;       // frame streams: which of alive_total[1..2] this harvest reports into
     int *cnt_dvn;             // [G][slots][lanes] newly resolved VNs of this iteration (trajectory mode)
@@ -296,7 +296,6 @@ struct BpParams {
     // per-launch
     int c0, c1, v0, v1;       // CN / VN ranges swept
     int iter;                 // iteration index inside the current loop
-    int vn_reverse;           // stream mode: the VN sweep walks graphs and VNs downwards (see bp_vn_stream_kernel)
     int max_it;               // cap of the current loop
     int first_iter;           // 1: the previous a-posteriori state is "all erased" (NumErasuresPrec = n)
     int stall_at_first;       // 1: the stall test is meaningful at first_iter (the sweep covers all n VNs)
@@ -478,6 +477,51 @@ static void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStre
     const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, args...);
     if (e != cudaSuccess && scldpc::launch_error_slot() == cudaSuccess) scldpc::launch_error_slot() = e;
 }
+
+// ---- compile-time degrees ----------------------------------------------------------------------------------------------
+// The (dv, dc) pairs the decoders are instantiated for: X(DV, DC, arg) once per pair.
+#define SCLDPC_DEGREES(X, arg) X(4, 8, arg) X(3, 6, arg) X(5, 10, arg) X(3, 9, arg) X(4, 12, arg)
+// CALL(DV, DC) for the pair (dv, dc); the enclosing function returns -1 if the pair is not instantiated
+#define SCLDPC_DISPATCH_CASE_(DV, DC, CALL) if (dv_ == DV && dc_ == DC) { CALL(DV, DC); } else
+#define SCLDPC_DISPATCH(dv, dc, CALL)                                  \
+    do {                                                               \
+        const int dv_ = (dv), dc_ = (dc);                              \
+        SCLDPC_DEGREES(SCLDPC_DISPATCH_CASE_, CALL) return -1;         \
+    } while (0)
+
+// ---- launch geometry ---------------------------------------------------------------------------------------------------
+inline int num_sms()
+{
+    static const int n = [] {
+        int dev = 0, sms = 0;
+        cudaGetDevice(&dev);
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        return sms > 0 ? sms : 148;
+    }();
+    return n;
+}
+
+// blocks of `kernel` resident on the whole device at `block` threads per block
+template <typename K>
+static int resident_blocks(K kernel, int block)
+{
+    int occ = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, block, 0) != cudaSuccess || occ < 1) occ = 2;
+    return occ * num_sms();
+}
+
+// grid.x for a grid-stride sweep over `items` threads-worth of work replicated over G graphs:
+// a whole number of waves of the machine (multiples of the SM count), capped by the work available.
+static inline dim3 sweep_grid(long long items, int G, int block, int blocks_per_sm)
+{
+    long long need = (items + block - 1) / block;
+    long long per_graph = (long long)num_sms() * blocks_per_sm;   // each graph can fill the machine on its own
+    long long gx = need < per_graph ? need : per_graph;
+    if (gx < 1) gx = 1;
+    return dim3((unsigned)gx, (unsigned)G, 1);
+}
+// blocks per SM of the per-iteration sweeps on sweep_grid (message sweeps, copy variant of the node-state window decoder)
+#define SWEEP_BLOCKS_PER_SM 8
 
 
 namespace scldpc {

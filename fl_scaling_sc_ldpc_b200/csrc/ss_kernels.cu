@@ -135,12 +135,7 @@ __global__ void ss_final_kernel(SsParams p)
 template <int DV, int DC>
 static void ss_launch_t(const SsParams &p, cudaStream_t st)
 {
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    long long need = (((long long)p.nk << p.chunk_shift) + 255) / 256;
-    long long gx = need < 4ll * sms ? need : 4ll * sms;
-    ss_ge3_kernel<DV, DC><<<dim3((unsigned)(gx < 1 ? 1 : gx), (unsigned)p.G), 256, 0, st>>>(p);
+    ss_ge3_kernel<DV, DC><<<sweep_grid((long long)p.nk << p.chunk_shift, p.G, 256, 4), 256, 0, st>>>(p);
     int bx = (p.vns_pos * p.chunks + 255) / 256;
     if (bx > 8) bx = 8;
     ss_classify_kernel<DV, DC><<<dim3(bx, p.L, p.G), 256, 0, st>>>(p);
@@ -150,12 +145,9 @@ static void ss_launch_t(const SsParams &p, cudaStream_t st)
 
 int ss_launch(const SsParams &p, cudaStream_t st)
 {
-    if (p.dv == 4 && p.dc == 8) ss_launch_t<4, 8>(p, st);
-    else if (p.dv == 3 && p.dc == 6) ss_launch_t<3, 6>(p, st);
-    else if (p.dv == 5 && p.dc == 10) ss_launch_t<5, 10>(p, st);
-    else if (p.dv == 3 && p.dc == 9) ss_launch_t<3, 9>(p, st);
-    else if (p.dv == 4 && p.dc == 12) ss_launch_t<4, 12>(p, st);
-    else return -1;
+#define CALL_SS(A, B) ss_launch_t<A, B>(p, st)
+    SCLDPC_DISPATCH(p.dv, p.dc, CALL_SS);
+#undef CALL_SS
     return 0;
 }
 

@@ -101,19 +101,12 @@ def test_full_bp_extreme_channels():
         check_bp(eng.decode_bp_full(fb, 0, is_term, trajectory=True, max_rows=32), ref, rows=True)
 
 
-@pytest.fixture(params=["node_state", "node_lists", "node_copy", "two_launches", "persistent"])
+@pytest.fixture(params=["node_state", "two_launches"])
 def window_mode(request, monkeypatch):
-    """the window decoder in node-state form (default: resolution lists for long windows, copy of the VN window for short
-    ones; both forced here), with message-passing sweeps as two launches per iteration, and with message-passing sweeps as
-    one cooperative launch per window"""
-    monkeypatch.setenv("SCLDPC_WINDOW_NODE", "1" if request.param.startswith("node") else "0")
-    monkeypatch.delenv("SCLDPC_WINDOW_LISTS", raising=False)
-    if request.param in ("node_lists", "node_copy"):
-        monkeypatch.setenv("SCLDPC_WINDOW_LISTS", "1" if request.param == "node_lists" else "0")
-    if request.param == "persistent":
-        monkeypatch.setenv("SCLDPC_PERSISTENT", "1")
-    else:
-        monkeypatch.delenv("SCLDPC_PERSISTENT", raising=False)
+    """the window decoder in node-state form and with message-passing sweeps (two launches per iteration).  The node-state
+    form takes resolution lists iff 2(W+dv-1) >= L and copies the VN window otherwise, so the windows below run both
+    variants: the copy at W=2 for (3,6) L=10 and at W=2, 3 for (4,8) L=14, the lists everywhere else"""
+    monkeypatch.setenv("SCLDPC_WINDOW_NODE", "1" if request.param == "node_state" else "0")
     return request.param
 
 

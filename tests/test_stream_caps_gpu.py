@@ -5,15 +5,17 @@ import pytest
 
 import fl_scaling_sc_ldpc_b200 as eng
 import oracle
+from tests import util
 
 pytestmark = pytest.mark.gpu
 STATS = ("residual", "blocks_err", "erasures_exp", "blocks_err_exp")
 CAP_LISTS = ([1, 2, 9, 40], [3, 7, 0], [5], [400, 800])
 
 
-def assert_caps_equal_capped(fbg, B, eps, seed, caps, **kw):
-    """one checkpointed stream against one capped stream per cap; returns the checkpointed result"""
-    r = eng.decode_bp_stream(fbg, B, eps, seed, first_graph_id=3, caps=caps, **kw)
+def assert_caps_equal_capped(fbg, B, eps, seed, caps, r=None, **kw):
+    """one checkpointed stream (r, if the caller has decoded it already) against one capped stream per cap; returns it"""
+    if r is None:
+        r = eng.decode_bp_stream(fbg, B, eps, seed, first_graph_id=3, caps=caps, **kw)
     assert isinstance(r, eng.StreamCapsResult) and r.caps == tuple(caps)
     assert r.iters.shape == (fbg.n_graphs, B) and r.residual.shape == (len(caps), fbg.n_graphs, B)
     for k, T in enumerate(caps):
@@ -100,15 +102,15 @@ def test_caps_full_size_with_lane_compaction():
     assert (r.iters > 350).any() and (r.residual[0] > r.residual[2]).any()
 
 
-def test_caps_compaction_off_gives_the_same_results(monkeypatch):
+def test_caps_with_lane_compaction_equal_capped_streams():
+    """512 lanes in the tail of 3000 frames per graph: the checkpointed stream compacts its lanes"""
     ens = eng.Ensemble(4, 8, 16, 64)
     fbg = eng.FrameBatch(ens, 2, 512).generate_graphs(47, first_graph_id=3)
-    out = {}
-    for c in ("0", "1"):
-        monkeypatch.setenv("SCLDPC_COMPACT", c)
-        out[c] = eng.decode_bp_stream(fbg, 3000, [0.48, 0.5], 5, first_graph_id=3, caps=[2, 20, 60, 0], harvest_every=4)
-    for key in ("iters",) + STATS:
-        assert (getattr(out["0"], key) == getattr(out["1"], key)).all(), key
+    eps, caps = [0.48, 0.5], [2, 20, 60, 0]
+    r = eng.decode_bp_stream(fbg, 3000, eps, 5, first_graph_id=3, caps=caps, harvest_every=4)
+    n_cmp, moved = util.stream_compactions(fbg)          # before the capped streams reuse the workspace
+    assert n_cmp >= 1 and moved >= n_cmp, (n_cmp, moved)
+    assert_caps_equal_capped(fbg, 3000, eps, 5, caps, r=r, harvest_every=4)
 
 
 def test_bad_caps_are_rejected():

@@ -4,6 +4,7 @@ import numpy as np
 import pytest
 
 import fl_scaling_sc_ldpc_b200 as eng
+from tests import util
 
 pytestmark = pytest.mark.gpu
 KEYS = ("iters", "residual", "blocks_err", "erasures_exp", "blocks_err_exp")
@@ -174,7 +175,6 @@ def test_resolution_list_overflow_falls_back_to_a_full_pass(cap, monkeypatch, st
     a = eng.decode_bp_full(fb, 0, True)
     w = eng.decode_bp_window(fb, 9, 4, 10)
     monkeypatch.setenv("SCLDPC_LIST_CAP", str(cap))
-    monkeypatch.setenv("SCLDPC_WINDOW_LISTS", "1")
     b = eng.decode_bp_full(fb, 0, True)
     w2 = eng.decode_bp_window(fb, 9, 4, 10)
     for key in KEYS:
@@ -182,17 +182,8 @@ def test_resolution_list_overflow_falls_back_to_a_full_pass(cap, monkeypatch, st
     assert bool((a.erased_words == b.erased_words).all()) and bool((w.erased_words == w2.erased_words).all())
 
 
-def _stream_compactions(fb):
-    """(compactions, frames moved) of the last node-state stream call on fb's workspace (scldpc_bp_sweep_stats)"""
-    import ctypes
-    from fl_scaling_sc_ldpc_b200 import _lib
-    st = (ctypes.c_longlong * 2)()
-    _lib.check(_lib.lib().scldpc_bp_sweep_stats(ctypes.byref(fb.dims), 32, ctypes.c_void_p(fb._ws.data_ptr()), st))   # SCLDPC_F_STREAM
-    return int(st[0]), int(st[1])
-
-
 @pytest.mark.parametrize("lanes,B,cap", [(1024, 1300, 0), (512, 512, 0), (256, 700, 9), (1024, 1024, 0)])
-def test_lane_compaction_in_the_tail_changes_nothing(lanes, B, cap, monkeypatch, stream_kernels):
+def test_lane_compaction_in_the_tail_changes_nothing(lanes, B, cap, stream_kernels):
     """Once a graph has handed out its last frame the live frames move into the lowest 128-lane chunks (ns_compact_*): the
     per-frame results must not depend on it, and it must really happen (several times: 8 -> 4 -> 2 -> 1 chunks)"""
     if stream_kernels == "messages":
@@ -202,29 +193,23 @@ def test_lane_compaction_in_the_tail_changes_nothing(lanes, B, cap, monkeypatch,
     eps = [0.44, 0.49, 0.52]                                     # the last one stalls: long-lived frames spread over all chunks
     ref = sync_reference(fbg, ens, B, eps, 9, True, max_it=cap)
     for H in (1, 4, 0):
-        monkeypatch.setenv("SCLDPC_COMPACT", "0")
-        a = eng.decode_bp_stream(fbg, B, eps, 9, first_graph_id=3, harvest_every=H, max_it=cap)
-        assert _stream_compactions(fbg) == (0, 0)
-        monkeypatch.setenv("SCLDPC_COMPACT", "1")
         b = eng.decode_bp_stream(fbg, B, eps, 9, first_graph_id=3, harvest_every=H, max_it=cap)
-        n_cmp, moved = _stream_compactions(fbg)
+        n_cmp, moved = util.stream_compactions(fbg)
         for key in KEYS:
-            assert (getattr(a, key) == ref[key]).all() and (getattr(b, key) == ref[key]).all(), (H, key)
+            assert (getattr(b, key) == ref[key]).all(), (H, key)
         if H == 1 and cap == 0:                                  # every iteration is a chance to compact
             assert n_cmp >= 3 and moved >= n_cmp, (n_cmp, moved)
 
 
-def test_many_graphs_finishing_at_different_times(monkeypatch):
+def test_many_graphs_finishing_at_different_times():
     """40 graphs with channels from easy to hopeless: graphs finish at very different times, the grids of the stream kernels
-    shrink to the list of graphs still decoding (more than one ballot word of graphs); with and without that list"""
+    shrink to the list of graphs still decoding (more than one ballot word of graphs)"""
     G = 40
     ens = eng.Ensemble(4, 8, 10, 32)
     fbg = eng.FrameBatch(ens, G, 64).generate_graphs(51, first_graph_id=3)
     eps = [0.30 + 0.24 * (g % 7) / 6 for g in range(G)]
     ref = sync_reference(fbg, ens, 150, eps, 13, True)
-    for grids in ("1", "0"):
-        monkeypatch.setenv("SCLDPC_ALIVE_GRIDS", grids)
-        for H in (1, 0):
-            s = eng.decode_bp_stream(fbg, 150, eps, 13, first_graph_id=3, harvest_every=H)
-            for key in KEYS:
-                assert (getattr(s, key) == ref[key]).all(), (grids, H, key)
+    for H in (1, 0):
+        s = eng.decode_bp_stream(fbg, 150, eps, 13, first_graph_id=3, harvest_every=H)
+        for key in KEYS:
+            assert (getattr(s, key) == ref[key]).all(), (H, key)

@@ -77,3 +77,12 @@ def oracle_sw(graphs, chan, W, max_it, init_it, square, is_term):
             out["iters"][g, f] = o["win_iters"].sum()
             out["erased"][g, f] = o["erased"]
     return out
+
+
+def stream_compactions(fb):
+    """(compactions, frames moved) of the last node-state stream call on fb's workspace (scldpc_bp_sweep_stats)"""
+    import ctypes
+    from fl_scaling_sc_ldpc_b200 import _lib
+    st = (ctypes.c_longlong * 2)()
+    _lib.check(_lib.lib().scldpc_bp_sweep_stats(ctypes.byref(fb.dims), 32, ctypes.c_void_p(fb._ws.data_ptr()), st))   # SCLDPC_F_STREAM
+    return int(st[0]), int(st[1])

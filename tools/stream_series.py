@@ -31,7 +31,7 @@ idx = np.array(idx[:n]); us = np.array(cn[:n]) * 1e3
 fi = int(r.iters.astype(np.int64).sum())
 print(json.dumps(dict(eps=a.eps, frames=a.frames, launched=r.iters_launched, wall_ms_unsampled=wall_plain, wall_ms_sampled=t0.elapsed_time(t1),
                       sum_sampled_kernel_ms_scaled=float(us.sum() * a.every / 1e3), lane_util=fi / (r.iters_launched * lanes),
-                      mean_iters=fi / a.frames, compact=os.environ.get("SCLDPC_COMPACT", "1"))))
+                      mean_iters=fi / a.frames)))
 step = max(1, r.iters_launched // a.buckets)
 for lo in range(0, r.iters_launched, step):
     m = (idx >= lo) & (idx < lo + step)

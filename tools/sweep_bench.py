@@ -58,8 +58,7 @@ def main():
                cn_us=float(np.median(cn_ms[keep]) * 1e3), vn_us=float(np.median(vn_ms[keep]) * 1e3),
                cn_GBs=float(cn_bytes / np.median(cn_ms[keep]) / 1e6), vn_GBs=float(vn_bytes / np.median(vn_ms[keep]) / 1e6),
                both_GBs=float((cn_bytes + vn_bytes) / (np.median(cn_ms[keep]) + np.median(vn_ms[keep])) / 1e6),
-               wall_ms_per_iter=float(ev0.elapsed_time(ev1) / a.reps / a.iters),
-               blocks_per_sm=os.environ.get("SCLDPC_BLOCKS_PER_SM", "default"))
+               wall_ms_per_iter=float(ev0.elapsed_time(ev1) / a.reps / a.iters))
     out["wall_GBs"] = float((cn_bytes + vn_bytes) / out["wall_ms_per_iter"] / 1e6)
     st = (ctypes.c_longlong * 2)()
     flags = _lib.F_TERMINATED | (_lib.F_TRAJECTORY if a.traj else 0)

@@ -1,3 +1,1 @@
 for W in 3 10; do for G in 4 8 16; do python tools/window_bench.py --W $W --graphs $G --nonterm --eps $( [ $W = 3 ] && echo 0.30 || echo 0.45 ); done; done
-for c in 80 120; do echo "== C10=$c"; SCLDPC_HARVEST_C10=$c python bench.py --steps 4 --warmup 2 --no-cpu-baseline --workloads none 2>/dev/null | python -c "
-import sys, json; d = json.loads(sys.stdin.read().strip().splitlines()[-1]); print(round(d['value'] / 1e13, 4), 'e13', round(d['frames_per_s']), 'frames/s', d['gpu_launches'], 'launches')"; done
