@@ -5,8 +5,8 @@ sliding-window BP, peeling decoding with trajectories) behind the reference's Py
 formats.  Hand-written sm_100a CUDA kernels in ``csrc/`` are reached through the C ABI of ``libscldpc.so``
 (``include/scldpc.h``); PyTorch only owns device buffers.  There is no CPU fallback.
 """
-from .engine import (UNLIMITED, BpResult, Ensemble, FrameBatch, StreamCapsResult, StreamResult, decode_bp_full,  # noqa: F401
-                     decode_bp_stream, decode_bp_window, decode_host, unpack_lanes, words_for)
+from .engine import (UNLIMITED, BpResult, Ensemble, FrameBatch, StreamCapsResult, StreamResult,  # noqa: F401
+                     StreamStoppingSetResult, decode_bp_full, decode_bp_stream, decode_bp_window, decode_host, unpack_lanes, words_for)
 from ._lib import ScldpcError  # noqa: F401
 
 __version__ = "0.1.0"

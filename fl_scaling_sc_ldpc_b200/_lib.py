@@ -28,7 +28,7 @@ EXPORTS = [
     "scldpc_graph_generate_scratch_bytes", "scldpc_channel_generate", "scldpc_channel_pack_host",
     "scldpc_bp_workspace_bytes", "scldpc_bp_full", "scldpc_bp_window", "scldpc_bp_window_range", "scldpc_decode_host",
     "scldpc_graph_generate_at", "scldpc_channel_generate_at",
-    "scldpc_bp_stream_workspace_bytes", "scldpc_bp_stream", "scldpc_bp_stream_caps_workspace_bytes", "scldpc_bp_stream_caps", "scldpc_stream_host", "scldpc_bp_position_counts", "scldpc_bp_stopping_sets", "scldpc_bp_trajectory_moments", "scldpc_pairwise_moments_accumulate", "scldpc_allreduce_counters",
+    "scldpc_bp_stream_workspace_bytes", "scldpc_bp_stream", "scldpc_bp_stream_caps_workspace_bytes", "scldpc_bp_stream_caps", "scldpc_bp_stream_stopping_sets_workspace_bytes", "scldpc_bp_stream_stopping_sets", "scldpc_stream_host", "scldpc_bp_position_counts", "scldpc_bp_stopping_sets", "scldpc_bp_trajectory_moments", "scldpc_pairwise_moments_accumulate", "scldpc_allreduce_counters",
     "scldpc_peel_workspace_bytes", "scldpc_peel_trajectories", "scldpc_peel_variance_accumulate", "scldpc_philox_picks",
     "scldpc_launch_count", "scldpc_profile_begin", "scldpc_profile_end", "scldpc_bp_sweep_stats",
 ]
@@ -67,6 +67,10 @@ class StreamOut(ctypes.Structure):
 
 class StreamCapsOut(ctypes.Structure):
     _fields_ = [(k, ctypes.c_void_p) for k in ("iters_dev", "residual_dev", "blocks_err_dev", "erasures_exp_dev", "blocks_err_exp_dev")]
+
+
+class StreamSsOut(ctypes.Structure):
+    _fields_ = [("iters_dev", ctypes.c_void_p), ("records_dev", ctypes.c_void_p)]
 
 
 MAX_CAPS = 16  # SCLDPC_MAX_CAPS
@@ -111,6 +115,7 @@ def lib() -> ctypes.CDLL:
         L.scldpc_bp_workspace_bytes.restype = ctypes.c_size_t
         L.scldpc_bp_stream_workspace_bytes.restype = ctypes.c_size_t
         L.scldpc_bp_stream_caps_workspace_bytes.restype = ctypes.c_size_t
+        L.scldpc_bp_stream_stopping_sets_workspace_bytes.restype = ctypes.c_size_t
         L.scldpc_graph_generate_scratch_bytes.restype = ctypes.c_size_t
         L.scldpc_launch_count.restype = ctypes.c_longlong
         L.scldpc_peel_workspace_bytes.restype = ctypes.c_size_t

@@ -544,6 +544,10 @@ static void launch_count_pairs(const BpParams &p, cudaStream_t st)
         q.lane_mask = p.done_mask;                              // every stopped frame is counted; the failed ones land in fail_mask
         bp_pos_count_kernel<<<dim3(bx, p.L, graphs_in_grid(p)), 256, 0, st>>>(q);
     } else bp_pos_count_kernel<<<dim3(bx, p.L, graphs_in_grid(p)), 256, 0, st>>>(p);
+    if (p.ss_records) {                                         // streams with stopping-set records classify instead (ss_launch_stream)
+        g_prof.launches += 1;
+        return;
+    }
     dim3 gp = sweep_grid((long long)p.n << p.chunk_shift, p.G, 256, (p.ex2 && p.lane_mask) ? 8 : 4);
     if (p.ex2 && p.lane_mask) {
         g_prof.launches += 3;

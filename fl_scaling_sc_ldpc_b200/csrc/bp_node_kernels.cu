@@ -61,10 +61,15 @@ namespace scldpc {
 // CKPT (streams with checkpoints, CAPPED as well): a frame that reaches its next checkpoint caps[lane_ck] without stopping
 // in that iteration pauses -- it leaves active for pause_mask, not done_mask -- and the harvest records its statistics and
 // puts it back into active.  A paused lane is masked like a capped one, and its lane_iter does not advance.
-template <int DV, int DC, bool CAPPED, bool CKPT = false>
+// HEAD (streams with stopping-set records, unlimited): the unscanned head of simulate_sc_ldpc with is_bounded = False, per lane.
+// A CN below cn_dis_lim that starts a frame with exactly one erased neighbour never resolves it (bpw_iter_kernel<.,.,HEAD>);
+// "starts" is the frame's first iteration, the launch after the harvest that armed its lane (head_arm), so the cn_dis bits of
+// the armed lanes are set there and every other lane keeps its own.
+template <int DV, int DC, bool CAPPED, bool CKPT = false, bool HEAD = false>
 __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
 {
     static_assert(CAPPED || !CKPT, "a paused frame must not be cleared");
+    static_assert(!(HEAD && CAPPED), "the unscanned head is an unlimited-decoder rule");
     static_assert(DC <= 16, "neighbour index is encoded in four bit planes");
     pdl_wait_then_release();
     const int g = graph_of(p, blockIdx.y);
@@ -132,6 +137,22 @@ __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
             }
             res = one & ~tw;                                    // frames in which exactly one neighbour of c is erased
             if (CAPPED) res &= act;
+            if (HEAD && (idx >> cs) < p.cn_dis_lim) {
+                // one 64-bit half at a time, with 32-bit word offsets (the plane offsets are below 2^32, see capi.cu): the u128
+                // merge with 64-bit pointers spilled the (4,12) and (3,9) sweeps
+                const unsigned dw = 2u * (((unsigned)g * (unsigned)p.cn_dis_lim + (unsigned)(idx >> cs)) * (unsigned)ch + (unsigned)k);
+                const unsigned aw = (unsigned)g * (unsigned)p.W + 2u * (unsigned)k;
+#pragma unroll
+                for (int h = 0; h < 2; h++) {
+                    u64 &r = h ? res.y : res.x;
+                    u64 *dp = reinterpret_cast<u64 *>(p.cn_dis) + dw + h;
+                    const u64 dis = *dp;
+                    const u64 arm = p.head_arm ? p.arm_mask[aw + h] : 0ull;
+                    const u64 nd = (r & arm) | (dis & ~arm);
+                    if (nd != dis) *dp = nd;
+                    r &= ~nd;
+                }
+            }
 #if NS_VARIANT & 16
             if (nz(res)) reinterpret_cast<int *>(p.pos_er)[((size_t)g * (p.L + DV - 1) + (idx >> cs) / p.cns_pos) * ch + k] = p.iter + 1;
 #endif
@@ -383,8 +404,8 @@ __global__ void __launch_bounds__(256, 4) ns_arm_kernel(BpParams p)
 // over all chunks -- about 1000 of the 14 500 iterations of the benchmarked eps = 0.49 graph run with a few dozen live frames
 // at the full price.  After a harvest that armed nothing, when the live frames fit into half the chunks in use, they move to
 // the lowest lanes: a frame's whole decoder state is its bit column in the (equal, settled) planes plus lane_frame and
-// lane_iter (and lane_ck in a stream with checkpoints, whose paused frames the harvest has just put back into active), so the
-// move is one pass over the plane; gshift[g] then tells ns_iter_kernel to spread its threads over the occupied chunks only.
+// lane_iter (and lane_ck in a stream with checkpoints, whose paused frames the harvest has just put back into active, and the
+// cn_dis rows in a stream with an unscanned head), so the move is one pass over the plane; gshift[g] then tells ns_iter_kernel to spread its threads over the occupied chunks only.
 // Frame results are stored under the frame id, so nothing downstream sees the lane change.
 __global__ void ns_compact_plan_kernel(BpParams p)
 {
@@ -449,12 +470,17 @@ __global__ void __launch_bounds__(256) ns_compact_kernel(BpParams p)
     __shared__ u128 s_in[CMP_ROWS * SCLDPC_MAX_WORDS / 2], s_out[CMP_ROWS * SCLDPC_MAX_WORDS / 2];
     const int ch = p.chunks, RWORDS = 2 * p.W, AW = (A + 31) >> 5;
     for (int i = threadIdx.x; i < A; i += blockDim.x) s_src[i] = (unsigned short)p.cmp_src[g * p.lanes + i];
-    u128 *__restrict__ x = p.x + (size_t)g * p.n * ch;
-    u128 *__restrict__ xb = p.xb + (size_t)g * p.n * ch;
     const unsigned *in32 = reinterpret_cast<const unsigned *>(s_in);
     unsigned *out32 = reinterpret_cast<unsigned *>(s_out);
-    for (int row0 = blockIdx.x * CMP_ROWS; row0 < p.n; row0 += gridDim.x * CMP_ROWS) {
-        const int rows = min(CMP_ROWS, p.n - row0);
+    // tiles of the two planes' rows, then (streams with an unscanned head) of the cn_dis rows, which are per-lane decoder state too
+    const int t_planes = (p.n + CMP_ROWS - 1) / CMP_ROWS;
+    const int t_all = t_planes + (p.cn_dis ? (p.cn_dis_lim + CMP_ROWS - 1) / CMP_ROWS : 0);
+    for (int t = blockIdx.x; t < t_all; t += gridDim.x) {
+        const bool dis = t >= t_planes;
+        const int row0 = (dis ? t - t_planes : t) * CMP_ROWS;
+        const int rows = min(CMP_ROWS, (dis ? p.cn_dis_lim : p.n) - row0);
+        u128 *__restrict__ x = dis ? p.cn_dis + (size_t)g * p.cn_dis_lim * ch : p.x + (size_t)g * p.n * ch;
+        u128 *__restrict__ xb = dis ? nullptr : p.xb + (size_t)g * p.n * ch;
         __syncthreads();
         for (int i = threadIdx.x; i < rows * ch; i += blockDim.x) {
             s_in[i] = x[(size_t)row0 * ch + i];
@@ -475,7 +501,10 @@ __global__ void __launch_bounds__(256) ns_compact_kernel(BpParams p)
         __syncthreads();
         for (int i = threadIdx.x; i < rows * ch; i += blockDim.x) {
             const u128 v = s_out[i];
-            if (neq(v, s_in[i])) { x[(size_t)row0 * ch + i] = v; xb[(size_t)row0 * ch + i] = v; }
+            if (neq(v, s_in[i])) {
+                x[(size_t)row0 * ch + i] = v;
+                if (xb) xb[(size_t)row0 * ch + i] = v;
+            }
         }
     }
 }
@@ -527,6 +556,7 @@ static void launch_node_iteration(const BpParams &p, bool after_harvest, cudaStr
     const bool pdl = !after_harvest && !sample;
     if (p.n_caps > 0) launch_pdl(ns_iter_kernel<DV, DC, true, true>, grid, block, st, pdl, p);
     else if (p.stream_cap > 0) launch_pdl(ns_iter_kernel<DV, DC, true>, grid, block, st, pdl, p);
+    else if (p.cn_dis_lim > 0) launch_pdl(ns_iter_kernel<DV, DC, false, false, true>, grid, block, st, pdl, p);
     else launch_pdl(ns_iter_kernel<DV, DC, false>, grid, block, st, pdl, p);
     if (sample) {
         cudaEventRecord(ev[1], st);

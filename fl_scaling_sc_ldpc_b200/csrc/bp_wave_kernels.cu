@@ -563,7 +563,7 @@ __global__ void bp_stream_harvest_kernel(BpParams p, int exp_all)
             e_exp += __shfl_xor_sync(0xffffffffu, e_exp, o);
             b_exp += __shfl_xor_sync(0xffffffffu, b_exp, o);
         }
-        if ((threadIdx.x & 31) == 0 && fr >= 0 && fr < B) {
+        if ((threadIdx.x & 31) == 0 && fr >= 0 && fr < B && p.s_residual) {     // (streams with stopping-set records: iters only)
             const size_t o = (size_t)g * B + fr;
             if (CKPT) {
                 const int k0 = p.lane_ck[g * p.lanes + l];
@@ -595,7 +595,7 @@ __global__ void bp_stream_harvest_kernel(BpParams p, int exp_all)
             p.s_iters[o] = its;
             atomicAdd(&s_frames, 1);
             atomicAdd(&s_its, (unsigned long long)its);
-            if (!((p.fail_mask[g * W + w] >> b) & 1ull)) {
+            if (!((p.fail_mask[g * W + w] >> b) & 1ull) && p.s_residual) {
                 if (CKPT) store_ck_slots(p, o, p.lane_ck[g * p.lanes + l], p.n_caps, 0, 0, 0, 0);
                 else {
                     p.s_residual[o] = 0;

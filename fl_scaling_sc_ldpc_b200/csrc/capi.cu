@@ -49,6 +49,7 @@ int peel_grid(int total_size, long long total_frames, int n_cn_all);
 size_t peel_state_words(int n_cn_all, int total_size);
 int peel_launch(PeelParams p, int grid, cudaStream_t st);
 int ss_launch(const SsParams &p, cudaStream_t st);
+int ss_launch_stream(const BpParams &p, cudaStream_t st);
 void corr_moments_launch(const int32_t *r1, int n_frames, int row_len, int start, int step, int K, long long *acc, cudaStream_t st);
 void traj_moments_launch(const int32_t *rows, const int32_t *iters, int G, int max_rows, int lanes, int n_frames, long long *acc,
                          cudaStream_t st);
@@ -181,6 +182,8 @@ static size_t list_stride(size_t max_nodes, size_t ch)
 
 // internal: workspace of scldpc_bp_stream_caps (per-lane checkpoint state on top of the node-state stream's)
 #define F_CAPS_WS 0x10000u
+// internal: workspace of scldpc_bp_stream_stopping_sets (unscanned-head plane and stopping-set accumulators on top of it)
+#define F_SS_WS 0x20000u
 
 static size_t carve(const scldpc_dims_t *d, uint32_t flags, void *ws, BpParams *p)
 {
@@ -249,6 +252,12 @@ static size_t carve(const scldpc_dims_t *d, uint32_t flags, void *ws, BpParams *
         }
     }
     q.cn_dis = (flags & SCLDPC_F_STREAM) ? nullptr : c.take<u128>(G * nk * ch);   // sized for the largest possible ignored head
+    if ((flags & F_SS_WS) && no_msgs) {
+        q.cn_dis = c.take<u128>(G * nk * ch);                         // as the synchronous path's
+        q.ss_lost = c.take<int>(G * d->L * lanes);
+        q.ss_big = c.take<int>(G * d->L * lanes);
+        q.ss_counted = c.take<unsigned char>(d->L);
+    }
     if (!(flags & (SCLDPC_F_STREAM | SCLDPC_F_MESSAGES))) {
         // node-state window decoder / synchronous full BP (bp_window_node_kernels.cu): per-warp resolution lists
         const size_t RW = list_regions(nk > n / 4 ? nk : n / 4, ch);
@@ -594,18 +603,33 @@ extern "C" size_t scldpc_bp_stream_caps_workspace_bytes(const scldpc_dims_t *d)
     return carve(d, SCLDPC_F_STREAM | F_CAPS_WS, nullptr, nullptr);
 }
 
-// Frame stream of scldpc_bp_stream (n_caps == 0: `out` holds the [G][B] results) or scldpc_bp_stream_caps (n_caps >= 1:
-// `out` holds iters [G][B] and the [K][G][B] statistics; the caps are validated by the caller).
+extern "C" size_t scldpc_bp_stream_stopping_sets_workspace_bytes(const scldpc_dims_t *d)
+{
+    if (check_dims(d)) return 0;
+    return carve(d, SCLDPC_F_STREAM | F_SS_WS, nullptr, nullptr);
+}
+
+// stopping-set records of scldpc_bp_stream_stopping_sets
+struct StreamSs {
+    const uint8_t *counted_pos_host;   // [L] or NULL (all positions)
+    int unscanned_head_cns;
+    int32_t *records_dev;              // [G][B][4]
+};
+
+// Frame stream of scldpc_bp_stream (n_caps == 0: `out` holds the [G][B] results), scldpc_bp_stream_caps (n_caps >= 1:
+// `out` holds iters [G][B] and the [K][G][B] statistics; the caps are validated by the caller) or
+// scldpc_bp_stream_stopping_sets (ss != NULL: `out` holds iters only, the records go to ss->records_dev).
 static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const scldpc_stream_cfg_t *cfg, const int32_t *caps,
-                          int n_caps, const scldpc_stream_out_t *out, void *workspace_dev, size_t workspace_bytes,
-                          long long *iters_launched_host, void *stream)
+                          int n_caps, const StreamSs *ss, const scldpc_stream_out_t *out, void *workspace_dev,
+                          size_t workspace_bytes, long long *iters_launched_host, void *stream)
 {
     int rc = check_dims(d);
     if (rc) return rc;
     if (!degrees_supported(d->dv, d->dc)) return fail(SCLDPC_EINVAL, "(dv,dc)=(%d,%d) not instantiated", d->dv, d->dc);
     if (!b || !b->vn_cn_dev || !b->vn_slot_dev || !b->cn_edge_dev) return fail(SCLDPC_EINVAL, "batch pointer is NULL");
     if (!cfg || !cfg->eps_host || cfg->frames_per_graph < 1) return fail(SCLDPC_EINVAL, "bad stream configuration");
-    if (!out || !out->iters_dev || !out->residual_dev || !out->blocks_err_dev || !out->erasures_exp_dev || !out->blocks_err_exp_dev)
+    if (!out || !out->iters_dev ||
+        (!ss && (!out->residual_dev || !out->blocks_err_dev || !out->erasures_exp_dev || !out->blocks_err_exp_dev)))
         return fail(SCLDPC_EINVAL, "output pointer is NULL");
     if (d->n_frames < 1) return fail(SCLDPC_EINVAL, "n_frames (lanes used per graph) must be >= 1");
     if ((cfg->flags & SCLDPC_F_MESSAGES) && d->L + d->dv - 1 > 1024) return fail(SCLDPC_EINVAL, "chain too long for the message-passing stream");
@@ -613,7 +637,7 @@ static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const
     // SCLDPC_F_MESSAGES selects the message-passing sweeps (the implementation of record); the default is the node-state
     // formulation of bp_node_kernels.cu, which yields the same erased set at every iteration with ~6x less HBM traffic
     const bool node = !(cfg->flags & SCLDPC_F_MESSAGES);
-    const uint32_t wflags = SCLDPC_F_STREAM | (cfg->flags & SCLDPC_F_MESSAGES) | (n_caps > 0 ? F_CAPS_WS : 0u);
+    const uint32_t wflags = SCLDPC_F_STREAM | (cfg->flags & SCLDPC_F_MESSAGES) | (n_caps > 0 ? F_CAPS_WS : 0u) | (ss ? F_SS_WS : 0u);
     const size_t need = carve(d, wflags, nullptr, nullptr);
     if (workspace_bytes < need) return fail(SCLDPC_ENOMEM, "workspace too small: %zu < %zu bytes", workspace_bytes, need);
     if ((rc = have_device())) return rc;
@@ -645,6 +669,15 @@ static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const
     p.s_erasures_exp = out->erasures_exp_dev; p.s_blocks_err_exp = out->blocks_err_exp_dev;
     p.lane_mask = p.fail_mask;                   // frames that stopped without erasures have all-zero counts already
     p.lazy_success = node ? 1 : 0;
+    std::vector<unsigned char> counted;
+    if (ss) {
+        if (ss->unscanned_head_cns < 0 || ss->unscanned_head_cns > p.c1)
+            return fail(SCLDPC_EINVAL, "unscanned_head_cns must be in [0, %d] (the CNs the decoder sweeps), got %d", p.c1, ss->unscanned_head_cns);
+        p.cn_dis_lim = ss->unscanned_head_cns;
+        p.ss_records = ss->records_dev;
+        counted.assign(d->L, 1);
+        if (ss->counted_pos_host) counted.assign(ss->counted_pos_host, ss->counted_pos_host + d->L);
+    }
     // per-graph channel thresholds and the doping profile
     std::vector<u64> thr(d->n_graphs);
     for (int g = 0; g < d->n_graphs; g++) {
@@ -658,6 +691,12 @@ static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const
     CU(cudaMemcpyAsync(const_cast<u64 *>(p.thr), thr.data(), sizeof(u64) * thr.size(), cudaMemcpyHostToDevice, st));
     if (doped) CU(cudaMemcpyAsync(const_cast<int32_t *>(p.known), known.data(), sizeof(int32_t) * d->L, cudaMemcpyHostToDevice, st));
     else p.known = nullptr;
+    if (ss) {
+        CU(cudaMemcpyAsync(const_cast<unsigned char *>(p.ss_counted), counted.data(), d->L, cudaMemcpyHostToDevice, st));
+        CU(cudaMemsetAsync(p.ss_lost, 0, sizeof(int) * (size_t)p.G * d->L * p.lanes, st));
+        CU(cudaMemsetAsync(p.ss_big, 0, sizeof(int) * (size_t)p.G * d->L * p.lanes, st));
+        CU(cudaMemsetAsync(p.cn_dis, 0, sizeof(u128) * (size_t)p.G * p.nk * p.chunks, st));
+    }
     CU(cudaStreamSynchronize(st));               // host vectors leave scope at return; keep it simple
     if (!node && p.stream_cap > 0) return fail(SCLDPC_EINVAL, "capped frame streams need the node-state sweeps (no SCLDPC_F_MESSAGES)");
     // state: no lane holds a frame yet.  Message sweeps: Lij = 1 (tail CNs of a truncated code are never swept), the rest 0
@@ -715,6 +754,7 @@ static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const
     for (;;) {
         for (int q = 0; q < H; q++, it++) {
             p.iter = (int)(it & 0x3fffffff);
+            p.head_arm = q == 0;                 // the first iteration of the lanes the last harvest armed
             if (node ? bp_launch_node_iteration(d->dv, d->dc, p, q == 0, st) : bp_launch_stream_iteration(d->dv, d->dc, p, q == 0, st))
                 return fail(SCLDPC_EINVAL, "unsupported degrees");
         }
@@ -724,6 +764,7 @@ static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const
         if (adaptive) CU(cudaMemsetAsync(p.alive_total + 1 + slot, 0x7f, sizeof(int), st));
         if (node) bp_launch_node_settle(d->dv, d->dc, p, st);
         bp_launch_count_pairs(d->dv, d->dc, p, st);
+        if (ss) ss_launch_stream(p, st);         // records of the stopped frames, before the harvest re-arms their lanes
         bp_launch_stream_harvest(p, (cfg->flags & SCLDPC_F_EXP_ALL) ? 1 : 0, st);
         if (node) {
             bp_launch_node_arm(p, st);
@@ -760,7 +801,7 @@ extern "C" int scldpc_bp_stream(const scldpc_dims_t *d, const scldpc_batch_t *b,
                                 const scldpc_stream_out_t *out, void *workspace_dev, size_t workspace_bytes,
                                 long long *iters_launched_host, void *stream)
 {
-    return bp_stream_impl(d, b, cfg, nullptr, 0, out, workspace_dev, workspace_bytes, iters_launched_host, stream);
+    return bp_stream_impl(d, b, cfg, nullptr, 0, nullptr, out, workspace_dev, workspace_bytes, iters_launched_host, stream);
 }
 
 // The same stream with checkpoints at the caps of an ascending list (include/scldpc.h).
@@ -781,7 +822,23 @@ extern "C" int scldpc_bp_stream_caps(const scldpc_dims_t *d, const scldpc_batch_
     if (cfg->flags & SCLDPC_F_MESSAGES) return fail(SCLDPC_EINVAL, "frame streams with caps need the node-state sweeps (no SCLDPC_F_MESSAGES)");
     if (!out) return fail(SCLDPC_EINVAL, "output pointer is NULL");
     const scldpc_stream_out_t o{out->iters_dev, out->residual_dev, out->blocks_err_dev, out->erasures_exp_dev, out->blocks_err_exp_dev};
-    return bp_stream_impl(d, b, cfg, caps_host, n_caps, &o, workspace_dev, workspace_bytes, iters_launched_host, stream);
+    return bp_stream_impl(d, b, cfg, caps_host, n_caps, nullptr, &o, workspace_dev, workspace_bytes, iters_launched_host, stream);
+}
+
+// The same stream (unlimited BP) with the stopping-set record of every frame in place of the size-two expurgation (include/scldpc.h).
+extern "C" int scldpc_bp_stream_stopping_sets(const scldpc_dims_t *d, const scldpc_batch_t *b, const scldpc_stream_cfg_t *cfg,
+                                              const uint8_t *counted_pos_host, int unscanned_head_cns,
+                                              const scldpc_stream_ss_out_t *out, void *workspace_dev, size_t workspace_bytes,
+                                              long long *iters_launched_host, void *stream)
+{
+    if (!cfg) return fail(SCLDPC_EINVAL, "bad stream configuration");
+    if (cfg->flags & SCLDPC_F_MESSAGES)
+        return fail(SCLDPC_EINVAL, "frame streams with stopping sets need the node-state sweeps (no SCLDPC_F_MESSAGES)");
+    if (cfg->max_it != 0) return fail(SCLDPC_EINVAL, "cfg->max_it must be 0: stopping sets are records of unlimited BP");
+    if (!out || !out->iters_dev || !out->records_dev) return fail(SCLDPC_EINVAL, "output pointer is NULL");
+    const StreamSs ss{counted_pos_host, unscanned_head_cns, out->records_dev};
+    const scldpc_stream_out_t o{out->iters_dev, nullptr, nullptr, nullptr, nullptr};
+    return bp_stream_impl(d, b, cfg, nullptr, 0, &ss, &o, workspace_dev, workspace_bytes, iters_launched_host, stream);
 }
 
 // first_window / n_windows: the windows [first_window, first_window + n_windows) of the chain (n_windows < 0: to the end).

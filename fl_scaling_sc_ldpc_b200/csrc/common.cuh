@@ -307,6 +307,11 @@ struct BpParams {
     int caps[SCLDPC_MAX_CAPS];
     int *lane_ck;             // [G][lanes] index of the next checkpoint of the lane's frame
     u64 *pause_mask;          // [G][W] lanes paused at a checkpoint, waiting for the harvest (left active, not in done_mask)
+    // frame streams with stopping-set records (scldpc_bp_stream_stopping_sets); cn_dis / cn_dis_lim hold the unscanned head
+    int head_arm;             // 1: this launch is the first iteration of the lanes in arm_mask, which set their cn_dis bits in it
+    int *ss_lost, *ss_big;    // [G][L][lanes] lost VNs / VNs of components with more than two VNs, per position (ss_classify_kernel)
+    const unsigned char *ss_counted;   // [L] positions whose VNs can be lost
+    int32_t *ss_records;      // [G][B][4] per-frame records, indexed by frame id
 };
 
 // graph handled by block coordinate b of a grid that is sized by the list of graphs still decoding
@@ -438,6 +443,9 @@ struct SsParams {
     u128 *ge3;                 // [G][nk][chunks]
     int *pos_lost, *pos_big;   // [G][L][lanes]
     int32_t *out;              // [G][lanes][4]
+    const u64 *lane_mask;      // [G][W] only these lanes are classified (NULL: all); 128-lane chunks without one are skipped
+    const int *glist;          // graphs to classify (grid.y / grid.z index this list; NULL: all G)
+    int n_glist;
 };
 
 // Programmatic dependent launch: the two node-state kernels of an iteration follow each other ~10^5 times per decode, so the launch

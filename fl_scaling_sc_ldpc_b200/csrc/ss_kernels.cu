@@ -14,13 +14,16 @@
 // Round 1 did this on the host (SciPy connected components, one device-to-host sync per failed frame).
 #include "common.cuh"
 
+#include <cstring>
+
 namespace scldpc {
 
 template <int DV, int DC>
 __global__ void __launch_bounds__(256) ss_ge3_kernel(SsParams p)
 {
-    const int g = blockIdx.y, ch = p.chunks;
-    const int k = threadIdx.x & (ch - 1);
+    const int g = p.glist ? p.glist[blockIdx.y] : (int)blockIdx.y, ch = p.chunks;
+    const int k = threadIdx.x & (ch - 1);                       // a thread keeps its chunk
+    if (p.lane_mask && !nz(reinterpret_cast<const u128 *>(p.lane_mask)[g * ch + k])) return;
     const u128 *xk = p.x + (size_t)g * p.n * ch + k;
     u128 *ge3 = p.ge3 + (size_t)g * p.nk * ch;
     const int32_t *cn_edge = p.cn_edge + (size_t)g * p.nk * DC;
@@ -70,8 +73,12 @@ template <int DV, int DC>
 __global__ void __launch_bounds__(256) ss_classify_kernel(SsParams p)
 {
     __shared__ int s_lost[SCLDPC_MAX_LANES], s_big[SCLDPC_MAX_LANES];
-    const int g = blockIdx.z, pos = blockIdx.y, ch = p.chunks;
+    const int g = p.glist ? p.glist[blockIdx.z] : (int)blockIdx.z, pos = blockIdx.y, ch = p.chunks;
     if (!p.counted[pos]) return;
+    // a thread keeps its chunk (blockDim and the stride are multiples of ch) and skips it without a selected lane; the mask is
+    // re-read where it is used (an L1 hit), so that it holds no registers over the loop
+    const u128 *lmask = reinterpret_cast<const u128 *>(p.lane_mask);
+    const int items = (!lmask || nz(lmask[g * ch + (threadIdx.x & (ch - 1))])) ? p.vns_pos * ch : 0;
     for (int i = threadIdx.x; i < p.lanes; i += blockDim.x) { s_lost[i] = 0; s_big[i] = 0; }
     __syncthreads();
     const u128 *x = p.x + (size_t)g * p.n * ch;
@@ -79,10 +86,10 @@ __global__ void __launch_bounds__(256) ss_classify_kernel(SsParams p)
     const u128 *ge3 = p.ge3 + (size_t)g * p.nk * ch;
     const int32_t *vn_cn = p.vn_cn + (size_t)g * p.n * DV;
     const int32_t *cn_edge = p.cn_edge + (size_t)g * p.nk * DC;
-    const int items = p.vns_pos * ch;
     for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < items; idx += gridDim.x * blockDim.x) {
         const int a = pos * p.vns_pos + (idx >> p.chunk_shift), k = idx & (ch - 1);
-        const u128 xa = x[(size_t)a * ch + k];
+        u128 xa = x[(size_t)a * ch + k];
+        if (lmask) xa &= lmask[g * ch + k];
         if (!nz(xa)) continue;
         int cs[DV];
         load_row<DV>(vn_cn + (size_t)a * DV, cs);
@@ -146,6 +153,69 @@ static void ss_launch_t(const SsParams &p, cudaStream_t st)
 int ss_launch(const SsParams &p, cudaStream_t st)
 {
 #define CALL_SS(A, B) ss_launch_t<A, B>(p, st)
+    SCLDPC_DISPATCH(p.dv, p.dc, CALL_SS);
+#undef CALL_SS
+    return 0;
+}
+
+// ---- frame streams with stopping-set records (scldpc_bp_stream_stopping_sets) ----------------------------------------------
+// At a harvest, after bp_pos_count_kernel has found the frames that stopped with erasures left (fail_mask): ss_ge3_kernel and
+// ss_classify_kernel run on the settled plane for those lanes of the graphs still decoding, then ss_stream_record_kernel writes
+// the record of every stopped frame under its frame id -- before bp_stream_harvest_kernel re-arms the lanes and overwrites
+// lane_frame.  The per-position accumulators of the consumed lanes are zero again afterwards; a frame that stopped without
+// erasures gets (0, 0, 0, 0).
+__global__ void ss_stream_record_kernel(BpParams p)
+{
+    const int g = graph_of(p, blockIdx.y), W = p.W;
+    if (ld_cg(p.alive + g) == 0) return;
+    const int l = blockIdx.x * blockDim.x + threadIdx.x;
+    if (l >= p.lanes) return;
+    const int w = l >> 6, b = l & 63;
+    if (!((p.done_mask[g * W + w] >> b) & 1ull)) return;
+    int lost = 0, big = 0, blocks = 0;
+    if ((p.fail_mask[g * W + w] >> b) & 1ull)
+        for (int q = 0; q < p.L; q++) {                         // as ss_final_kernel
+            const size_t o = ((size_t)g * p.L + q) * p.lanes + l;
+            const int lq = p.ss_lost[o], bq = p.ss_big[o];
+            if (lq) p.ss_lost[o] = 0;
+            if (bq) p.ss_big[o] = 0;
+            lost += lq;
+            big += bq;
+            blocks += bq > 0;
+        }
+    const int fr = p.lane_frame[g * p.lanes + l];
+    if (fr >= 0 && fr < p.frames_per_graph) {
+        int32_t *o = p.ss_records + ((size_t)g * p.frames_per_graph + fr) * 4;
+        o[0] = lost; o[1] = big > 0; o[2] = big; o[3] = blocks;
+    }
+}
+
+template <int DV, int DC>
+static void ss_launch_stream_t(const BpParams &b, cudaStream_t st)
+{
+    SsParams p;
+    memset(&p, 0, sizeof p);
+    p.dv = b.dv; p.dc = b.dc; p.n = b.n; p.nk = b.nk; p.E = b.E; p.L = b.L; p.vns_pos = b.vns_pos; p.G = b.G; p.W = b.W;
+    p.chunks = b.chunks; p.chunk_shift = b.chunk_shift; p.lanes = b.lanes;
+    p.vn_cn = b.vn_cn; p.cn_edge = b.cn_edge; p.x = b.x; p.counted = b.ss_counted;
+    p.ge3 = b.ex2;                                              // the pair search's plane: not used in this mode
+    p.pos_lost = b.ss_lost; p.pos_big = b.ss_big;
+    p.lane_mask = b.fail_mask;
+    p.glist = b.glist; p.n_glist = b.n_glist;
+    const unsigned gy = graphs_in_grid(b);
+    dim3 ge = sweep_grid((long long)p.nk << p.chunk_shift, p.G, 256, 4);
+    ge.y = gy;
+    ss_ge3_kernel<DV, DC><<<ge, 256, 0, st>>>(p);
+    int bx = (p.vns_pos * p.chunks + 255) / 256;
+    if (bx > 8) bx = 8;
+    ss_classify_kernel<DV, DC><<<dim3(bx, p.L, gy), 256, 0, st>>>(p);
+    ss_stream_record_kernel<<<dim3((p.lanes + 255) / 256, gy), 256, 0, st>>>(b);
+    g_prof.launches += 3;
+}
+
+int ss_launch_stream(const BpParams &p, cudaStream_t st)
+{
+#define CALL_SS(A, B) ss_launch_stream_t<A, B>(p, st)
     SCLDPC_DISPATCH(p.dv, p.dc, CALL_SS);
 #undef CALL_SS
     return 0;

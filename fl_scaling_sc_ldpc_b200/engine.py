@@ -381,9 +381,21 @@ class StreamCapsResult:
     edge_updates: int = 0
 
 
+@dataclass
+class StreamStoppingSetResult:
+    """Per-frame outputs of ``decode_bp_stream(..., stopping_sets=counted)``, indexed by frame id: ``iters``
+    [n_graphs][frames_per_graph] of unlimited BP and ``records`` [n_graphs][frames_per_graph][4] = (num_lost, has a stopping
+    set of more than two VNs, VNs in such sets, VN positions they touch) -- what ``stopping_set_records`` gives for the
+    frame after ``decode_bp_full`` with the same ``unscanned_head_cns``."""
+    iters: np.ndarray
+    records: np.ndarray
+    iters_launched: int = 0
+    edge_updates: int = 0
+
+
 def decode_bp_stream(fb: FrameBatch, frames_per_graph: int, eps, seed: int, first_graph_id: int = 0, is_term: bool = True,
                      doping_points=(), harvest_every: int = 0, exp_all: bool = False, collect: bool = True, max_it: int = 0,
-                     messages: bool | None = None, caps=None):
+                     messages: bool | None = None, caps=None, stopping_sets=None, unscanned_head_cns: int = 0):
     """Full BP (unlimited, or at most ``max_it`` iterations per frame) over a stream of ``frames_per_graph`` frames per
     graph with lane recycling (``scldpc_bp_stream``).  Frame f of graph g is the channel realisation ``generate_erasures(..., first_frame=...)``
     puts in lane f - first_frame; the graphs are the ones resident in ``fb`` (``fb.n_frames`` lanes are used).
@@ -391,7 +403,16 @@ def decode_bp_stream(fb: FrameBatch, frames_per_graph: int, eps, seed: int, firs
     ``caps``: strictly ascending iteration caps (at most 16, each >= 1; the last may be <= 0, unlimited) in place of
     ``max_it``.  One decode up to the largest cap gives the results of every cap (``scldpc_bp_stream_caps``): a
     ``StreamCapsResult``, or with ``collect=False`` the device tensors (iters [G][B], statistics [4][K][G][B]) and the
-    iterations launched."""
+    iterations launched.
+
+    ``stopping_sets``: the counted positions (bool [L], ``counted_positions``) -- the stream records every frame's stopping
+    sets in place of the size-two expurgation (``scldpc_bp_stream_stopping_sets``, unlimited BP only), with the unscanned
+    head of ``simulate_sc_ldpc(is_bounded=False)`` below ``unscanned_head_cns``: a ``StreamStoppingSetResult``, or with
+    ``collect=False`` the device tensors (iters [G][B], records [G][B][4]) and the iterations launched."""
+    if stopping_sets is not None and (caps is not None or max_it):
+        raise ValueError("stopping_sets needs unlimited BP: it cannot be combined with caps or max_it")
+    if stopping_sets is None and unscanned_head_cns:
+        raise ValueError("unscanned_head_cns applies to stopping_sets streams only")
     L = _lib.lib()
     G, B = fb.n_graphs, int(frames_per_graph)
     eps_arr = np.full(G, float(eps)) if np.ndim(eps) == 0 else np.asarray(eps, np.float64)
@@ -411,6 +432,10 @@ def decode_bp_stream(fb: FrameBatch, frames_per_graph: int, eps, seed: int, firs
         cfg = _lib.StreamCfg(B, int(harvest_every), flags, len(hard), len(soft_p), ptr(eps_arr), ptr(a_h), ptr(a_sp), ptr(a_sc),
                              int(seed), int(first_graph_id), int(max_it))
         return _decode_bp_stream_caps(fb, cfg, caps, collect)
+    if stopping_sets is not None:
+        cfg = _lib.StreamCfg(B, int(harvest_every), flags, len(hard), len(soft_p), ptr(eps_arr), ptr(a_h), ptr(a_sp), ptr(a_sc),
+                             int(seed), int(first_graph_id), 0)
+        return _decode_bp_stream_ss(fb, cfg, stopping_sets, int(unscanned_head_cns), collect)
     cfg = _lib.StreamCfg(B, int(harvest_every), flags, len(hard), len(soft_p), ptr(eps_arr), ptr(a_h), ptr(a_sp), ptr(a_sc),
                          int(seed), int(first_graph_id), max(0, int(max_it)))
     res = torch.zeros((5, G, B), dtype=torch.int32, device=fb.device)
@@ -456,6 +481,33 @@ def _decode_bp_stream_caps(fb: FrameBatch, cfg, caps, collect: bool):
     it, st = iters.cpu().numpy(), stats.cpu().numpy()
     return StreamCapsResult(tuple(int(c) for c in caps_arr), it, st[0], st[1], st[2], st[3], iters_launched=launched.value,
                             edge_updates=int(it.astype(np.int64).sum()) * 2 * fb.ens.E)
+
+
+def _decode_bp_stream_ss(fb: FrameBatch, cfg, counted, unscanned_head_cns: int, collect: bool):
+    L = _lib.lib()
+    G, B = fb.n_graphs, int(cfg.frames_per_graph)
+    cp = np.ascontiguousarray(np.asarray(counted, dtype=np.uint8))
+    if cp.shape != (fb.ens.L,):
+        raise ValueError("stopping_sets needs one counted flag per position")
+    iters = torch.zeros((G, B), dtype=torch.int32, device=fb.device)
+    records = torch.zeros((G, B, 4), dtype=torch.int32, device=fb.device)
+    out = _lib.StreamSsOut(iters.data_ptr(), records.data_ptr())
+    need = L.scldpc_bp_stream_stopping_sets_workspace_bytes(ctypes.byref(fb.dims))
+    if need == 0:
+        raise _lib.ScldpcError(L.scldpc_last_error().decode())
+    if fb._ws is None or fb._ws.numel() < need:
+        fb._ws = None
+        fb._ws = torch.empty(need, dtype=torch.uint8, device=fb.device)
+    launched = ctypes.c_longlong(0)
+    _lib.check(L.scldpc_bp_stream_stopping_sets(ctypes.byref(fb.dims), ctypes.byref(fb.cbatch), ctypes.byref(cfg),
+                                                cp.ctypes.data_as(ctypes.c_void_p), unscanned_head_cns, ctypes.byref(out),
+                                                ctypes.c_void_p(fb._ws.data_ptr()), ctypes.c_size_t(fb._ws.numel()),
+                                                ctypes.byref(launched), _stream()))
+    if not collect:
+        return iters, records, launched.value
+    it = iters.cpu().numpy()
+    return StreamStoppingSetResult(it, records.cpu().numpy(), iters_launched=launched.value,
+                                   edge_updates=int(it.astype(np.int64).sum()) * 2 * fb.ens.E)
 
 
 def decode_host(ens: Ensemble, vn_cn: np.ndarray, erased: np.ndarray, W: int = 0, max_it: int = UNLIMITED, init_it: int = 0,

@@ -236,6 +236,10 @@ def counted_positions(l, L, num_positions, ignored_head, ignored_tail, is_tail_b
     return ((cpos >= ignored_head) & (cpos < num_positions - ignored_tail)).any(axis=1) & (cpos < num_positions).all(axis=1)
 
 
+# simulate_sc_ldpc decodes on frame streams from this many frames per graph on (the rule of bp_lim_iter --stream auto)
+STREAM_MIN_FRAMES_PER_GRAPH = 1024
+
+
 def simulate_sc_ldpc(e, l, r, L, M, is_terminated, is_protograph, is_bounded, is_tail_biting, num_repeats=int(1e5),
                      max_fuckups=2000, doping_points=[], *, seed=None, frames_per_graph=128, graphs_per_batch=8, first_frame=0,
                      progress=True, _batch_factory=None, _records_fn=None):
@@ -245,7 +249,12 @@ def simulate_sc_ldpc(e, l, r, L, M, is_terminated, is_protograph, is_bounded, is
 
     The in-order ``sic_round`` scan (PD.py:656-657) reaches the peeling fixed point, which is the residual of unlimited
     flooding BP; that is what runs on the GPU.  Frames are decoded in batches and then accounted in frame order, so
-    the ``max_fuckups`` early stop (PD.py:698) cuts at the same frame as a sequential run would."""
+    the ``max_fuckups`` early stop (PD.py:698) cuts at the same frame as a sequential run would.
+
+    From ``STREAM_MIN_FRAMES_PER_GRAPH`` frames per graph on, each graph's frames are decoded as a frame stream on at most
+    1024 lanes (``decode_bp_stream(..., stopping_sets=...)``): a lane whose frame has stopped takes the graph's next frame, so
+    no frame waits for the slowest of its word, and any number of frames per graph works.  Frame f of graph g is the same
+    channel realisation on both paths, so the records and the 13-tuple do not depend on the path."""
     _check_ensemble(is_protograph, doping_points, is_tail_biting)
     seed = _state["seed"] if seed is None else seed
     is_soft = isinstance(doping_points, dict)
@@ -267,7 +276,7 @@ def simulate_sc_ldpc(e, l, r, L, M, is_terminated, is_protograph, is_bounded, is
 
     ens = engine.Ensemble(l, r, L, M)
     fpg = int(frames_per_graph)
-    nw = engine.words_for(fpg)
+    use_stream = fpg >= STREAM_MIN_FRAMES_PER_GRAPH and _batch_factory is None and _records_fn is None
     counted = counted_positions(l, L, num_positions, ignored_head, ignored_tail, bool(is_tail_biting))
 
     from . import dist as D
@@ -287,17 +296,23 @@ def simulate_sc_ldpc(e, l, r, L, M, is_terminated, is_protograph, is_bounded, is
             return rec
         if _records_fn is not None:                                      # CPU tests of the round / gather / replay logic
             return np.asarray(_records_fn(G, fpg, gid0), np.int64).reshape(G * fpg, 4)
-        if _batch_factory is not None:                                   # tests inject codes and erasure masks here
-            fb = _batch_factory(ens, G, fpg, gid0)
-        else:
-            fb = engine.FrameBatch(ens, G, fpg, nw)
-            fb.generate_graphs(seed, first_graph_id=gid0, tail_biting=bool(is_tail_biting), protograph=bool(is_protograph))
-            fb.generate_erasures(e, seed + 1, first_graph_id=gid0, doping_points=doping_points)
         # non-terminated: the decoder never uses CNs >= total_size (truncated BP, BP_TRAJ.c:944-948 semantics).
         # unbounded: slots below ignored_head_schedule*cns_per_pos are never scanned (PD.py:656), they only decode
         # when a removal leaves them with one user -- scldpc_bp_full's unscanned_head_cns
-        res = engine.decode_bp_full(fb, engine.UNLIMITED, is_term=bool(is_terminated) and not is_tail_biting,
-                                    unscanned_head_cns=unscanned)
+        is_term = bool(is_terminated) and not is_tail_biting
+        if use_stream:                                                   # the stream draws the channels of its frames itself
+            fb = engine.FrameBatch(ens, G, min(fpg, 1024))
+            fb.generate_graphs(seed, first_graph_id=gid0, tail_biting=bool(is_tail_biting), protograph=bool(is_protograph))
+            res = engine.decode_bp_stream(fb, fpg, e, seed + 1, first_graph_id=gid0, is_term=is_term, doping_points=doping_points,
+                                          stopping_sets=counted, unscanned_head_cns=unscanned)
+            return res.records.reshape(G * fpg, 4).astype(np.int64)
+        if _batch_factory is not None:                                   # tests inject codes and erasure masks here
+            fb = _batch_factory(ens, G, fpg, gid0)
+        else:
+            fb = engine.FrameBatch(ens, G, fpg, engine.words_for(fpg))
+            fb.generate_graphs(seed, first_graph_id=gid0, tail_biting=bool(is_tail_biting), protograph=bool(is_protograph))
+            fb.generate_erasures(e, seed + 1, first_graph_id=gid0, doping_points=doping_points)
+        res = engine.decode_bp_full(fb, engine.UNLIMITED, is_term=is_term, unscanned_head_cns=unscanned)
         # stopping sets of the lost VNs (PD.py:668-691) on the device: one record per frame, one copy per batch
         return stopping_set_records(fb, res.erased_words, counted)[:, :fpg].reshape(G * fpg, 4).astype(np.int64)
 
@@ -401,9 +416,26 @@ def main_simulate_variance(argv=None):
     return ssquares, counts
 
 
+def parse_sc_ldpc_options(extra):
+    """Optional trailing arguments of ``main_simulate_sc_ldpc`` after the 13 positional ones of PD.py:1328-1340:
+    ``--frames-per-graph N`` (default 128) and ``--graphs-per-batch G`` (default 8).  Returns (frames_per_graph,
+    graphs_per_batch)."""
+    import argparse
+    ap = argparse.ArgumentParser(prog="ber_sim", description="options after the 13 positional arguments")
+    ap.add_argument("--frames-per-graph", type=int, default=128,
+                    help="frames decoded per graph realisation (from %d on: frame streams, any number)" % STREAM_MIN_FRAMES_PER_GRAPH)
+    ap.add_argument("--graphs-per-batch", type=int, default=8, help="graphs decoded at once per GPU")
+    a = ap.parse_args(list(extra))
+    if a.frames_per_graph < 1 or a.graphs_per_batch < 1:
+        ap.error("--frames-per-graph and --graphs-per-batch must be >= 1")
+    return a.frames_per_graph, a.graphs_per_batch
+
+
 def main_simulate_sc_ldpc(argv=None):
-    """argv: fname l r L M "es" T|N P|U B|U TB|NTB num_repeats max_fuckups "doping"  (PD.py:1328-1340)."""
+    """argv: fname l r L M "es" T|N P|U B|U TB|NTB num_repeats max_fuckups "doping"  (PD.py:1328-1340), optionally followed
+    by ``--frames-per-graph N`` and ``--graphs-per-batch G`` (``parse_sc_ldpc_options``)."""
     argv = sys.argv if argv is None else argv
+    fpg, gpb = parse_sc_ldpc_options(argv[14:])
     fname = argv[1]
     l = int(argv[2]); r = int(argv[3]); L = int(argv[4]); M = int(argv[5])
     es = eval(argv[6])
@@ -425,7 +457,8 @@ def main_simulate_sc_ldpc(argv=None):
         f.flush()
         for e in es:
             ber, ber_truncated, plr, plr_exp, fbl, tbl, fbit, tgen, _flrs, _gens, fblocks, tblocks, bler = simulate_sc_ldpc(
-                e, l, r, L, M, is_terminated, is_protograph, is_bounded, is_tail_biting, num_repeats, max_fuckups, doping_points)
+                e, l, r, L, M, is_terminated, is_protograph, is_bounded, is_tail_biting, num_repeats, max_fuckups, doping_points,
+                frames_per_graph=fpg, graphs_per_batch=gpb)
             print(e, ber, ber_truncated, plr, plr_exp, fbl, tbl, fbit, tgen, fblocks, tblocks, bler, file=f)
             if rank == 0:
                 print(e, ber, ber_truncated, plr, plr_exp, fbl, tbl, fbit, tgen, fblocks, tblocks, bler)

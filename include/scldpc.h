@@ -218,6 +218,26 @@ int scldpc_bp_stream_caps(const scldpc_dims_t *d, const scldpc_batch_t *b, const
                           const int32_t *caps_host, int n_caps, const scldpc_stream_caps_out_t *out,
                           void *workspace_dev, size_t workspace_bytes, long long *iters_launched_host, void *stream);
 
+/* Frame streams with stopping-set records: simulate_sc_ldpc (PD.py:591-701) on unlimited BP with lane recycling.  Each frame
+ * decodes to the peeling fixed point (the in-order sic_round scan, PD.py:656-657); its record is what
+ * scldpc_bp_stopping_sets returns for it (PD.py:659-691): (num_lost, any component with more than 2 VNs, VNs in such
+ * components, VN positions they touch), lost VNs being the erased VNs of the positions with counted_pos_host[p] != 0 (NULL =
+ * all).  unscanned_head_cns > 0 is is_bounded = False (PD.py:604-606, :656) as in scldpc_bp_full: a CN below it that starts a
+ * frame with exactly one erased neighbour never resolves it; it must not exceed the CNs the decoder sweeps
+ * ((L+dv-1)*cns_pos with SCLDPC_F_TERMINATED, L*cns_pos without).  Frame f of graph g is the frame scldpc_bp_stream decodes,
+ * and its iterations are what scldpc_bp_full(..., unscanned_head_cns) counts for it.  cfg->max_it must be 0 and
+ * SCLDPC_F_MESSAGES is not supported (node-state sweeps only).  The workspace comes from
+ * scldpc_bp_stream_stopping_sets_workspace_bytes. */
+typedef struct {
+    int32_t *iters_dev;     /* [G][B] iterations of each frame (unlimited BP)                                   */
+    int32_t *records_dev;   /* [G][B][4] (num_lost, big component?, VNs in big components, positions they touch) */
+} scldpc_stream_ss_out_t;
+size_t scldpc_bp_stream_stopping_sets_workspace_bytes(const scldpc_dims_t *d);
+int scldpc_bp_stream_stopping_sets(const scldpc_dims_t *d, const scldpc_batch_t *b, const scldpc_stream_cfg_t *cfg,
+                                   const uint8_t *counted_pos_host /* [L], NULL = all */, int unscanned_head_cns,
+                                   const scldpc_stream_ss_out_t *out, void *workspace_dev, size_t workspace_bytes,
+                                   long long *iters_launched_host, void *stream);
+
 /* scldpc_bp_stream with HOST buffers: graph tables vn_cn_host [G][n][dv] in, per-frame results int32
  * [G][frames_per_graph] out (any may be NULL); channel realisations are drawn on the device. */
 int scldpc_stream_host(const scldpc_dims_t *d, const int32_t *vn_cn_host, const scldpc_stream_cfg_t *cfg,
