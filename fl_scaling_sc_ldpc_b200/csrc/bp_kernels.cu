@@ -312,7 +312,7 @@ __global__ void __launch_bounds__(256) bp_pos_count_kernel(BpParams p)
     // a thread keeps its chunk (blockDim and the stride are multiples of ch); chunks without a selected lane are skipped.
     // Streams with checkpoints also count the frames paused at a checkpoint.
     u128 mask = p.lane_mask ? reinterpret_cast<const u128 *>(p.lane_mask)[g * ch + (threadIdx.x & (ch - 1))] : ones128();
-    if (p.pause_mask) mask |= reinterpret_cast<const u128 *>(p.pause_mask)[g * ch + (threadIdx.x & (ch - 1))];
+    if (p.stream_mode == SM_CKPT) mask |= reinterpret_cast<const u128 *>(p.pause_mask)[g * ch + (threadIdx.x & (ch - 1))];
     if (nz(mask))
         for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < items; idx += gridDim.x * blockDim.x) {
             const u128 xv = x[idx] & mask;
@@ -544,7 +544,7 @@ static void launch_count_pairs(const BpParams &p, cudaStream_t st)
         q.lane_mask = p.done_mask;                              // every stopped frame is counted; the failed ones land in fail_mask
         bp_pos_count_kernel<<<dim3(bx, p.L, graphs_in_grid(p)), 256, 0, st>>>(q);
     } else bp_pos_count_kernel<<<dim3(bx, p.L, graphs_in_grid(p)), 256, 0, st>>>(p);
-    if (p.ss_records) {                                         // streams with stopping-set records classify instead (ss_launch_stream)
+    if (p.stream_mode == SM_HEAD) {                             // streams with stopping-set records classify instead (ss_launch_stream)
         g_prof.launches += 1;
         return;
     }

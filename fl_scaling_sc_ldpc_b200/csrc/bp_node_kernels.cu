@@ -32,21 +32,6 @@
 // Useful work is still accounted as the reference's: 2E edge updates per frame-iteration.
 #include "common.cuh"
 
-// NS_VARIANT: timing experiments only (tools/build_variants.sh); bits: 1 = ld.cg gathers instead of ld.nc.L1::no_allocate
-// (measured: +8 us per launch), 2 = no list stores, 4 = no replay, 8 = no prefix sum.  Variants 2, 4 and 8 decode wrongly by
-// construction (the planes drift apart), so their timings only bound the cost of the part they leave out.
-// 16 = wave instrumentation (tools/wave_skip_measure.py): per iteration, how many (CN position, 128-lane chunk) pairs could a
-// sweep skip because no VN of the dv positions feeding them was resolved in the previous iteration (VERDICT r1 item 5).
-#ifndef NS_VARIANT
-#define NS_VARIANT 0
-#endif
-// NS_PREFETCH = 1 fetches the index row of the next trip while this trip's gathers are in flight.  The row load is 16 % of the
-// stall samples (profiles/r02c), but with 32 resident warps per SM other warps cover it: measured 52.2 us per launch with the
-// prefetch against 50.1 us without (gpurun_out/r2d_variants.log) -- off.
-#ifndef NS_PREFETCH
-#define NS_PREFETCH 0
-#endif
-
 namespace scldpc {
 
 // ------------------------------------------------------------------------------------------------------------
@@ -56,20 +41,20 @@ namespace scldpc {
 // Resolutions are sparse (a VN is resolved once per frame; about 0.5 per thread and trip), so the scatter is a short divergent
 // loop; the index of the neighbour to clear is carried in bit planes next to the saturating count.
 // The sweep is bound by L2 latency and instruction issue, not by HBM (DESIGN.md section 4).
-// CAPPED (streams with an iteration cap): a frame that hit the cap is not at a fixed point, so its bits must not be cleared
+// M is the stream mode (common.cuh); SM_PLAIN streams run unlimited BP and nothing more.
+// SM_CAPPED (streams with an iteration cap): a frame that hit the cap is not at a fixed point, so its bits must not be cleared
 // while it waits for the harvest -- the resolutions are masked with the frames still iterating.
-// CKPT (streams with checkpoints, CAPPED as well): a frame that reaches its next checkpoint caps[lane_ck] without stopping
+// SM_CKPT (streams with checkpoints, capped as well): a frame that reaches its next checkpoint caps[lane_ck] without stopping
 // in that iteration pauses -- it leaves active for pause_mask, not done_mask -- and the harvest records its statistics and
 // puts it back into active.  A paused lane is masked like a capped one, and its lane_iter does not advance.
-// HEAD (streams with stopping-set records, unlimited): the unscanned head of simulate_sc_ldpc with is_bounded = False, per lane.
-// A CN below cn_dis_lim that starts a frame with exactly one erased neighbour never resolves it (bpw_iter_kernel<.,.,HEAD>);
+// SM_HEAD (streams with stopping-set records, unlimited): the unscanned head of simulate_sc_ldpc with is_bounded = False, per
+// lane.  A CN below cn_dis_lim that starts a frame with exactly one erased neighbour never resolves it (bpw_iter_kernel<.,.,HEAD>);
 // "starts" is the frame's first iteration, the launch after the harvest that armed its lane (head_arm), so the cn_dis bits of
 // the armed lanes are set there and every other lane keeps its own.
-template <int DV, int DC, bool CAPPED, bool CKPT = false, bool HEAD = false>
+template <int DV, int DC, StreamMode M>
 __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
 {
-    static_assert(CAPPED || !CKPT, "a paused frame must not be cleared");
-    static_assert(!(HEAD && CAPPED), "the unscanned head is an unlimited-decoder rule");
+    constexpr bool CAPPED = M == SM_CAPPED || M == SM_CKPT;     // resolutions masked with the frames still iterating
     static_assert(DC <= 16, "neighbour index is encoded in four bit planes");
     pdl_wait_then_release();
     const int g = graph_of(p, blockIdx.y);
@@ -94,7 +79,7 @@ __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
 
     // ---- the write plane catches up with the previous iteration ----
     if (ld_cg(p.nl_ovf + g * 2 + (par ^ 1))) ns_catch_up(rd, wr, 0, p.n << p.chunk_shift);
-    else if (!(NS_VARIANT & 4)) ns_replay_region(p, g, par ^ 1, wr32, rid, false);
+    else ns_replay_region(p, g, par ^ 1, wr32, rid, false);
 
     // ---- check-node sweep ----
     const u128 act = reinterpret_cast<const u128 *>(p.active)[g * ch + k];
@@ -106,23 +91,16 @@ __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
     const int stride = gridDim.x * blockDim.x;
     int wcount = 0;                                             // entries this warp has logged (warp-uniform)
     u128 acc_new = zero128();
-    // the index row of the NEXT trip is fetched while this trip's gathers are in flight (the row load was 16 % of the stall
-    // samples as a dependent step in front of the gathers: profiles/r02c)
-    int e[DC];
-    {
-        const int idx0 = blockIdx.x * blockDim.x + threadIdx.x;
-        if (NS_PREFETCH && lane_work && idx0 < items) load_row<DC>(cn_row + (size_t)(idx0 >> cs) * DC, e);
-    }
     for (int base = blockIdx.x * blockDim.x + (threadIdx.x & ~31); base < items; base += stride) {
         const int idx = base + lane;
         u128 res = zero128(), b0 = zero128(), b1 = zero128(), b2 = zero128(), b3 = zero128();
         const int32_t *row = cn_row + (size_t)(idx >> cs) * DC;
         if (lane_work && idx < items) {
-            if (!NS_PREFETCH) load_row<DC>(row, e);
+            int e[DC];
+            load_row<DC>(row, e);
             u128 in[DC];
 #pragma unroll
-            for (int j = 0; j < DC; j++) in[j] = (NS_VARIANT & 1) ? ld_cg128(rdk + (unsigned)e[j]) : ld_stream(rdk + (unsigned)e[j]);
-            if (NS_PREFETCH && idx + stride < items) load_row<DC>(row + (size_t)(stride >> cs) * DC, e);
+            for (int j = 0; j < DC; j++) in[j] = ld_stream(rdk + (unsigned)e[j]);
             // saturating count of erased neighbours (one / two planes) and, in bit planes b0..b3, the index j of an erased
             // neighbour -- exact where it is needed, i.e. in the frames with exactly one
             u128 one = zero128(), tw = zero128();
@@ -137,7 +115,7 @@ __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
             }
             res = one & ~tw;                                    // frames in which exactly one neighbour of c is erased
             if (CAPPED) res &= act;
-            if (HEAD && (idx >> cs) < p.cn_dis_lim) {
+            if (M == SM_HEAD && (idx >> cs) < p.cn_dis_lim) {
                 // one 64-bit half at a time, with 32-bit word offsets (the plane offsets are below 2^32, see capi.cu): the u128
                 // merge with 64-bit pointers spilled the (4,12) and (3,9) sweeps
                 const unsigned dw = 2u * (((unsigned)g * (unsigned)p.cn_dis_lim + (unsigned)(idx >> cs)) * (unsigned)ch + (unsigned)k);
@@ -153,23 +131,18 @@ __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
                     r &= ~nd;
                 }
             }
-#if NS_VARIANT & 16
-            if (nz(res)) reinterpret_cast<int *>(p.pos_er)[((size_t)g * (p.L + DV - 1) + (idx >> cs) / p.cns_pos) * ch + k] = p.iter + 1;
-#endif
         }
         if (__ballot_sync(0xffffffffu, nz(res)) == 0u) continue;
         // slots of this trip's resolutions in the warp's region: exclusive prefix sum of the per-thread counts
         const int c = __popcll(res.x) + __popcll(res.y);
         int incl = c;
-        if (!(NS_VARIANT & 8)) {
 #pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const int t = __shfl_up_sync(0xffffffffu, incl, o);
-                if (lane >= o) incl += t;
-            }
+        for (int o = 1; o < 32; o <<= 1) {
+            const int t = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += t;
         }
         int slot = wcount + incl - c;
-        if (!(NS_VARIANT & 8)) wcount += __shfl_sync(0xffffffffu, incl, 31);
+        wcount += __shfl_sync(0xffffffffu, incl, 31);
         if (c) {
             acc_new |= res;
             const unsigned rw[4] = {(unsigned)res.x, (unsigned)(res.x >> 32), (unsigned)res.y, (unsigned)(res.y >> 32)};
@@ -187,7 +160,7 @@ __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
                     if (DC > 8) j |= ((w3[q] >> b) & 1u) << 3;
                     const unsigned widx = 4u * ((unsigned)__ldg(row + j) + (unsigned)k) + (unsigned)q;   // L1 hit
                     red_and(wr32 + widx, ~(1u << b));
-                    if (!(NS_VARIANT & 2) && slot < p.nl_cap) st_cg_u2(reg + slot, make_uint2(widx, 1u << b));
+                    if (slot < p.nl_cap) st_cg_u2(reg + slot, make_uint2(widx, 1u << b));
                     slot++;
                 }
             }
@@ -215,11 +188,11 @@ __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
     __threadfence();
     // ---- end of the iteration for graph g ----
     __shared__ u64 s_act[SCLDPC_MAX_WORDS], s_cap[SCLDPC_MAX_WORDS];
-    __shared__ u64 s_ck[CKPT ? SCLDPC_MAX_WORDS : 1];
+    __shared__ u64 s_ck[M == SM_CKPT ? SCLDPC_MAX_WORDS : 1];
     const int W = p.W;
     for (int w = threadIdx.x; w < W; w += blockDim.x) {
         s_act[w] = p.active[g * W + w]; s_cap[w] = 0;
-        if (CKPT) s_ck[w] = 0;
+        if (M == SM_CKPT) s_ck[w] = 0;
     }
     __syncthreads();
     for (int l = threadIdx.x; l < p.lanes; l += blockDim.x) {
@@ -228,7 +201,7 @@ __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
             const int li = p.lane_iter[g * p.lanes + l] + 1;
             p.lane_iter[g * p.lanes + l] = li;
             if (CAPPED && li >= p.stream_cap) atomicOr(reinterpret_cast<unsigned long long *>(&s_cap[w]), 1ull << b);   // while (iter < MaxNumIt)
-            else if (CKPT) {
+            else if (M == SM_CKPT) {
                 const int ck = p.lane_ck[g * p.lanes + l];
                 if (ck < p.n_caps - 1 && li >= p.caps[ck]) atomicOr(reinterpret_cast<unsigned long long *>(&s_ck[w]), 1ull << b);
             }
@@ -241,7 +214,7 @@ __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
         // channel left some VN known (first_new)
         const u64 nw = ld_cg(p.any_new + g * W + w) | ld_cg(p.first_new + g * W + w);
         const u64 stop = a & (~nw | s_cap[w]);                  // NumErasures == NumErasuresPrec (or == 0, one iteration late) || cap
-        if (CKPT) {
+        if (M == SM_CKPT) {
             const u64 pause = s_ck[w] & ~stop;                  // a frame that stops at a checkpoint stops
             p.active[g * W + w] = a & ~stop & ~pause;
             if (pause) p.pause_mask[g * W + w] |= pause;
@@ -252,25 +225,6 @@ __global__ void __launch_bounds__(32 * NS_WARPS, 4) ns_iter_kernel(BpParams p)
         p.any_new[g * W + w] = 0;
         p.first_new[g * W + w] = 0;
     }
-#if NS_VARIANT & 16
-    {
-        // a CN position must be swept in the next iteration iff a resolution happened within dv-1 positions of it (the resolved
-        // VN sits up to dv-1 positions below the resolving CN and feeds CNs up to dv-1 positions above itself)
-        const int *stamp = reinterpret_cast<const int *>(p.pos_er) + (size_t)g * (p.L + DV - 1) * ch;
-        int needed = 0, total = 0;
-        for (int i = threadIdx.x; i < p.cn_pos_lim * ch; i += blockDim.x) {
-            const int q = i / ch, kk = i % ch;
-            if (!(s_act[2 * kk] | s_act[2 * kk + 1])) continue;
-            total++;
-            bool need = false;
-            for (int d = -(DV - 1); d <= DV - 1; d++)
-                if (q + d >= 0 && q + d < p.L + DV - 1 && stamp[(q + d) * ch + kk] == p.iter + 1) need = true;
-            needed += need;
-        }
-        atomicAdd(reinterpret_cast<unsigned long long *>(p.swept + 2 * g), (unsigned long long)needed);
-        atomicAdd(reinterpret_cast<unsigned long long *>(p.swept + 2 * g + 1), (unsigned long long)total);
-    }
-#endif
     if (threadIdx.x == 0) {
         p.nl_ovf[g * 2 + (par ^ 1)] = 0;                        // consumed by every block of this launch
         p.ticket[g] = 0;
@@ -437,14 +391,14 @@ __global__ void ns_compact_plan_kernel(BpParams p)
             p.cmp_src[g * p.lanes + i] = l;
             s_fr[i] = p.lane_frame[g * p.lanes + l];
             s_it[i] = p.lane_iter[g * p.lanes + l];
-            if (p.lane_ck) s_ck[i] = p.lane_ck[g * p.lanes + l];
+            if (p.stream_mode == SM_CKPT) s_ck[i] = p.lane_ck[g * p.lanes + l];
         }
     }
     __syncthreads();
     for (int l = threadIdx.x; l < p.lanes; l += blockDim.x) {
         p.lane_frame[g * p.lanes + l] = l < A ? s_fr[l] : -1;
         p.lane_iter[g * p.lanes + l] = l < A ? s_it[l] : 0;
-        if (p.lane_ck) p.lane_ck[g * p.lanes + l] = l < A ? s_ck[l] : 0;
+        if (p.stream_mode == SM_CKPT) p.lane_ck[g * p.lanes + l] = l < A ? s_ck[l] : 0;
     }
     for (int w = threadIdx.x; w < W; w += blockDim.x)
         p.active[g * W + w] = A >= 64 * (w + 1) ? ~0ull : (A <= 64 * w ? 0ull : ((1ull << (A - 64 * w)) - 1ull));
@@ -453,10 +407,8 @@ __global__ void ns_compact_plan_kernel(BpParams p)
         while ((128 << s) < A) s++;
         p.gshift[g] = s;
         p.cmp_cnt[g] = A;
-#if !(NS_VARIANT & 16)
         p.swept[2 * g] += 1;                                    // scldpc_bp_sweep_stats on a stream workspace: compactions, lanes moved
         p.swept[2 * g + 1] += A;
-#endif
     }
 }
 
@@ -474,7 +426,7 @@ __global__ void __launch_bounds__(256) ns_compact_kernel(BpParams p)
     unsigned *out32 = reinterpret_cast<unsigned *>(s_out);
     // tiles of the two planes' rows, then (streams with an unscanned head) of the cn_dis rows, which are per-lane decoder state too
     const int t_planes = (p.n + CMP_ROWS - 1) / CMP_ROWS;
-    const int t_all = t_planes + (p.cn_dis ? (p.cn_dis_lim + CMP_ROWS - 1) / CMP_ROWS : 0);
+    const int t_all = t_planes + (p.stream_mode == SM_HEAD ? (p.cn_dis_lim + CMP_ROWS - 1) / CMP_ROWS : 0);
     for (int t = blockIdx.x; t < t_all; t += gridDim.x) {
         const bool dis = t >= t_planes;
         const int row0 = (dis ? t - t_planes : t) * CMP_ROWS;
@@ -536,7 +488,7 @@ static dim3 node_grid(const BpParams &p)
     const int block = 32 * NS_WARPS;
     static int res = 0;
     if (!res) {
-        res = resident_blocks(ns_iter_kernel<DV, DC, false>, block);
+        res = resident_blocks(ns_iter_kernel<DV, DC, SM_PLAIN>, block);
         if (res > NS_MAX_BLOCKS) res = NS_MAX_BLOCKS;
     }
     long long need = (((long long)p.cn_pos_lim * p.cns_pos << p.chunk_shift) + block - 1) / block;
@@ -554,10 +506,14 @@ static void launch_node_iteration(const BpParams &p, bool after_harvest, cudaStr
     g_prof.launches += 1;
     // the first launch after a harvest follows ordinary kernels: full serialisation there
     const bool pdl = !after_harvest && !sample;
-    if (p.n_caps > 0) launch_pdl(ns_iter_kernel<DV, DC, true, true>, grid, block, st, pdl, p);
-    else if (p.stream_cap > 0) launch_pdl(ns_iter_kernel<DV, DC, true>, grid, block, st, pdl, p);
-    else if (p.cn_dis_lim > 0) launch_pdl(ns_iter_kernel<DV, DC, false, false, true>, grid, block, st, pdl, p);
-    else launch_pdl(ns_iter_kernel<DV, DC, false>, grid, block, st, pdl, p);
+    switch (p.stream_mode) {
+    case SM_CAPPED: launch_pdl(ns_iter_kernel<DV, DC, SM_CAPPED>, grid, block, st, pdl, p); break;
+    case SM_CKPT: launch_pdl(ns_iter_kernel<DV, DC, SM_CKPT>, grid, block, st, pdl, p); break;
+    case SM_HEAD:
+        if (p.cn_dis_lim > 0) { launch_pdl(ns_iter_kernel<DV, DC, SM_HEAD>, grid, block, st, pdl, p); break; }
+        [[fallthrough]];                                        // an empty head (is_bounded = True) leaves plain BP
+    case SM_PLAIN: launch_pdl(ns_iter_kernel<DV, DC, SM_PLAIN>, grid, block, st, pdl, p); break;
+    }
     if (sample) {
         cudaEventRecord(ev[1], st);
         cudaEventRecord(ev[2], st);                             // one kernel per iteration: the second interval is empty

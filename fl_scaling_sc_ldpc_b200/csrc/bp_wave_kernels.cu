@@ -513,6 +513,7 @@ __global__ void bp_stream_harvest_kernel(BpParams p, int exp_all)
 {
     const int g = graph_of(p, blockIdx.x), L = p.L, W = p.W, B = p.frames_per_graph;
     if (ld_cg(p.alive + g) == 0) return;
+    const bool stats = p.stream_mode != SM_HEAD;                // streams with stopping-set records store iters only
     __shared__ int s_rank[SCLDPC_MAX_WORDS + 1];
     __shared__ u64 s_done[SCLDPC_MAX_WORDS], s_arm[SCLDPC_MAX_WORDS];
     __shared__ u64 s_pause[CKPT ? SCLDPC_MAX_WORDS : 1];
@@ -563,7 +564,7 @@ __global__ void bp_stream_harvest_kernel(BpParams p, int exp_all)
             e_exp += __shfl_xor_sync(0xffffffffu, e_exp, o);
             b_exp += __shfl_xor_sync(0xffffffffu, b_exp, o);
         }
-        if ((threadIdx.x & 31) == 0 && fr >= 0 && fr < B && p.s_residual) {     // (streams with stopping-set records: iters only)
+        if ((threadIdx.x & 31) == 0 && fr >= 0 && fr < B && stats) {
             const size_t o = (size_t)g * B + fr;
             if (CKPT) {
                 const int k0 = p.lane_ck[g * p.lanes + l];
@@ -595,7 +596,7 @@ __global__ void bp_stream_harvest_kernel(BpParams p, int exp_all)
             p.s_iters[o] = its;
             atomicAdd(&s_frames, 1);
             atomicAdd(&s_its, (unsigned long long)its);
-            if (!((p.fail_mask[g * W + w] >> b) & 1ull) && p.s_residual) {
+            if (!((p.fail_mask[g * W + w] >> b) & 1ull) && stats) {
                 if (CKPT) store_ck_slots(p, o, p.lane_ck[g * p.lanes + l], p.n_caps, 0, 0, 0, 0);
                 else {
                     p.s_residual[o] = 0;
@@ -763,7 +764,7 @@ void bp_launch_stream_harvest(const BpParams &p, int exp_all, cudaStream_t st)
 {
     g_prof.launches += 1;
     // one warp per failed frame: 32 at a time
-    if (p.n_caps > 0) bp_stream_harvest_kernel<true><<<graphs_in_grid(p), 1024, 0, st>>>(p, exp_all);
+    if (p.stream_mode == SM_CKPT) bp_stream_harvest_kernel<true><<<graphs_in_grid(p), 1024, 0, st>>>(p, exp_all);
     else bp_stream_harvest_kernel<false><<<graphs_in_grid(p), 1024, 0, st>>>(p, exp_all);
 }
 

@@ -180,12 +180,10 @@ static size_t list_stride(size_t max_nodes, size_t ch)
     return s;
 }
 
-// internal: workspace of scldpc_bp_stream_caps (per-lane checkpoint state on top of the node-state stream's)
-#define F_CAPS_WS 0x10000u
-// internal: workspace of scldpc_bp_stream_stopping_sets (unscanned-head plane and stopping-set accumulators on top of it)
-#define F_SS_WS 0x20000u
-
-static size_t carve(const scldpc_dims_t *d, uint32_t flags, void *ws, BpParams *p)
+// Workspace layout of a decoder call with `flags`; a frame stream (SCLDPC_F_STREAM) of mode SM_CKPT or SM_HEAD adds its
+// per-lane state at the end.  Every region before those keeps its offset whatever the mode, so that scldpc_bp_sweep_stats and
+// scldpc_bp_position_counts, which re-carve with the caller's flags, find their counters on every stream workspace.
+static size_t carve(const scldpc_dims_t *d, uint32_t flags, StreamMode mode, void *ws, BpParams *p)
 {
     const size_t G = d->n_graphs, W = d->n_words, ch = W / 2, lanes = 64 * W;
     const size_t n = (size_t)d->L * d->vns_pos, nk = (size_t)(d->L + d->dv - 1) * d->cns_pos, E = n * d->dv;
@@ -245,15 +243,16 @@ static size_t carve(const scldpc_dims_t *d, uint32_t flags, void *ws, BpParams *
             q.gshift = c.take<int>(G);
             q.cmp_cnt = c.take<int>(G);
             q.cmp_src = c.take<int>(G * lanes);
-            if (flags & F_CAPS_WS) {
+            if (mode == SM_CKPT) {
                 q.lane_ck = c.take<int>(G * lanes);
                 q.pause_mask = c.take<u64>(G * W);
             }
         }
     }
-    q.cn_dis = (flags & SCLDPC_F_STREAM) ? nullptr : c.take<u128>(G * nk * ch);   // sized for the largest possible ignored head
-    if ((flags & F_SS_WS) && no_msgs) {
-        q.cn_dis = c.take<u128>(G * nk * ch);                         // as the synchronous path's
+    // the unscanned head of the synchronous decoders and of streams with stopping-set records, sized for the largest possible head
+    const bool head = !(flags & SCLDPC_F_STREAM) || mode == SM_HEAD;
+    q.cn_dis = head ? c.take<u128>(G * nk * ch) : nullptr;
+    if (mode == SM_HEAD) {
         q.ss_lost = c.take<int>(G * d->L * lanes);
         q.ss_big = c.take<int>(G * d->L * lanes);
         q.ss_counted = c.take<unsigned char>(d->L);
@@ -278,7 +277,7 @@ static size_t carve(const scldpc_dims_t *d, uint32_t flags, void *ws, BpParams *
 extern "C" size_t scldpc_bp_workspace_bytes(const scldpc_dims_t *d, uint32_t flags)
 {
     if (check_dims(d)) return 0;
-    return carve(d, flags, nullptr, nullptr);
+    return carve(d, flags, SM_PLAIN, nullptr, nullptr);
 }
 
 static int setup_params(const scldpc_dims_t *d, const scldpc_batch_t *b, uint32_t flags, const scldpc_bp_out_t *out,
@@ -294,10 +293,10 @@ static int setup_params(const scldpc_dims_t *d, const scldpc_batch_t *b, uint32_
     if ((flags & SCLDPC_F_TRAJECTORY) && (!out->rows_dev || out->max_rows <= 0))
         return fail(SCLDPC_EINVAL, "trajectory mode needs rows_dev and max_rows > 0");
     if (!ws) return fail(SCLDPC_EINVAL, "workspace is NULL");
-    const size_t need = carve(d, flags, nullptr, nullptr);
+    const size_t need = carve(d, flags, SM_PLAIN, nullptr, nullptr);
     if (ws_bytes < need) return fail(SCLDPC_ENOMEM, "workspace too small: %zu < %zu bytes", ws_bytes, need);
     if ((rc = have_device())) return rc;
-    carve(d, flags, ws, p);
+    carve(d, flags, SM_PLAIN, ws, p);
     p->dv = d->dv; p->dc = d->dc;
     p->n = d->L * d->vns_pos;
     p->nk = (d->L + d->dv - 1) * d->cns_pos;
@@ -594,56 +593,66 @@ extern "C" int scldpc_bp_full(const scldpc_dims_t *d, const scldpc_batch_t *b, i
 extern "C" size_t scldpc_bp_stream_workspace_bytes(const scldpc_dims_t *d, uint32_t flags)
 {
     if (check_dims(d)) return 0;
-    return carve(d, SCLDPC_F_STREAM | (flags & SCLDPC_F_MESSAGES), nullptr, nullptr);
+    return carve(d, SCLDPC_F_STREAM | (flags & SCLDPC_F_MESSAGES), SM_PLAIN, nullptr, nullptr);
 }
 
 extern "C" size_t scldpc_bp_stream_caps_workspace_bytes(const scldpc_dims_t *d)
 {
     if (check_dims(d)) return 0;
-    return carve(d, SCLDPC_F_STREAM | F_CAPS_WS, nullptr, nullptr);
+    return carve(d, SCLDPC_F_STREAM, SM_CKPT, nullptr, nullptr);
 }
 
 extern "C" size_t scldpc_bp_stream_stopping_sets_workspace_bytes(const scldpc_dims_t *d)
 {
     if (check_dims(d)) return 0;
-    return carve(d, SCLDPC_F_STREAM | F_SS_WS, nullptr, nullptr);
+    return carve(d, SCLDPC_F_STREAM, SM_HEAD, nullptr, nullptr);
 }
 
-// stopping-set records of scldpc_bp_stream_stopping_sets
-struct StreamSs {
-    const uint8_t *counted_pos_host;   // [L] or NULL (all positions)
+// What a stream mode takes beyond scldpc_stream_cfg_t; the entry point of the mode has validated it.
+struct StreamInputs {
+    const int32_t *caps;               // SM_CKPT: [n_caps] ascending iteration caps
+    int n_caps;
+    const uint8_t *counted_pos_host;   // SM_HEAD: [L] or NULL (all positions)
     int unscanned_head_cns;
-    int32_t *records_dev;              // [G][B][4]
+    int32_t *records_dev;              // SM_HEAD: [G][B][4]
 };
 
-// Frame stream of scldpc_bp_stream (n_caps == 0: `out` holds the [G][B] results), scldpc_bp_stream_caps (n_caps >= 1:
-// `out` holds iters [G][B] and the [K][G][B] statistics; the caps are validated by the caller) or
-// scldpc_bp_stream_stopping_sets (ss != NULL: `out` holds iters only, the records go to ss->records_dev).
-static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const scldpc_stream_cfg_t *cfg, const int32_t *caps,
-                          int n_caps, const StreamSs *ss, const scldpc_stream_out_t *out, void *workspace_dev,
-                          size_t workspace_bytes, long long *iters_launched_host, void *stream)
+// The frame stream behind the three entry points below.  `out` holds the [G][B] results (SM_PLAIN, which becomes SM_CAPPED
+// when cfg->max_it > 0), iters [G][B] and the [K][G][B] statistics (SM_CKPT) or iters only (SM_HEAD: the records go to
+// in.records_dev).
+static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const scldpc_stream_cfg_t *cfg, StreamMode mode,
+                          const StreamInputs &in, const scldpc_stream_out_t *out, void *workspace_dev, size_t workspace_bytes,
+                          long long *iters_launched_host, void *stream)
 {
+    if (!cfg) return fail(SCLDPC_EINVAL, "bad stream configuration");
+    if (mode == SM_CKPT && cfg->max_it != 0) return fail(SCLDPC_EINVAL, "cfg->max_it must be 0 with caps: the caps replace it");
+    if (mode == SM_HEAD && cfg->max_it != 0) return fail(SCLDPC_EINVAL, "cfg->max_it must be 0: stopping sets are records of unlimited BP");
+    if (mode == SM_PLAIN && cfg->max_it > 0) mode = SM_CAPPED;
+    // SCLDPC_F_MESSAGES selects the message-passing sweeps (the implementation of record), for unlimited streams only; the
+    // default is the node-state formulation of bp_node_kernels.cu, which yields the same erased set at every iteration with
+    // ~6x less HBM traffic
+    const bool node = !(cfg->flags & SCLDPC_F_MESSAGES);
+    static const char *const node_only[] = {"", "capped frame streams", "frame streams with caps", "frame streams with stopping sets"};
+    if (!node && mode != SM_PLAIN) return fail(SCLDPC_EINVAL, "%s need the node-state sweeps (no SCLDPC_F_MESSAGES)", node_only[mode]);
     int rc = check_dims(d);
     if (rc) return rc;
     if (!degrees_supported(d->dv, d->dc)) return fail(SCLDPC_EINVAL, "(dv,dc)=(%d,%d) not instantiated", d->dv, d->dc);
     if (!b || !b->vn_cn_dev || !b->vn_slot_dev || !b->cn_edge_dev) return fail(SCLDPC_EINVAL, "batch pointer is NULL");
-    if (!cfg || !cfg->eps_host || cfg->frames_per_graph < 1) return fail(SCLDPC_EINVAL, "bad stream configuration");
+    if (!cfg->eps_host || cfg->frames_per_graph < 1) return fail(SCLDPC_EINVAL, "bad stream configuration");
     if (!out || !out->iters_dev ||
-        (!ss && (!out->residual_dev || !out->blocks_err_dev || !out->erasures_exp_dev || !out->blocks_err_exp_dev)))
+        (mode != SM_HEAD && (!out->residual_dev || !out->blocks_err_dev || !out->erasures_exp_dev || !out->blocks_err_exp_dev)))
         return fail(SCLDPC_EINVAL, "output pointer is NULL");
     if (d->n_frames < 1) return fail(SCLDPC_EINVAL, "n_frames (lanes used per graph) must be >= 1");
-    if ((cfg->flags & SCLDPC_F_MESSAGES) && d->L + d->dv - 1 > 1024) return fail(SCLDPC_EINVAL, "chain too long for the message-passing stream");
+    if (!node && d->L + d->dv - 1 > 1024) return fail(SCLDPC_EINVAL, "chain too long for the message-passing stream");
     if (!workspace_dev) return fail(SCLDPC_EINVAL, "workspace is NULL");
-    // SCLDPC_F_MESSAGES selects the message-passing sweeps (the implementation of record); the default is the node-state
-    // formulation of bp_node_kernels.cu, which yields the same erased set at every iteration with ~6x less HBM traffic
-    const bool node = !(cfg->flags & SCLDPC_F_MESSAGES);
-    const uint32_t wflags = SCLDPC_F_STREAM | (cfg->flags & SCLDPC_F_MESSAGES) | (n_caps > 0 ? F_CAPS_WS : 0u) | (ss ? F_SS_WS : 0u);
-    const size_t need = carve(d, wflags, nullptr, nullptr);
+    const uint32_t wflags = SCLDPC_F_STREAM | (cfg->flags & SCLDPC_F_MESSAGES);
+    const size_t need = carve(d, wflags, mode, nullptr, nullptr);
     if (workspace_bytes < need) return fail(SCLDPC_ENOMEM, "workspace too small: %zu < %zu bytes", workspace_bytes, need);
     if ((rc = have_device())) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     BpParams p;
-    carve(d, wflags, workspace_dev, &p);
+    carve(d, wflags, mode, workspace_dev, &p);
+    p.stream_mode = mode;
     p.dv = d->dv; p.dc = d->dc;
     p.n = d->L * d->vns_pos; p.nk = (d->L + d->dv - 1) * d->cns_pos; p.E = p.n * d->dv;
     p.L = d->L; p.vns_pos = d->vns_pos; p.cns_pos = d->cns_pos;
@@ -661,22 +670,25 @@ static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const
     p.c0 = 0; p.c1 = p.cn_pos_lim * d->cns_pos; p.v0 = 0; p.v1 = p.n;
     p.max_it = INT_MAX; p.first_iter = 0; p.stall_at_first = 1;
     p.frames_per_graph = cfg->frames_per_graph; p.seed = cfg->seed; p.first_graph = cfg->first_graph_id;
-    p.stream_cap = cfg->max_it > 0 ? cfg->max_it : 0;
-    p.n_caps = n_caps;
-    for (int k = 0; k < n_caps; k++) p.caps[k] = caps[k];
-    if (n_caps > 0) p.stream_cap = caps[n_caps - 1] > 0 ? caps[n_caps - 1] : INT_MAX;
+    p.stream_cap = mode == SM_CAPPED ? cfg->max_it : 0;
+    if (mode == SM_CKPT) {
+        p.n_caps = in.n_caps;
+        for (int k = 0; k < in.n_caps; k++) p.caps[k] = in.caps[k];
+        p.stream_cap = in.caps[in.n_caps - 1] > 0 ? in.caps[in.n_caps - 1] : INT_MAX;
+    }
     p.s_iters = out->iters_dev; p.s_residual = out->residual_dev; p.s_blocks_err = out->blocks_err_dev;
     p.s_erasures_exp = out->erasures_exp_dev; p.s_blocks_err_exp = out->blocks_err_exp_dev;
     p.lane_mask = p.fail_mask;                   // frames that stopped without erasures have all-zero counts already
     p.lazy_success = node ? 1 : 0;
     std::vector<unsigned char> counted;
-    if (ss) {
-        if (ss->unscanned_head_cns < 0 || ss->unscanned_head_cns > p.c1)
-            return fail(SCLDPC_EINVAL, "unscanned_head_cns must be in [0, %d] (the CNs the decoder sweeps), got %d", p.c1, ss->unscanned_head_cns);
-        p.cn_dis_lim = ss->unscanned_head_cns;
-        p.ss_records = ss->records_dev;
+    if (mode == SM_HEAD) {
+        // (checked here rather than by scldpc_bp_stream_stopping_sets: the range is the CNs the decoder sweeps)
+        if (in.unscanned_head_cns < 0 || in.unscanned_head_cns > p.c1)
+            return fail(SCLDPC_EINVAL, "unscanned_head_cns must be in [0, %d] (the CNs the decoder sweeps), got %d", p.c1, in.unscanned_head_cns);
+        p.cn_dis_lim = in.unscanned_head_cns;
+        p.ss_records = in.records_dev;
         counted.assign(d->L, 1);
-        if (ss->counted_pos_host) counted.assign(ss->counted_pos_host, ss->counted_pos_host + d->L);
+        if (in.counted_pos_host) counted.assign(in.counted_pos_host, in.counted_pos_host + d->L);
     }
     // per-graph channel thresholds and the doping profile
     std::vector<u64> thr(d->n_graphs);
@@ -691,14 +703,13 @@ static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const
     CU(cudaMemcpyAsync(const_cast<u64 *>(p.thr), thr.data(), sizeof(u64) * thr.size(), cudaMemcpyHostToDevice, st));
     if (doped) CU(cudaMemcpyAsync(const_cast<int32_t *>(p.known), known.data(), sizeof(int32_t) * d->L, cudaMemcpyHostToDevice, st));
     else p.known = nullptr;
-    if (ss) {
+    if (mode == SM_HEAD) {
         CU(cudaMemcpyAsync(const_cast<unsigned char *>(p.ss_counted), counted.data(), d->L, cudaMemcpyHostToDevice, st));
         CU(cudaMemsetAsync(p.ss_lost, 0, sizeof(int) * (size_t)p.G * d->L * p.lanes, st));
         CU(cudaMemsetAsync(p.ss_big, 0, sizeof(int) * (size_t)p.G * d->L * p.lanes, st));
         CU(cudaMemsetAsync(p.cn_dis, 0, sizeof(u128) * (size_t)p.G * p.nk * p.chunks, st));
     }
     CU(cudaStreamSynchronize(st));               // host vectors leave scope at return; keep it simple
-    if (!node && p.stream_cap > 0) return fail(SCLDPC_EINVAL, "capped frame streams need the node-state sweeps (no SCLDPC_F_MESSAGES)");
     // state: no lane holds a frame yet.  Message sweeps: Lij = 1 (tail CNs of a truncated code are never swept), the rest 0
     const size_t ch = p.chunks, plane = ((size_t)p.G * p.n + 1) * ch;
     CU(cudaMemsetAsync(p.x, 0, sizeof(u128) * plane, st));
@@ -709,9 +720,9 @@ static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const
         CU(cudaMemsetAsync(p.noprog, 0, sizeof(u64) * (size_t)p.G * p.W, st));
         CU(cudaMemsetAsync(p.nl_cnt, 0, sizeof(int) * (size_t)p.G * 2 * RW, st));
         CU(cudaMemsetAsync(p.nl_ovf, 0, sizeof(int) * (size_t)p.G * 2, st));
-        CU(cudaMemsetAsync(p.swept, 0, sizeof(long long) * (size_t)p.G * 2, st));        // instrumented builds only
+        CU(cudaMemsetAsync(p.swept, 0, sizeof(long long) * (size_t)p.G * 2, st));        // compactions (scldpc_bp_sweep_stats)
         CU(cudaMemsetAsync(p.pos_er, 0, sizeof(u64) * (size_t)p.G * d->L * p.W, st));
-        if (n_caps > 0) {
+        if (mode == SM_CKPT) {
             CU(cudaMemsetAsync(p.lane_ck, 0, sizeof(int) * (size_t)p.G * p.lanes, st));
             CU(cudaMemsetAsync(p.pause_mask, 0, sizeof(u64) * (size_t)p.G * p.W, st));
         }
@@ -764,7 +775,7 @@ static int bp_stream_impl(const scldpc_dims_t *d, const scldpc_batch_t *b, const
         if (adaptive) CU(cudaMemsetAsync(p.alive_total + 1 + slot, 0x7f, sizeof(int), st));
         if (node) bp_launch_node_settle(d->dv, d->dc, p, st);
         bp_launch_count_pairs(d->dv, d->dc, p, st);
-        if (ss) ss_launch_stream(p, st);         // records of the stopped frames, before the harvest re-arms their lanes
+        if (mode == SM_HEAD) ss_launch_stream(p, st);   // records of the stopped frames, before the harvest re-arms their lanes
         bp_launch_stream_harvest(p, (cfg->flags & SCLDPC_F_EXP_ALL) ? 1 : 0, st);
         if (node) {
             bp_launch_node_arm(p, st);
@@ -801,7 +812,7 @@ extern "C" int scldpc_bp_stream(const scldpc_dims_t *d, const scldpc_batch_t *b,
                                 const scldpc_stream_out_t *out, void *workspace_dev, size_t workspace_bytes,
                                 long long *iters_launched_host, void *stream)
 {
-    return bp_stream_impl(d, b, cfg, nullptr, 0, nullptr, out, workspace_dev, workspace_bytes, iters_launched_host, stream);
+    return bp_stream_impl(d, b, cfg, SM_PLAIN, StreamInputs{}, out, workspace_dev, workspace_bytes, iters_launched_host, stream);
 }
 
 // The same stream with checkpoints at the caps of an ascending list (include/scldpc.h).
@@ -817,12 +828,10 @@ extern "C" int scldpc_bp_stream_caps(const scldpc_dims_t *d, const scldpc_batch_
         if (k > 0 && !unlimited_last && caps_host[k] <= caps_host[k - 1])
             return fail(SCLDPC_EINVAL, "caps must be strictly ascending: cap %d (%d) <= cap %d (%d)", k, caps_host[k], k - 1, caps_host[k - 1]);
     }
-    if (!cfg) return fail(SCLDPC_EINVAL, "bad stream configuration");
-    if (cfg->max_it != 0) return fail(SCLDPC_EINVAL, "cfg->max_it must be 0 with caps: the caps replace it");
-    if (cfg->flags & SCLDPC_F_MESSAGES) return fail(SCLDPC_EINVAL, "frame streams with caps need the node-state sweeps (no SCLDPC_F_MESSAGES)");
     if (!out) return fail(SCLDPC_EINVAL, "output pointer is NULL");
     const scldpc_stream_out_t o{out->iters_dev, out->residual_dev, out->blocks_err_dev, out->erasures_exp_dev, out->blocks_err_exp_dev};
-    return bp_stream_impl(d, b, cfg, caps_host, n_caps, nullptr, &o, workspace_dev, workspace_bytes, iters_launched_host, stream);
+    return bp_stream_impl(d, b, cfg, SM_CKPT, StreamInputs{caps_host, n_caps, nullptr, 0, nullptr}, &o, workspace_dev, workspace_bytes,
+                          iters_launched_host, stream);
 }
 
 // The same stream (unlimited BP) with the stopping-set record of every frame in place of the size-two expurgation (include/scldpc.h).
@@ -831,14 +840,10 @@ extern "C" int scldpc_bp_stream_stopping_sets(const scldpc_dims_t *d, const scld
                                               const scldpc_stream_ss_out_t *out, void *workspace_dev, size_t workspace_bytes,
                                               long long *iters_launched_host, void *stream)
 {
-    if (!cfg) return fail(SCLDPC_EINVAL, "bad stream configuration");
-    if (cfg->flags & SCLDPC_F_MESSAGES)
-        return fail(SCLDPC_EINVAL, "frame streams with stopping sets need the node-state sweeps (no SCLDPC_F_MESSAGES)");
-    if (cfg->max_it != 0) return fail(SCLDPC_EINVAL, "cfg->max_it must be 0: stopping sets are records of unlimited BP");
-    if (!out || !out->iters_dev || !out->records_dev) return fail(SCLDPC_EINVAL, "output pointer is NULL");
-    const StreamSs ss{counted_pos_host, unscanned_head_cns, out->records_dev};
+    if (!out || !out->records_dev) return fail(SCLDPC_EINVAL, "output pointer is NULL");
     const scldpc_stream_out_t o{out->iters_dev, nullptr, nullptr, nullptr, nullptr};
-    return bp_stream_impl(d, b, cfg, nullptr, 0, &ss, &o, workspace_dev, workspace_bytes, iters_launched_host, stream);
+    return bp_stream_impl(d, b, cfg, SM_HEAD, StreamInputs{nullptr, 0, counted_pos_host, unscanned_head_cns, out->records_dev}, &o,
+                          workspace_dev, workspace_bytes, iters_launched_host, stream);
 }
 
 // first_window / n_windows: the windows [first_window, first_window + n_windows) of the chain (n_windows < 0: to the end).
@@ -1008,7 +1013,7 @@ extern "C" int scldpc_bp_position_counts(const scldpc_dims_t *d, uint32_t flags,
     if (!workspace_dev || !pos_cnt_dev || !pos_pairs_dev) return fail(SCLDPC_EINVAL, "NULL pointer");
     if ((rc = have_device())) return rc;
     BpParams p;
-    carve(d, flags, workspace_dev, &p);
+    carve(d, flags, SM_PLAIN, workspace_dev, &p);
     const size_t bytes = sizeof(int32_t) * (size_t)d->n_graphs * d->L * 64 * d->n_words;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     CU(cudaMemcpyAsync(pos_cnt_dev, p.pos_cnt, bytes, cudaMemcpyDeviceToDevice, st));
@@ -1114,7 +1119,7 @@ extern "C" int scldpc_bp_sweep_stats(const scldpc_dims_t *d, uint32_t flags, voi
     if (rc) return rc;
     if (!workspace_dev || !out_host) return fail(SCLDPC_EINVAL, "NULL pointer");
     BpParams p;
-    carve(d, flags, workspace_dev, &p);
+    carve(d, flags, SM_PLAIN, workspace_dev, &p);
     std::vector<long long> h(2 * (size_t)d->n_graphs);
     CU(cudaMemcpy(h.data(), p.swept, sizeof(long long) * h.size(), cudaMemcpyDeviceToHost));
     out_host[0] = out_host[1] = 0;

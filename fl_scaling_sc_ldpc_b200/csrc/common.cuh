@@ -205,6 +205,16 @@ __device__ __forceinline__ void load_row(const int32_t *row, int (&e)[D])
     }
 }
 
+// Which frame stream a BpParams describes.  bp_stream_impl (capi.cu) decides it once per call; every kernel and launcher that
+// treats the streams differently reads BpParams::stream_mode.  0 is also the value of every decoder that is not a stream (their
+// parameter blocks start zeroed).
+enum StreamMode : int {
+    SM_PLAIN = 0,   // unlimited BP (scldpc_bp_stream with cfg->max_it == 0)
+    SM_CAPPED,      // at most stream_cap iterations per frame (scldpc_bp_stream with cfg->max_it > 0)
+    SM_CKPT,        // checkpoints at caps[0 .. n_caps-1], capped at the last (scldpc_bp_stream_caps)
+    SM_HEAD,        // unlimited BP with the unscanned head and stopping-set records (scldpc_bp_stream_stopping_sets)
+};
+
 // Internal parameter block (by value to every BP kernel).
 struct BpParams {
     // dimensions
@@ -312,6 +322,7 @@ struct BpParams {
     int *ss_lost, *ss_big;    // [G][L][lanes] lost VNs / VNs of components with more than two VNs, per position (ss_classify_kernel)
     const unsigned char *ss_counted;   // [L] positions whose VNs can be lost
     int32_t *ss_records;      // [G][B][4] per-frame records, indexed by frame id
+    StreamMode stream_mode;   // frame streams: which stream this is (SM_PLAIN for every other decoder)
 };
 
 // graph handled by block coordinate b of a grid that is sized by the list of graphs still decoding

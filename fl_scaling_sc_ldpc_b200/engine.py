@@ -68,6 +68,14 @@ def words_for(n_frames: int) -> int:
     raise ValueError("at most 1024 frames per graph")
 
 
+def _doping(doping_points, M: int):
+    """(hard positions, soft positions, soft counts) of ``doping_points``: a list of positions (hard doping) or a dict
+    {position: alpha} (soft doping: the first int(alpha*M) VNs of the position are known, PD.py:175-183)."""
+    if isinstance(doping_points, dict):
+        return [], [int(p) for p in doping_points], [int(a * M) for a in doping_points.values()]
+    return [int(p) for p in doping_points], [], []
+
+
 def _device(device=None) -> torch.device:
     if not torch.cuda.is_available():
         raise _lib.ScldpcError("no CUDA device: fl_scaling_sc_ldpc_b200 has no CPU fallback")
@@ -98,7 +106,6 @@ class FrameBatch:
         self._graph_err = torch.zeros(1, dtype=torch.int32, device=dev)
         self._keys = None
         self._ws = None
-        self._ws_flags = None
         self.cbatch = _lib.Batch(self.vn_cn.data_ptr(), self.vn_slot.data_ptr(), self.cn_edge.data_ptr(), self.chan.data_ptr())
 
     # ---- graphs ------------------------------------------------------------------------------------------
@@ -177,13 +184,7 @@ class FrameBatch:
                 ctypes.byref(self.dims), ctypes.c_void_p(self.chan.data_ptr()), ctypes.c_double(float(eps)), a, len(hard),
                 ctypes.c_uint64(seed), ctypes.c_uint64(first_graph_id), ctypes.c_uint32(first_frame), ctypes.c_uint32(first_vn), _stream()))
             return self
-        hard, soft_p, soft_c = [], [], []
-        if isinstance(doping_points, dict):
-            for pos, alpha in doping_points.items():
-                soft_p.append(int(pos))
-                soft_c.append(int(alpha * self.ens.M))
-        else:
-            hard = [int(p) for p in doping_points]
+        hard, soft_p, soft_c = _doping(doping_points, self.ens.M)
         arr = lambda xs: (ctypes.c_int32 * max(1, len(xs)))(*xs)
         L = _lib.lib()
         if np.ndim(eps) == 0:
@@ -207,7 +208,10 @@ class FrameBatch:
 
     # ---- workspace ---------------------------------------------------------------------------------------
     def workspace(self, flags: int) -> torch.Tensor:
-        need = _lib.lib().scldpc_bp_workspace_bytes(ctypes.byref(self.dims), flags)
+        return self._workspace_bytes(_lib.lib().scldpc_bp_workspace_bytes(ctypes.byref(self.dims), flags))
+
+    def _workspace_bytes(self, need: int) -> torch.Tensor:
+        """The workspace grown to ``need`` bytes, the result of a size query (0: the query failed)."""
         if need == 0:
             raise _lib.ScldpcError(_lib.lib().scldpc_last_error().decode())
         if self._ws is None or self._ws.numel() < need:
@@ -414,100 +418,57 @@ def decode_bp_stream(fb: FrameBatch, frames_per_graph: int, eps, seed: int, firs
     if stopping_sets is None and unscanned_head_cns:
         raise ValueError("unscanned_head_cns applies to stopping_sets streams only")
     L = _lib.lib()
-    G, B = fb.n_graphs, int(frames_per_graph)
+    G, B, dev = fb.n_graphs, int(frames_per_graph), fb.device
     eps_arr = np.full(G, float(eps)) if np.ndim(eps) == 0 else np.asarray(eps, np.float64)
     assert eps_arr.shape == (G,)
-    hard, soft_p, soft_c = [], [], []
-    if isinstance(doping_points, dict):
-        for pos, alpha in doping_points.items():
-            soft_p.append(int(pos)); soft_c.append(int(alpha * fb.ens.M))
-    else:
-        hard = [int(p) for p in doping_points]
     arr = lambda xs: np.asarray(xs or [0], np.int32)
+    hard, soft_p, soft_c = _doping(doping_points, fb.ens.M)
     a_h, a_sp, a_sc = arr(hard), arr(soft_p), arr(soft_c)
     ptr = lambda a: a.ctypes.data_as(ctypes.c_void_p).value
     flags = (F_TERMINATED if is_term else 0) | (F_EXP_ALL if exp_all else 0) | _sweep_flags("SCLDPC_STREAM_NODE", messages)
-    if caps is not None:
-        # the library validates the list; max_it goes through unchanged so that a combination with caps is rejected there too
-        cfg = _lib.StreamCfg(B, int(harvest_every), flags, len(hard), len(soft_p), ptr(eps_arr), ptr(a_h), ptr(a_sp), ptr(a_sc),
-                             int(seed), int(first_graph_id), int(max_it))
-        return _decode_bp_stream_caps(fb, cfg, caps, collect)
-    if stopping_sets is not None:
-        cfg = _lib.StreamCfg(B, int(harvest_every), flags, len(hard), len(soft_p), ptr(eps_arr), ptr(a_h), ptr(a_sp), ptr(a_sc),
-                             int(seed), int(first_graph_id), 0)
-        return _decode_bp_stream_ss(fb, cfg, stopping_sets, int(unscanned_head_cns), collect)
+    # with caps, max_it goes through unchanged so that the library rejects a combination with caps
     cfg = _lib.StreamCfg(B, int(harvest_every), flags, len(hard), len(soft_p), ptr(eps_arr), ptr(a_h), ptr(a_sp), ptr(a_sc),
-                         int(seed), int(first_graph_id), max(0, int(max_it)))
-    res = torch.zeros((5, G, B), dtype=torch.int32, device=fb.device)
-    out = _lib.StreamOut(*[res[i].data_ptr() for i in range(5)])
-    need = L.scldpc_bp_stream_workspace_bytes(ctypes.byref(fb.dims), flags)
-    if need == 0:
-        raise _lib.ScldpcError(L.scldpc_last_error().decode())
-    if fb._ws is None or fb._ws.numel() < need:
-        fb._ws = None
-        fb._ws = torch.empty(need, dtype=torch.uint8, device=fb.device)
+                         int(seed), int(first_graph_id), int(max_it) if caps is not None else max(0, int(max_it)))
+    dims = ctypes.byref(fb.dims)
+    if caps is not None:                       # scldpc_bp_stream_caps (the library validates the list)
+        caps_arr = np.ascontiguousarray([int(c) for c in caps], np.int32)
+        iters = torch.zeros((G, B), dtype=torch.int32, device=dev)
+        stats = torch.zeros((4, max(len(caps_arr), 1), G, B), dtype=torch.int32, device=dev)
+        outs = (iters, stats)
+        call, need = L.scldpc_bp_stream_caps, L.scldpc_bp_stream_caps_workspace_bytes(dims)
+        args = (caps_arr.ctypes.data_as(ctypes.c_void_p), len(caps_arr),
+                ctypes.byref(_lib.StreamCapsOut(iters.data_ptr(), *[stats[i].data_ptr() for i in range(4)])))
+    elif stopping_sets is not None:            # scldpc_bp_stream_stopping_sets
+        cp = np.ascontiguousarray(np.asarray(stopping_sets, dtype=np.uint8))
+        if cp.shape != (fb.ens.L,):
+            raise ValueError("stopping_sets needs one counted flag per position")
+        iters = torch.zeros((G, B), dtype=torch.int32, device=dev)
+        records = torch.zeros((G, B, 4), dtype=torch.int32, device=dev)
+        outs = (iters, records)
+        call, need = L.scldpc_bp_stream_stopping_sets, L.scldpc_bp_stream_stopping_sets_workspace_bytes(dims)
+        args = (cp.ctypes.data_as(ctypes.c_void_p), int(unscanned_head_cns),
+                ctypes.byref(_lib.StreamSsOut(iters.data_ptr(), records.data_ptr())))
+    else:                                      # scldpc_bp_stream: [5][G][B], iters first
+        res = torch.zeros((5, G, B), dtype=torch.int32, device=dev)
+        outs = (res,)
+        call, need = L.scldpc_bp_stream, L.scldpc_bp_stream_workspace_bytes(dims, flags)
+        args = (ctypes.byref(_lib.StreamOut(*[res[i].data_ptr() for i in range(5)])),)
+    ws = fb._workspace_bytes(need)
     launched = ctypes.c_longlong(0)
-    _lib.check(L.scldpc_bp_stream(ctypes.byref(fb.dims), ctypes.byref(fb.cbatch), ctypes.byref(cfg), ctypes.byref(out),
-                                  ctypes.c_void_p(fb._ws.data_ptr()), ctypes.c_size_t(fb._ws.numel()), ctypes.byref(launched),
-                                  _stream()))
+    _lib.check(call(dims, ctypes.byref(fb.cbatch), ctypes.byref(cfg), *args, ctypes.c_void_p(ws.data_ptr()),
+                    ctypes.c_size_t(ws.numel()), ctypes.byref(launched), _stream()))
     if not collect:
-        return res, launched.value
-    r = res.cpu().numpy()
-    return StreamResult(r[0], r[1], r[2], r[3], r[4], iters_launched=launched.value,
-                        edge_updates=int(r[0].astype(np.int64).sum()) * 2 * fb.ens.E)
-
-
-def _decode_bp_stream_caps(fb: FrameBatch, cfg, caps, collect: bool):
-    L = _lib.lib()
-    G, B = fb.n_graphs, int(cfg.frames_per_graph)
-    caps_arr = np.ascontiguousarray([int(c) for c in caps], np.int32)
-    K = len(caps_arr)
-    iters = torch.zeros((G, B), dtype=torch.int32, device=fb.device)
-    stats = torch.zeros((4, max(K, 1), G, B), dtype=torch.int32, device=fb.device)
-    out = _lib.StreamCapsOut(iters.data_ptr(), *[stats[i].data_ptr() for i in range(4)])
-    need = L.scldpc_bp_stream_caps_workspace_bytes(ctypes.byref(fb.dims))
-    if need == 0:
-        raise _lib.ScldpcError(L.scldpc_last_error().decode())
-    if fb._ws is None or fb._ws.numel() < need:
-        fb._ws = None
-        fb._ws = torch.empty(need, dtype=torch.uint8, device=fb.device)
-    launched = ctypes.c_longlong(0)
-    _lib.check(L.scldpc_bp_stream_caps(ctypes.byref(fb.dims), ctypes.byref(fb.cbatch), ctypes.byref(cfg),
-                                       caps_arr.ctypes.data_as(ctypes.c_void_p), K, ctypes.byref(out),
-                                       ctypes.c_void_p(fb._ws.data_ptr()), ctypes.c_size_t(fb._ws.numel()), ctypes.byref(launched),
-                                       _stream()))
-    if not collect:
-        return iters, stats, launched.value
-    it, st = iters.cpu().numpy(), stats.cpu().numpy()
-    return StreamCapsResult(tuple(int(c) for c in caps_arr), it, st[0], st[1], st[2], st[3], iters_launched=launched.value,
-                            edge_updates=int(it.astype(np.int64).sum()) * 2 * fb.ens.E)
-
-
-def _decode_bp_stream_ss(fb: FrameBatch, cfg, counted, unscanned_head_cns: int, collect: bool):
-    L = _lib.lib()
-    G, B = fb.n_graphs, int(cfg.frames_per_graph)
-    cp = np.ascontiguousarray(np.asarray(counted, dtype=np.uint8))
-    if cp.shape != (fb.ens.L,):
-        raise ValueError("stopping_sets needs one counted flag per position")
-    iters = torch.zeros((G, B), dtype=torch.int32, device=fb.device)
-    records = torch.zeros((G, B, 4), dtype=torch.int32, device=fb.device)
-    out = _lib.StreamSsOut(iters.data_ptr(), records.data_ptr())
-    need = L.scldpc_bp_stream_stopping_sets_workspace_bytes(ctypes.byref(fb.dims))
-    if need == 0:
-        raise _lib.ScldpcError(L.scldpc_last_error().decode())
-    if fb._ws is None or fb._ws.numel() < need:
-        fb._ws = None
-        fb._ws = torch.empty(need, dtype=torch.uint8, device=fb.device)
-    launched = ctypes.c_longlong(0)
-    _lib.check(L.scldpc_bp_stream_stopping_sets(ctypes.byref(fb.dims), ctypes.byref(fb.cbatch), ctypes.byref(cfg),
-                                                cp.ctypes.data_as(ctypes.c_void_p), unscanned_head_cns, ctypes.byref(out),
-                                                ctypes.c_void_p(fb._ws.data_ptr()), ctypes.c_size_t(fb._ws.numel()),
-                                                ctypes.byref(launched), _stream()))
-    if not collect:
-        return iters, records, launched.value
-    it = iters.cpu().numpy()
-    return StreamStoppingSetResult(it, records.cpu().numpy(), iters_launched=launched.value,
-                                   edge_updates=int(it.astype(np.int64).sum()) * 2 * fb.ens.E)
+        return (*outs, launched.value)
+    host = [t.cpu().numpy() for t in outs]
+    kw = lambda it: dict(iters_launched=launched.value, edge_updates=int(it.astype(np.int64).sum()) * 2 * fb.ens.E)
+    if caps is not None:
+        it, st = host
+        return StreamCapsResult(tuple(int(c) for c in caps_arr), it, *st, **kw(it))
+    if stopping_sets is not None:
+        it, rec = host
+        return StreamStoppingSetResult(it, rec, **kw(it))
+    (r,) = host
+    return StreamResult(*r, **kw(r[0]))
 
 
 def decode_host(ens: Ensemble, vn_cn: np.ndarray, erased: np.ndarray, W: int = 0, max_it: int = UNLIMITED, init_it: int = 0,
