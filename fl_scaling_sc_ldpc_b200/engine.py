@@ -120,7 +120,11 @@ class FrameBatch:
                         first_position: int = 0) -> "FrameBatch":
         """Draw graphs on the device: the semi-structured ensemble (``generate_code`` BP_FULL.c:1656 / ``SC.gen_slots``
         SC.py:53), its tail-biting variant, or the protograph-based ensemble (``sc_ldpc_protograph.py``).
-        ``first_position`` > 0: the batch is a piece of a longer chain starting at that absolute position (streams)."""
+        ``first_position`` > 0: the batch is a piece of a longer chain starting at that absolute position (streams).
+        Absolute CN positions are 32-bit Philox counter words, so ``first_position + L + dv - 1 <= 2**32``; a piece
+        beyond that raises ``ValueError`` rather than reusing the permutations of position 0 onwards."""
+        if first_position < 0 or first_position + self.ens.L + self.ens.dv - 1 > 1 << 32:
+            raise ValueError(f"first_position {first_position} + L + dv - 1 exceeds 2**32 CN positions")
         L = _lib.lib()
         if first_position:
             if tail_biting or protograph:
@@ -174,7 +178,14 @@ class FrameBatch:
         ``doping_points``: list of positions (hard doping) or dict {position: alpha} (soft doping: the first
         int(alpha*M) VNs are known, PD.py:175-183).  Lane f holds frame ``first_frame + f`` of the graph's channel
         stream (``first_frame`` a multiple of 4).  ``first_vn`` > 0: the batch is a piece of a longer chain whose first VN
-        has that absolute index (hard doping only; positions are local to the piece)."""
+        has that absolute index (hard doping only; positions are local to the piece).
+        VN and frame ids are 32-bit Philox counter words: ``first_vn + n <= 2**32`` and
+        ``first_frame + 64 * n_words <= 2**32`` (every lane, used or not, has its frame id), else ``ValueError`` -- ids
+        past 2**32 would wrap and repeat earlier realisations."""
+        if first_vn < 0 or first_vn + self.ens.n > 1 << 32:
+            raise ValueError(f"first_vn {first_vn} + n ({self.ens.n}) exceeds 2**32 VN ids")
+        if first_frame < 0 or first_frame + 64 * self.n_words > 1 << 32:
+            raise ValueError(f"first_frame {first_frame} + 64 * n_words ({64 * self.n_words}) exceeds 2**32 frame ids")
         if first_vn:
             if isinstance(doping_points, dict) or np.ndim(eps) != 0:
                 raise ValueError("chain pieces take one eps and hard doping only")

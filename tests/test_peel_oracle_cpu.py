@@ -9,10 +9,10 @@ import pytest
 
 import oracle
 from fl_scaling_sc_ldpc_b200 import peeling_decoding as pdx
+from tests.util import M32, philox4x32_10
 
 Z = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "peel_golden.npz"))
 PEEL_SEED = 777
-M32 = 0xFFFFFFFF
 
 
 def _pool_map(fn, jobs):
@@ -76,17 +76,6 @@ def test_fast_oracle_edge_cases():
             assert len(a[0]) == steps + 1 and (a[0] == b[0]).all() and a[1] == b[1]
 
 
-# ---- Philox-4x32-10 (Salmon et al., SC'11; Random123), restated from the paper's round function ----
-def philox4x32_10(ctr, key):
-    c0, c1, c2, c3 = ctr
-    k0, k1 = key
-    for _ in range(10):
-        p0, p1 = 0xD2511F53 * c0, 0xCD9E8D57 * c2
-        c0, c1, c2, c3 = (p1 >> 32) ^ c1 ^ k0, p1 & M32, (p0 >> 32) ^ c3 ^ k1, p0 & M32
-        k0, k1 = (k0 + 0x9E3779B9) & M32, (k1 + 0xBB67AE85) & M32
-    return [c0, c1, c2, c3]
-
-
 def picks_restated(seed, frame_id, n):
     """draw s of a frame = philox4x32_10(counter = (s // 4, 0, frame_id.lo, frame_id.hi), key = (seed.lo ^ 'peel',
     seed.hi))[s % 4]"""
@@ -104,6 +93,15 @@ def test_philox_restatement_reproduces_random123_known_answers():
             (0xD16CFE09, 0x94FDCCEB, 0x5001E420, 0x24126EA1))]
     for ctr, key, want in kat:
         assert philox4x32_10(ctr, key) == list(want)
+    # the vectorised form (uint64 arrays, as the generator restatements in test_generators_gpu.py use it) gives the same
+    # words element by element, with the counters mixed with ints and broadcast
+    c0 = np.array([kat[0][0][0], kat[1][0][0], kat[2][0][0]] * 2, np.int64)
+    for j, (ctr, key, want) in enumerate(kat):
+        out = philox4x32_10((c0,) + ctr[1:], key)
+        assert all(o.dtype == np.uint64 and o.shape == (6,) for o in out)
+        assert [int(o[j]) for o in out] == list(want) and [int(o[j + 3]) for o in out] == list(want)
+        arr = philox4x32_10(tuple(np.full((2, 3), c, np.uint64) for c in ctr), key)
+        assert all((o == w).all() for o, w in zip(arr, want))
 
 
 def test_philox_picks_known_answer():

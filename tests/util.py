@@ -7,6 +7,20 @@ import numpy as np
 import oracle
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+M32 = 0xFFFFFFFF
+
+
+def philox4x32_10(ctr, key):
+    """Philox-4x32-10 (Salmon et al., SC'11; Random123), restated from the paper's round function.  The counter words are
+    ints or NumPy integer arrays (broadcast together, computed as uint64), the key words ints; returns the four output
+    words, ints or uint64 arrays."""
+    c0, c1, c2, c3 = (x.astype(np.uint64) if isinstance(x, np.ndarray) else x for x in ctr)
+    k0, k1 = key
+    for _ in range(10):
+        p0, p1 = 0xD2511F53 * c0, 0xCD9E8D57 * c2
+        c0, c1, c2, c3 = (p1 >> 32) ^ c1 ^ k0, p1 & M32, (p0 >> 32) ^ c3 ^ k1, p0 & M32
+        k0, k1 = (k0 + 0x9E3779B9) & M32, (k1 + 0xBB67AE85) & M32
+    return [c0, c1, c2, c3]
 
 
 def golden_files():
